@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PINN residual-and-gradient hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P] [--dump-outputs DIR]
 
 A step = one training evaluation (forward + Laplacian + loss + parameter gradients; for N>1 including the
 sum of the 8 + 1521 float64 over the ranks, fused into the reduction kernel or, --allreduce nccl, as a
@@ -169,8 +169,8 @@ def dense_grid_inference(dev, n_axis=464):
 def run_reference(args):
     """--impl reference: the reference's CPU implementation of the path on the host cores (rank 0 only): float64 nested
     autograd (oracle/ref_autograd.py, pinned to the real reference by tests/test_oracle.py) on the SAME workload as the
-    GPU arm - one full batch of --points (2^18) points per step, --steps steps, all host threads (set explicitly).  The
-    step count is only clipped if the run would exceed ~3 minutes (0.4 s per step on 16 cores)."""
+    GPU arm - one full batch of --points (2^18) points per step, --steps steps (about 0.4 s each on 16 cores), all host
+    threads (set explicitly)."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -183,20 +183,24 @@ def run_reference(args):
     g = torch.Generator().manual_seed(1234)
     x, y, z, R, i1, i2 = ra.sample_box(ns, "poc", g)
     th = torch.tensor(theta, dtype=torch.float64)
-    t0 = time.time()
     ra.loss_and_grad("poc", th, x, y, z, R, i1, i2)
-    t_first = time.time() - t0
     W = max(0, min(args.warmup, 3) - 1)
     for _ in range(W):
         ra.loss_and_grad("poc", th, x, y, z, R, i1, i2)
-    steps = max(1, min(args.steps, int(180.0 / max(t_first, 1e-3))))
+    steps = max(1, args.steps)
     t0 = time.time()
     for _ in range(steps):
-        ra.loss_and_grad("poc", th, x, y, z, R, i1, i2)
+        r = ra.loss_and_grad("poc", th, x, y, z, R, i1, i2)
     dt = (time.time() - t0) / steps
     v = ns / dt
+    if args.dump_outputs:
+        E = r[3]
+        if E.shape[0] > DUMP_MAX_POINTS:   # a fixed, seeded sample of the per-point energies keeps the dump small
+            keep = np.sort(np.random.default_rng(0).choice(E.shape[0], DUMP_MAX_POINTS, replace=False))
+            E = E[torch.from_numpy(keep)]
+        dump_outputs(args.dump_outputs, loss=torch.stack(r[:3]), dtheta=r[4], E=E)
     sample = ("each step = one full batch of %d points; float64 nested autograd (oracle/ref_autograd.py), %d threads; "
-              "%d of the %d requested steps timed" % (ns, cores, steps, args.steps))
+              "%d steps timed" % (ns, cores, steps))
     emit({
         "impl": "reference", "metric": "collocation points/sec per training step (fwd+lap+bwd)", "value": v,
         "unit": "points/s", "n_gpus": args.gpus, "steps": steps, "warmup": W + 1, "ms_per_step": dt * 1e3,
@@ -240,6 +244,18 @@ def claim_stdout():
 def emit(line):
     _RESULT_OUT.write(json.dumps(line) + "\n")
     _RESULT_OUT.flush()
+
+
+DUMP_MAX_POINTS = 1 << 20          # --dump-outputs: per-point arrays beyond this many points are sampled (8 MB float64)
+
+
+def dump_outputs(directory, **arrays):
+    """--dump-outputs DIR: the arrays the timed path returned in its last step, one float64 DIR/<name>.npy each, so that
+    two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  Both arms
+    write loss.npy (Ltot, Lpde, Lbc) and dtheta.npy under the same names."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.detach().cpu().numpy().astype(np.float64))
 
 
 def tensor_ceiling(flop_per_launch, kernel_ms):
@@ -481,6 +497,11 @@ def main():
     ap.add_argument("--allreduce", default="fused", choices=["fused", "nccl"],
                     help="N>1: sum over ranks fused into the reduction kernel over NVLink peer memory (pinn_dp_*), or a "
                          "separate NCCL all-reduce per step (the baseline it replaces)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned as DIR/<name>.npy (float64): "
+                         "loss.npy (Ltot, Lpde, Lbc), dtheta.npy (1521) and sums.npy (the 8 sums of the C ABI); "
+                         "--impl reference: loss.npy, dtheta.npy and E.npy (E per point, a fixed seeded sample of "
+                         "%d points when the batch is larger)" % DUMP_MAX_POINTS)
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -588,6 +609,8 @@ def main():
         step(i_spin)
         i_spin += 1
     torch.cuda.synchronize()
+    # however long the spin-up took, the timed region starts on batch 0: its last step sees the same batch in every run
+    i_spin = -(-i_spin // N_BATCHES) * N_BATCHES
     # Two back-to-back timed regions of the same K steps (clocks sampled over both): the first without any extra stream
     # operation gives `value`; the second brackets every step-kernel launch with CUDA events on the launching stream
     # (pinn_profile_begin/collect) and gives the kernel's average duration for the roofline.  (The event records sit
@@ -597,6 +620,7 @@ def main():
     t0 = time.time()
     ms = timed(step, i_spin, K)
     launches = h.launch_count() - launches0
+    last = out.clone() if args.dump_outputs else None
     h.profile_begin()
     ms_profiled = timed(step, i_spin + K, K)
     kern_ms, kern_n = h.profile_collect()
@@ -777,6 +801,8 @@ def main():
         if not args.no_cpu_baseline and world == 1 and not args.no_extras and not args.scaling_legs_only:
             v, cores, sample, _ = cpu_reference_points_per_s(np.ascontiguousarray(load_theta()), args.cpu_seconds, n)
             line["cpu_baseline"] = {"value": v, "unit": "points/s", "cores": cores, "kind": "port", "sample": sample}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, loss=last[:3], dtheta=last[8:], sums=last[:8])
         emit(line)
     if fused:
         h.dp_status()

@@ -555,3 +555,31 @@ def test_prepared_host_step_equals_the_plain_host_call(init_theta):
     assert abs(s2[0] - ref["Ltot"]) / ref["Ltot"] < 1e-5
     t = pk.Handle.get(0).host_timing()
     assert t["total"] > 0 and abs(t["enqueue"] + t["wait"] + t["copy_out"] - t["total"]) < 1.0
+
+
+def test_bench_dumps_what_its_last_timed_step_computed(tmp_path):
+    """bench.py --dump-outputs: loss.npy, dtheta.npy and sums.npy are, bit for bit, the evaluation of the batch the last
+    of the --steps timed steps used (the timed region starts on batch 0 whatever the spin-up took), so that two builds run
+    with the same arguments can be compared output for output."""
+    import json
+    import subprocess
+    import sys
+    import bench    # the repository root is on sys.path (tests/conftest.py)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    from pinn_for_quantum_wavefunction_surfaces_b200 import dp
+    n, steps = 4096, 7
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "3",
+                        "--points", str(n), "--no-extras", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+    loss, sums, dth = (np.load(tmp_path / (k + ".npy")) for k in ("loss", "sums", "dtheta"))
+    assert loss.dtype == sums.dtype == dth.dtype == np.float64
+    assert loss.shape == (3,) and sums.shape == (8,) and dth.shape == (1521,) and np.array_equal(loss, sums[:3])
+    b = bench.synth_batch(n, (steps - 1) % bench.N_BATCHES)
+    r1 = torch.sqrt((b[0] - b[3]) ** 2 + b[1] ** 2 + b[2] ** 2)
+    r2 = torch.sqrt((b[0] + b[3]) ** 2 + b[1] ** 2 + b[2] ** 2)
+    w = dp.global_weights(n, int((r1 >= 17.5).sum()), int((r2 >= 17.5).sum()), device=dev())
+    theta = torch.from_numpy(bench.load_theta().astype(np.float32)).to(dev())
+    s, g, _ = pk.loss_and_grad_raw(0, *[b[k].contiguous().to(dev()) for k in range(4)], theta, None, w)
+    assert np.array_equal(sums, s.cpu().numpy()) and np.array_equal(dth, g.cpu().numpy())
