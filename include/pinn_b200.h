@@ -15,7 +15,9 @@
  *    workspaces (per-CTA partial sums, set counters): ONE PER STREAM that calls in,
  *    allocated on the first call on that stream.  No allocation happens on later
  *    calls, so every *device* entry point is CUDA-graph capturable once one plain
- *    call has been made on the capturing stream.
+ *    call has been made on the capturing stream.  pinn_spheroidal_reduce also keeps
+ *    room for the largest sweep it has run on the stream: a capture of it needs one
+ *    plain call at least as large (nR * ceil(ns*nnu/128)) first.
  *  - every call takes the stream explicitly (as a void* holding a cudaStream_t) and
  *    selects the handle's device itself, so it may be called from any host thread
  *    (torch runs autograd.Function.backward on its own thread).  Calls on ONE stream
@@ -317,6 +319,25 @@ int pinn_enet_curve(pinn_handle* h, const float* theta, const double* R, int n, 
  */
 int pinn_grid_reduce(pinn_handle* h, int variant, const float* theta, int nx, int ny, int nz, const double lim[6], double R,
                      const double* wx, const double* wy, const double* wz, double* out, void* stream);
+
+/*
+ * Converged E(R): the Rayleigh-quotient sums of pinn_grid_reduce for a whole sweep of R in one launch (+ one finishing
+ * reduction), on a prolate-spheroidal node set instead of a Cartesian grid.  With the nuclei at x = +-R,
+ * s = (r1 + r2)/2 - R >= 0 and nu = (r2 - r1)/(2R) in [-1, 1], the point of node (s_i, nu_j) at R is
+ *     x = R (1 + s/R) nu,  y = sqrt(s (2R + s) (1 - nu^2)),  z = 0      (each operation in double, rounded as written)
+ * with weight 2 pi ws_i wnu_j ((R + s)^2 - (R nu)^2): the volume element r1 r2 ds dnu dphi cancels every 1/r of H psi and
+ * tensor Gauss-Legendre nodes converge exponentially (the model depends on (x,y,z) through r1, r2 only).
+ * R: device float64 [nR], every value > 0 - a row with R <= 0 is all NaN (R is not read on the host).
+ * s, ws: device float64 [ns]; nu, wnu: device float64 [nnu].  A node with s = 0 and nu = +-1 sits on a nucleus and gives
+ * NaN sums, like a grid point on a nucleus in pinn_grid_reduce.
+ * out (device, [nR][8] double): the row layout of pinn_grid_reduce per R, except slot 4 (the Hellmann-Feynman integrand
+ * is not smooth in these coordinates) = 0.  Rows are deterministic: row k is the same bits as a call with R[k] alone.
+ * nR * ceil(ns * nnu / 128) * 128 must stay below 2^31.  The call keeps 256 bytes per 128 node slots of one R for the largest
+ * sweep made so far on the stream (grown on a larger call, which is therefore not CUDA-graph capturable: make the largest call
+ * once outside the capture first).
+ */
+int pinn_spheroidal_reduce(pinn_handle* h, int variant, const float* theta, int nR, const double* R, int ns, const double* s,
+                           const double* ws, int nnu, const double* nu, const double* wnu, double* out, void* stream);
 
 #ifdef __cplusplus
 }

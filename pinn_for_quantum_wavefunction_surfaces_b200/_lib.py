@@ -11,7 +11,7 @@ EXPORTS = [
     "pinn_version", "pinn_theta_size", "pinn_theta_offsets", "pinn_create", "pinn_destroy", "pinn_last_error",
     "pinn_launch_count", "pinn_set_engine", "pinn_get_engine", "pinn_profile_begin", "pinn_profile_collect", "pinn_loss_fwd_bwd", "pinn_fields", "pinn_loss_fwd_bwd_host",
     "pinn_loss_fwd_bwd_tensors", "pinn_mask_from_index_sets", "pinn_measure_fp32_peak", "pinn_step_kernel_clock",
-    "pinn_sample", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
+    "pinn_sample", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_spheroidal_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
     "pinn_trainer_load_state", "pinn_trainer_set_batch", "pinn_trainer_run", "pinn_trainer_read", "pinn_trainer_batch",
     "pinn_trainer_stream",
     "pinn_host_timing", "pinn_dp_init", "pinn_dp_connect", "pinn_dp_connect_local", "pinn_dp_enable", "pinn_dp_status", "pinn_dp_set_timeout", "pinn_dp_shutdown",
@@ -99,6 +99,8 @@ def lib():
         L.pinn_enet_curve.restype = i32
         L.pinn_grid_reduce.argtypes = [vp, i32, vp, i32, i32, i32, ctypes.POINTER(f64), f64, vp, vp, vp, vp, vp]
         L.pinn_grid_reduce.restype = i32
+        L.pinn_spheroidal_reduce.argtypes = [vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, vp, vp, vp]
+        L.pinn_spheroidal_reduce.restype = i32
         L.pinn_trainer_create.argtypes = [vp, ctypes.POINTER(TrainConfig), vp, ctypes.POINTER(vp)]
         L.pinn_trainer_create.restype = i32
         L.pinn_trainer_destroy.argtypes = [vp]

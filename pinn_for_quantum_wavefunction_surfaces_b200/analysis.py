@@ -6,10 +6,15 @@
     energy_from_psi_LCAO     <->  energy_from_psi_LCAO(Ri, params)                          poc/main.py:467-492
     dEdR_int                 <->  dEdR_int(Ri, params) (Hellmann-Feynman)                   poc/main.py:646-676
     calculate_E_R            <->  calculate_E_R(params)                                     poc/main.py:495-517
+    spheroidal_sums          <->  the E_int / Elcao sums of calculate_E_R, converged (prolate-spheroidal Gauss-Legendre)
+    rayleigh_curve           <->  E_int, Elcao, E_net of calculate_E_R for a whole R sweep in one launch
     enet_curve / returnGate  <->  E-net on an R grid, -dE/dR, d2E/dR2, gate                 energy.py:21-33; poc/main.py:164-176, 1324-1332
 
 The grid is never materialised: the kernel generates the points from the three linspaces and accumulates the
-Simpson-weighted sums (pinn_grid_reduce); 10^8 points cost the same memory as 10^3.
+Simpson-weighted sums (pinn_grid_reduce); 10^8 points cost the same memory as 10^3.  That grid cannot resolve the cusps
+of psi at the nuclei (E_int is off by ~3e-3 at n_test = 80); spheroidal_sums / rayleigh_curve integrate in
+prolate-spheroidal coordinates instead, where the volume element cancels the 1/r terms and ~1000 nodes per R reach
+float32 accuracy (pinn_spheroidal_reduce, INTEGRATION.md).
 """
 import ctypes
 
@@ -112,6 +117,58 @@ def calculate_E_R(theta, params=None, **kw):
         d["E_net"][i] = s["E_net"]
         d["dEdR_HF"][i] = s["dVdR_psi2"] / s["psi2"] - 1.0 / (2.0 * Ri ** 2)
     return d
+
+
+def spheroidal_nodes(n_s=16, n_nu=24, panels=(0, 2, 6, 18)):
+    """(s, ws, nu, wnu), float64: Gauss-Legendre with n_s nodes on every panel [panels[i], panels[i+1]] of
+    s = (r1 + r2)/2 - R and n_nu nodes on nu = (r2 - r1)/(2R) in [-1, 1].  The domain is the spheroid
+    r1 + r2 <= 2 (R + panels[-1]); the same nodes serve every R."""
+    panels = np.asarray(panels, np.float64)
+    if n_s < 1 or n_nu < 1 or panels.size < 2 or panels[0] < 0 or np.any(np.diff(panels) <= 0):
+        raise ValueError("need n_s, n_nu >= 1 and increasing panel edges starting at s >= 0")
+    t, wt = np.polynomial.legendre.leggauss(int(n_s))
+    half = 0.5 * np.diff(panels)
+    s = (panels[:-1, None] + half[:, None] * (t[None, :] + 1.0)).ravel()
+    ws = (half[:, None] * wt[None, :]).ravel()
+    nu, wnu = np.polynomial.legendre.leggauss(int(n_nu))
+    return s, ws, nu, wnu
+
+
+def spheroidal_sums(theta, R, variant="poc", n_s=16, n_nu=24, panels=(0, 2, 6, 18), params=None, device=None):
+    """psiHpsi, psi2, lcaoHlcao, lcao2 (the sums of grid_sums) and E_net at every R, on the spheroidal node set of
+    spheroidal_nodes -> dict of float64 arrays over R.  One launch (+ one finishing reduction) for the whole sweep, one
+    host synchronisation.  The Hellmann-Feynman sum is not formed: its integrand is not smooth in these coordinates."""
+    if not torch.cuda.is_available():
+        raise PinnError("no CUDA device: the PINN hot path has no CPU fallback")
+    check_supported_model(params or {})
+    Rh = np.asarray(R, np.float64).ravel()
+    if Rh.size == 0 or not np.all(Rh > 0) or not np.all(np.isfinite(Rh)):
+        raise ValueError("R must be a non-empty list of finite values > 0")
+    h = Handle.get(torch.cuda.current_device() if device is None else device)
+    dev = torch.device("cuda", h.device)
+    variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
+    s, ws, nu, wnu = [torch.as_tensor(a).to(dev) for a in spheroidal_nodes(n_s, n_nu, panels)]
+    Rd = torch.as_tensor(Rh).to(dev)
+    out = torch.empty((Rh.size, 8), dtype=torch.float64, device=dev)
+    th = _theta32(theta, dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    rc = h.L.pinn_spheroidal_reduce(h.h, variant, _ptr(th), Rh.size, _ptr(Rd), s.numel(), _ptr(s), _ptr(ws), nu.numel(),
+                                    _ptr(nu), _ptr(wnu), _ptr(out), ctypes.c_void_p(stream))
+    h.check(rc, "pinn_spheroidal_reduce")
+    o = out.cpu().numpy()
+    return {"psiHpsi": o[:, 0], "psi2": o[:, 1], "lcaoHlcao": o[:, 2], "lcao2": o[:, 3], "E_net": o[:, 5]}
+
+
+def rayleigh_curve(theta, R=None, params=None, **kw):
+    """E_int = <psi|H|psi>/<psi|psi>, Elcao and E_net over an R sweep, converged (spheroidal_sums) -> dict of arrays.
+    R defaults to the R list of calculate_E_R (RxL .. RxR step 0.1)."""
+    pr = dict(_DEFAULTS)
+    pr.update(params or {})
+    if R is None:
+        R = np.round(np.arange(pr["RxL"], pr["RxR"] + .1, .1), 2)
+    R = np.asarray(R, np.float64).ravel()
+    s = spheroidal_sums(theta, R, params=pr, **kw)
+    return {"R": R, "E_int": s["psiHpsi"] / s["psi2"], "Elcao": s["lcaoHlcao"] / s["lcao2"], "E_net": s["E_net"]}
 
 
 def enet_curve(theta, R, device=None):

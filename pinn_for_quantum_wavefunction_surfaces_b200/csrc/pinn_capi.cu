@@ -84,7 +84,7 @@ int pinn_create(int device, pinn_handle** out) {
 }  // extern "C"
 
 static void ws_free(pinn_workspace& w) {
-  cudaFree(w.partials); cudaFree(w.weights); cudaFree(w.counts); cudaFree(w.grid_partials);
+  cudaFree(w.partials); cudaFree(w.weights); cudaFree(w.counts); cudaFree(w.grid_partials); cudaFree(w.sph_partials);
   w = pinn_workspace();
 }
 
@@ -160,6 +160,31 @@ pinn_workspace* ws_for(pinn_handle* h, cudaStream_t st, int rows) {
   w->rows = rows;
   w->last_use = ++h->ws_clock;
   return w;
+}
+
+bool ws_sph_rows(pinn_handle* h, pinn_workspace* w, cudaStream_t st, int rows) {
+  if (w->sph_rows >= rows) return true;
+  if (stream_is_capturing(st)) {
+    fail(h, PINN_EINVAL, "spheroidal sweep larger than any earlier one on a stream under CUDA-graph capture: make the largest "
+                         "call once on this stream outside the capture first");
+    return false;
+  }
+  if (w->in_graph) {
+    fail(h, PINN_EINVAL, "this stream's workspace is referenced by a captured graph and cannot grow");
+    return false;
+  }
+  cudaStreamSynchronize(st);  // the old rows may still be read by queued kernels
+  cudaFree(w->sph_partials);
+  w->sph_partials = nullptr;
+  w->sph_rows = 0;
+  cudaError_t e = cudaMalloc(&w->sph_partials, (size_t)rows * 8 * sizeof(double));
+  if (e != cudaSuccess) {
+    w->sph_partials = nullptr;
+    fail(h, (int)e, "spheroidal workspace allocation (cudaMalloc)");
+    return false;
+  }
+  w->sph_rows = rows;
+  return true;
 }
 
 // With the data-parallel exchange enabled the handle's exchange buffers carry one sequence of steps: calls must reach the

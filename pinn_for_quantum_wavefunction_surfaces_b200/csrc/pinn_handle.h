@@ -21,6 +21,8 @@ struct pinn_workspace {
   double* weights = nullptr;        // 4 doubles: the output of the set-count kernels when the caller passes no loss weights
   unsigned long long* counts = nullptr;  // [0..1] boundary-set sizes, [2] batch index of pinn_sample, [3] its block ticket
   double* grid_partials = nullptr;  // [sm_count + 1][8] dense-grid quadrature rows
+  double* sph_partials = nullptr;   // [sph_rows][8] rows of the spheroidal sweep (ws_sph_rows: grows, never shrinks)
+  int sph_rows = 0;
   uint64_t last_use = 0;
   bool in_graph = false;            // a call on this stream was captured into a CUDA graph: the addresses above must stay valid
 };
@@ -113,6 +115,9 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st);
 // The workspace of stream `st` with room for at least `rows` partial rows (created / grown on first use; the handle mutex
 // is held by the caller).  NULL + error message on failure.
 pinn_workspace* ws_for(pinn_handle* h, cudaStream_t st, int rows);
+// Room for `rows` rows of the spheroidal sweep in w (the workspace of st): allocated only when a call needs more rows than
+// any earlier call on the stream, which is refused under CUDA-graph capture.  false + error message on failure.
+bool ws_sph_rows(pinn_handle* h, pinn_workspace* w, cudaStream_t st, int rows);
 void ws_release(pinn_handle* h, cudaStream_t st);
 
 extern std::string g_create_err;

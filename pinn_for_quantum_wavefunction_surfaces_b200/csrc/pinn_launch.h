@@ -10,13 +10,20 @@ namespace pinn {
 // Dense-grid mode of the inference kernel (SURVEY.md 8f-3; poc/main.py:438-517, 639-676): point p of the n = nx*ny*nz
 // grid is (i,j,k) = meshgrid 'ij' order of three linspaces, R is one value, and instead of per-point stores the kernel
 // accumulates the quadrature sums  S = sum_p w_p * {psi H psi, psi^2, lcao H lcao, lcao^2, (dV/dR) psi^2}.
+// Second generator, sph = 1 (pinn_spheroidal_reduce): a sweep over nR values of R with the prolate-spheroidal node set
+// (s_i, nu_j) at every R.  Each R owns tiles_per_R super-tiles of 128 slots (slot l = i * nnu + j; the slots behind
+// ns * nnu repeat the last node with weight 0), so every super-tile has ONE R, and every warp of role 0 writes one row
+// {4 sums, -, E(R)} of its 32 points: [tiles][4 groups][8] in partials.  No tile's row depends on the other R of the sweep.
 struct GridDesc {
   int on;
+  int sph;
   int nx, ny, nz;
   double x0, dx, y0, dy, z0, dz;  // linspace start / step
   double R;
   const double *wx, *wy, *wz;     // 1-D quadrature weights (Simpson), device
-  double* partials;               // [gridDim.x][8]
+  double* partials;               // [gridDim.x][8] (sph: [nR * tiles_per_R * 4][8])
+  int ns, nnu, tiles_per_R;       // sph: node counts, super-tiles per R
+  const double *Rs, *s, *ws, *nu, *wnu;  // sph: device, [nR], [ns], [ns], [nnu], [nnu]
 };
 
 struct StepParams {
@@ -77,6 +84,8 @@ cudaError_t launch_prep(const float* theta, Wts* out, cudaStream_t st);
 // tcgen05 engine (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st);
 cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, cudaStream_t st);
+// sums the rows_per_R rows of every R in a fixed order -> out [nR][8]; a row with R <= 0 (or NaN) is all NaN
+cudaError_t launch_sph_finish(const double* partials, int nR, int rows_per_R, const double* Rs, double* out, cudaStream_t st);
 cudaError_t launch_count(const StepParams& p, unsigned long long* counts, double* weights, cudaStream_t st);
 // Data-parallel exchange fused into the reduction kernel (SURVEY.md 8e): every rank owns one exchange buffer that all
 // peers of the box can write through NVLink peer memory (cudaIpc / peer access).

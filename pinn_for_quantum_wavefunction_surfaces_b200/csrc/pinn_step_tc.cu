@@ -918,7 +918,9 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
     // quadrature 8.3e9 -> 1.03e10 points/s, same bits).  Letting the idle E-net warps also produce the geometry one tile ahead
     // (filled / consumed barriers, two buffers) is correct and SLOWER, 9.3e9: one producer warp per group with 64-bit index
     // divisions does not keep up with two MLP warps whose inference tile is short.
-    const bool enet_once = !TRAIN && p.grid.on;
+    // (the spheroidal sweep has one R per super-tile, not per CTA: there the E-net role stays in the tile loop and evaluates
+    //  E(R) and the gate per point, as in the fields mode)
+    const bool enet_once = !TRAIN && p.grid.on && !p.grid.sph;
     if (enet_once) {
       if (!IS_MLP) {
         const float Rg = (float)p.grid.R;
@@ -949,7 +951,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       Geom g;
       float cur_dx1, cur_dx2, mk_f = 0.0f;
       if (!TRAIN) {
-        const RawPt raw = p.grid.on ? tc_grid_point(p, pi) : coord_stage_read(p, cbuf, slot);
+        const RawPt raw = p.grid.on ? (p.grid.sph ? tc_sph_point(p.grid, pi) : tc_grid_point(p, pi)) : coord_stage_read(p, cbuf, slot);
         g = geom_from_raw(raw);
         cur_dx1 = raw.dx1; cur_dx2 = raw.dx2;
       } else {
@@ -1038,6 +1040,27 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       const float res = fmaf(gate, inner, fmaf(cE * E, psi, lcao));
 
       if (!TRAIN) {
+        if (p.grid.sph) {
+          // one row per warp of role 0 and super-tile (its 32 points share one R): no state carried across tiles, so the
+          // rows of one R are the same bits whatever else the launch sweeps.  Every slot is valid (padded to 128 per R).
+          if (role == 0) {
+            const double wq = sph_weight(p.grid, pidx);
+            const float hl = fmaf(-0.5f, fs, -fmaf(g.f1, g.ir2, g.f2 * g.ir1));
+            const float hpsi = fmaf(gate, fmaf(-0.5f, DN, -q * N), hl);
+            double v0 = wq * (double)(psi * hpsi), v1 = wq * (double)(psi * psi);
+            double v2 = wq * (double)(fs * hl), v3 = wq * (double)(fs * fs);
+  #pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+              v0 += __shfl_xor_sync(0xffffffffu, v0, o); v1 += __shfl_xor_sync(0xffffffffu, v1, o);
+              v2 += __shfl_xor_sync(0xffffffffu, v2, o); v3 += __shfl_xor_sync(0xffffffffu, v3, o);
+            }
+            if (lane == 0) {
+              double* row = p.grid.partials + 8 * (size_t)(st * 4 + grp);
+              row[0] = v0; row[1] = v1; row[2] = v2; row[3] = v3; row[5] = (double)E;
+            }
+          }
+          continue;
+        }
         if (p.grid.on) {
           if (valid && role == 0) {
             int ix, iy, iz;
@@ -1131,7 +1154,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(c.tbase) : "memory");
     }
     if (!TRAIN) {
-      if (p.grid.on) {  // one row of quadrature sums per CTA, fixed order
+      if (p.grid.on && !p.grid.sph) {  // one row of quadrature sums per CTA, fixed order
         double* red = reinterpret_cast<double*>(stash);
         if (role == 0) {
   #pragma unroll
@@ -1273,6 +1296,28 @@ __global__ void grid_finish_kernel(const double* __restrict__ partials, int nrow
 }
 cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, cudaStream_t st) {
   grid_finish_kernel<<<1, 32, 0, st>>>(partials, nrows, out);
+  return cudaGetLastError();
+}
+
+// one thread per (R, slot): the rows of one R added in row order (tile-major, then group), E(R) from its first row
+__global__ void sph_finish_kernel(const double* __restrict__ partials, int nR, int rows_per_R, const double* __restrict__ Rs,
+                                  double* __restrict__ out) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= 8ll * nR) return;
+  const int k = (int)(t >> 3), slot = (int)(t & 7);
+  const double* rows = partials + 8 * (size_t)k * rows_per_R;
+  double v = 0.0;
+  if (slot < 4) {
+    for (int r = 0; r < rows_per_R; r++) v += rows[8 * (size_t)r + slot];
+  } else if (slot == 5) {
+    v = rows[5];
+  }
+  if (!(Rs[k] > 0.0)) v = __longlong_as_double(0x7ff8000000000000ll);  // R <= 0 is no molecule: a NaN row, never numbers
+  out[t] = v;
+}
+cudaError_t launch_sph_finish(const double* partials, int nR, int rows_per_R, const double* Rs, double* out, cudaStream_t st) {
+  const long long n = 8ll * nR;
+  sph_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partials, nR, rows_per_R, Rs, out);
   return cudaGetLastError();
 }
 

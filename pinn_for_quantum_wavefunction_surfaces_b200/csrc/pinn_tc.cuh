@@ -200,4 +200,43 @@ __device__ __forceinline__ RawPt tc_grid_point(const StepParams& p, long long i)
   return r;
 }
 
+// Spheroidal sweep (GridDesc::sph): point i -> R index k and node indices (is, jn); pad = a slot behind the R's ns*nnu
+// nodes (it repeats the last node, so that it is finite, and gets weight 0).  The launcher keeps every index below 2^31.
+__device__ __forceinline__ void sph_index(const GridDesc& g, long long i, int& k, int& is, int& jn, bool& pad) {
+  const unsigned u = (unsigned)i, per = (unsigned)g.tiles_per_R * 128u, nn = (unsigned)(g.ns * g.nnu), nnu = (unsigned)g.nnu;
+  k = (int)(u / per);
+  unsigned l = u - (unsigned)k * per;
+  pad = l >= nn;
+  if (pad) l = nn - 1;
+  is = (int)(l / nnu);
+  jn = (int)(l - (unsigned)is * nnu);
+}
+// x = R (1 + s/R) nu, y = sqrt(s (2R + s) (1 - nu^2)), z = 0: every operation in double, rounded as written (the _rn
+// intrinsics forbid contraction into FMAs), so that a host that evaluates the same expressions gets the same points;
+// s (2R + s) is R^2 (mu^2 - 1) without the cancellation near the axis
+__device__ __forceinline__ RawPt tc_sph_point(const GridDesc& g, long long i) {
+  int k, is, jn;
+  bool pad;
+  sph_index(g, i, k, is, jn, pad);
+  const double R = g.Rs[k], s = g.s[is], nu = g.nu[jn];
+  const double x = __dmul_rn(__dmul_rn(R, __dadd_rn(1.0, __ddiv_rn(s, R))), nu);
+  RawPt r;
+  r.dx1 = (float)__dsub_rn(x, R);
+  r.dx2 = (float)__dadd_rn(x, R);
+  r.y = (float)__dsqrt_rn(__dmul_rn(__dmul_rn(s, __dadd_rn(__dmul_rn(2.0, R), s)), __dsub_rn(1.0, __dmul_rn(nu, nu))));
+  r.z = 0.0f;
+  r.R = (float)R;
+  return r;
+}
+// quadrature weight of point i: 2 pi ws wnu r1 r2 with r1 r2 = (R + s)^2 - (R nu)^2 (the volume element in (s, nu, phi)),
+// 0 for a padding slot
+__device__ __forceinline__ double sph_weight(const GridDesc& g, long long i) {
+  int k, is, jn;
+  bool pad;
+  sph_index(g, i, k, is, jn, pad);
+  const double R = g.Rs[k], s = g.s[is], nu = g.nu[jn];
+  const double rs = R + s, rn = R * nu;
+  return pad ? 0.0 : 6.283185307179586 * g.ws[is] * g.wnu[jn] * (rs * rs - rn * rn);
+}
+
 }  // namespace pinn

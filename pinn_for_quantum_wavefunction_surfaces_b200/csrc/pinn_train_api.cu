@@ -212,6 +212,40 @@ int pinn_grid_reduce(pinn_handle* h, int variant, const float* theta, int nx, in
   return 0;
 }
 
+int pinn_spheroidal_reduce(pinn_handle* h, int variant, const float* theta, int nR, const double* R, int ns, const double* s,
+                           const double* ws, int nnu, const double* nu, const double* wnu, double* out, void* stream) {
+  if (!h) return PINN_EINVAL;
+  std::lock_guard<std::mutex> lk(h->mu);
+  if (!theta || !R || !s || !ws || !nu || !wnu || !out) return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: NULL pointer argument");
+  if (nR < 1 || ns < 1 || nnu < 1) return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: nR, ns and nnu must be at least 1");
+  StepParams p{};
+  int nev = 0;
+  if (variant == PINN_VARIANT_POC) { p.vc = {1.0f, -0.5f, -1.0f, -1.0f}; nev = 2; }
+  else if (variant == PINN_VARIANT_TRAINPY) { p.vc = {2.0f, 1.0f, 1.0f, 1.0f}; nev = 1; }
+  else return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: unknown variant");
+  // every R owns whole super-tiles; the kernel's index arithmetic is 32-bit
+  const long long tiles_per_R = ((long long)ns * nnu + 127) / 128;
+  const long long tiles = tiles_per_R * nR;
+  if (tiles * 128 >= 0x80000000ll)
+    return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: nR * ceil(ns * nnu / 128) * 128 must stay below 2^31 points");
+  DevGuard dev_guard(h->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  pinn_workspace* wk = ws_for(h, st, h->sm_count);
+  if (!wk) return PINN_EINVAL;
+  if (!ws_sph_rows(h, wk, st, (int)(tiles * 4))) return PINN_EINVAL;
+  p.n = tiles * 128;
+  p.theta = theta;
+  p.grid.on = 1; p.grid.sph = 1;
+  p.grid.ns = ns; p.grid.nnu = nnu; p.grid.tiles_per_R = (int)tiles_per_R;
+  p.grid.Rs = R; p.grid.s = s; p.grid.ws = ws; p.grid.nu = nu; p.grid.wnu = wnu;
+  p.grid.partials = wk->sph_partials;
+  const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+  CU(h, launch_step_tc(nev, false, p, grid, st));
+  CU(h, launch_sph_finish(wk->sph_partials, nR, (int)tiles_per_R * 4, R, out, st));
+  h->launches += 2;
+  return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // device-resident trainer
 // ---------------------------------------------------------------------------------------------
