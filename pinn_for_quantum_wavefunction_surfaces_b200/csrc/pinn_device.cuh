@@ -330,6 +330,29 @@ __device__ __forceinline__ float2 sigm2_pre(const float2 up) {
   return make_float2(rcp_approx(d.x), rcp_approx(d.y));
 }
 
+// 1 - s of two sigmoids s = 1/(1+e) as e s.  Where s rounds next to 1 (u > 0) the difference 1 - s keeps only
+// e^u 2^-24 of relative accuracy (9e-3 at u = 12), and s(1-s), s'' and s''' inherit it; e s is accurate to a few ulps.
+// The product saturates to [0, 1] (FMUL.SAT; there is no packed form), which also turns e = inf, s = 0 (u < -88) into 0
+// rather than NaN.
+__device__ __forceinline__ float2 one_minus_sigm2(const float2 e, const float2 s) {
+  return make_float2(__saturatef(__fmul_rn(e.x, s.x)), __saturatef(__fmul_rn(e.y, s.y)));
+}
+
+// sigm2_pre, and 1 - s of both sigmoids (one_minus_sigm2)
+__device__ __forceinline__ float2 sigm2_pre(const float2 up, float2& om) {
+  const float2 e = make_float2(ex2_approx(up.x), ex2_approx(up.y));
+  const float2 d = __fadd2_rn(e, make_float2(1.0f, 1.0f));
+  const float2 s = make_float2(rcp_approx(d.x), rcp_approx(d.y));
+  om = one_minus_sigm2(e, s);
+  return s;
+}
+
+// 1 - s of sigmoids s that sigm2_pre formed earlier from the same arguments (the reverse sweeps read s back from the
+// stash and form the exponential again)
+__device__ __forceinline__ float2 one_minus_sigm2_pre(const float2 up, const float2 s) {
+  return one_minus_sigm2(make_float2(ex2_approx(up.x), ex2_approx(up.y)), s);
+}
+
 // one sigmoid whose argument already carries the factor -log2(e)
 __device__ __forceinline__ float sigm_pre(float up) { return rcp_approx(1.0f + ex2_approx(up)); }
 

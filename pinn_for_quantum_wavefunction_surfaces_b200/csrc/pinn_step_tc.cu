@@ -174,8 +174,9 @@ __device__ __forceinline__ void tc_mlp_forward(const Wts& w, TcCtx& c, uint32_t 
     for (int i = 0; i < 4; i += 2) {  // two hidden units per instruction; u = -log2(e) * pre-activation, one rounding
       const float2 u = f2fma(f2bc(a), make_float2(w0a[i], w0a[i + 1]),
                              f2fma(f2bc(b), make_float2(w1a[i], w1a[i + 1]), make_float2(b1a[i], b1a[i + 1])));
-      const float2 s = sigm2_pre(u);
-      const float2 sp = f2fma(f2neg(s), s, s);                      // s(1-s)
+      float2 om;
+      const float2 s = sigm2_pre(u, om);
+      const float2 sp = f2mul(om, s);                               // s(1-s)
       const float2 spp = f2fma(f2mul(f2bc(-2.0f), s), sp, sp);      // s'(1-2s)
       s_[k4 + i] = s.x; s_[k4 + i + 1] = s.y;
       sp_[k4 + i] = sp.x; sp_[k4 + i + 1] = sp.y;
@@ -265,8 +266,9 @@ __device__ __forceinline__ void tc_mlp_forward(const Wts& w, TcCtx& c, uint32_t 
         const float2 v3 = f2fma(f2bc(al1), v1, f2fma(f2bc(al2), v2,
                           f2fma(f2bc(al11), make_float2(P00[j], P00[j + 1]),
                                 f2fma(f2bc(al12), make_float2(P01[j], P01[j + 1]), f2mul(f2bc(al22), make_float2(P11[j], P11[j + 1]))))));
-        const float2 t = sigm2_pre(f2fma(make_float2(V0[j], V0[j + 1]), f2bc(NEG_LOG2E), make_float2(b2a[i], b2a[i + 1])));
-        const float2 tp = f2fma(f2neg(t), t, t);
+        float2 om;
+        const float2 t = sigm2_pre(f2fma(make_float2(V0[j], V0[j + 1]), f2bc(NEG_LOG2E), make_float2(b2a[i], b2a[i + 1])), om);
+        const float2 tp = f2mul(om, t);
         const float2 tpp = f2fma(f2mul(f2bc(-2.0f), t), tp, tp);
         const float2 Q = quad_form2(al11, al12, al22, v1, v2);
         const float2 gD = f2fma(tp, v3, f2mul(tpp, Q));
@@ -446,9 +448,23 @@ __device__ __forceinline__ void tc_mlp_backward(const Wts& w, TcCtx& c, uint32_t
     for (int k4 = 0; k4 < 8; k4 += 4) {
       const int kk = k8 + k4;
       const float4 sv = LD4(&Hrow[kk ^ sx]);  // h channel 0 = s_k
+      const float sa[4] = {sv.x, sv.y, sv.z, sv.w};
+      float spa[4];
+      {  // s(1-s) with 1 - s from the exponential of the forward's pre-activation (same expression, same bits), not from s
+        const float4 w0sv = LD4(&w.w0s[kk]), w1sv = LD4(&w.w1s[kk]), b1sv = LD4(&w.b1s[kk]);
+        const float w0sa[4] = {w0sv.x, w0sv.y, w0sv.z, w0sv.w}, w1sa[4] = {w1sv.x, w1sv.y, w1sv.z, w1sv.w};
+        const float b1sa[4] = {b1sv.x, b1sv.y, b1sv.z, b1sv.w};
+#pragma unroll
+        for (int i = 0; i < 4; i += 2) {
+          const float2 s = make_float2(sa[i], sa[i + 1]);
+          const float2 u = f2fma(f2bc(a), make_float2(w0sa[i], w0sa[i + 1]),
+                                 f2fma(f2bc(b), make_float2(w1sa[i], w1sa[i + 1]), make_float2(b1sa[i], b1sa[i + 1])));
+          const float2 sp = f2mul(one_minus_sigm2_pre(u, s), s);
+          spa[i] = sp.x; spa[i + 1] = sp.y;
+        }
+      }
       const float4 w0v = LD4(&w.w0[kk]), w1v = LD4(&w.w1[kk]);
       const float4 q00 = LD4(&w.ww00[kk]), q01 = LD4(&w.ww01[kk]), q11 = LD4(&w.ww11[kk]);
-      const float sa[4] = {sv.x, sv.y, sv.z, sv.w};
       const float w0a[4] = {w0v.x, w0v.y, w0v.z, w0v.w}, w1a[4] = {w1v.x, w1v.y, w1v.z, w1v.w};
       const float q00a[4] = {q00.x, q00.y, q00.z, q00.w}, q01a[4] = {q01.x, q01.y, q01.z, q01.w};
       const float q11a[4] = {q11.x, q11.y, q11.z, q11.w};
@@ -462,7 +478,7 @@ __device__ __forceinline__ void tc_mlp_backward(const Wts& w, TcCtx& c, uint32_t
         const float2 w0 = make_float2(w0a[i], w0a[i + 1]), w1 = make_float2(w1a[i], w1a[i + 1]);
         const float2 q00p = make_float2(q00a[i], q00a[i + 1]), q01p = make_float2(q01a[i], q01a[i + 1]);
         const float2 q11p = make_float2(q11a[i], q11a[i + 1]);
-        const float2 sp = f2fma(f2neg(s), s, s);
+        const float2 sp = make_float2(spa[i], spa[i + 1]);
         const float2 spp = f2fma(f2mul(f2bc(-2.0f), s), sp, sp);
         const float2 sppp = f2mul(sp, f2fma(f2bc(-6.0f), sp, f2bc(1.0f)));
         const float2 d1 = f2fma(f2bc(al1), w0, f2mul(f2bc(al2), w1));
@@ -520,9 +536,14 @@ __device__ __forceinline__ float tc_enet_forward(const Wts& w, TcCtx& c, float R
       // exponential instead of two, like the MLP roles
       const float4 wv = LD4(&w.WE1s[k16 + k4]), bv = LD4(&w.bE1s[k16 + k4]);
       // two units per instruction (FFMA2 / FADD2), the same operations and roundings as the scalar form
-      const float2 sa = sigm2_pre(f2fma(f2bc(R), make_float2(wv.x, wv.y), make_float2(bv.x, bv.y)));
-      const float2 sb = sigm2_pre(f2fma(f2bc(R), make_float2(wv.z, wv.w), make_float2(bv.z, bv.w)));
+      float2 oa, ob;
+      const float2 sa = sigm2_pre(f2fma(f2bc(R), make_float2(wv.x, wv.y), make_float2(bv.x, bv.y)), oa);
+      const float2 sb = sigm2_pre(f2fma(f2bc(R), make_float2(wv.z, wv.w), make_float2(bv.z, bv.w)), ob);
       e1[k4 + 0] = sa.x; e1[k4 + 1] = sa.y; e1[k4 + 2] = sb.x; e1[k4 + 3] = sb.y;
+      if (STASH) {  // s'(1-s) for the reverse sweep: the stash keeps e1 only
+        const float2 pa = f2mul(oa, sa), pb = f2mul(ob, sb);
+        tc_st4f(c.tlane + TC_SP_PARK + k16 + k4, pa.x, pa.y, pb.x, pb.y);
+      }
       if (STASH) ST4(&E1row[(k16 + k4) ^ sx], e1[k4], e1[k4 + 1], e1[k4 + 2], e1[k4 + 3]);
     }
     tc_st_split16<true>(t0 + E_A_HI + k16, t0 + E_A_LO + k16, e1);
@@ -560,13 +581,19 @@ __device__ __forceinline__ float tc_enet_forward(const Wts& w, TcCtx& c, float R
       float e2[4];
 #pragma unroll
       for (int i = 0; i < 4; i += 2) {
-        const float2 s2 = sigm2_pre(f2fma(make_float2(v[j4 + i], v[j4 + i + 1]), f2bc(NEG_LOG2E), make_float2(b2a[i], b2a[i + 1])));
+        float2 om;
+        const float2 s2 = sigm2_pre(f2fma(make_float2(v[j4 + i], v[j4 + i + 1]), f2bc(NEG_LOG2E), make_float2(b2a[i], b2a[i + 1])), om);
+        if (STASH) {  // v is consumed: its registers take s'(1-s) for the reverse sweep
+          const float2 sp = f2mul(om, s2);
+          v[j4 + i] = sp.x; v[j4 + i + 1] = sp.y;
+        }
         e2[i] = s2.x; e2[i + 1] = s2.y;
         E = fmaf(wEa[i], e2[i], E);
         E = fmaf(wEa[i + 1], e2[i + 1], E);
       }
       if (STASH) ST4(&Vrow[(j16 + j4) ^ sx], e2[0], e2[1], e2[2], e2[3]);
     }
+    if (STASH) tc_st16f(t0 + E_D + j16, v);  // D is dead until the reverse MMA; the stash keeps e2 only
   }
   return E;
 }
@@ -588,6 +615,7 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
   float* E1row = E1s + lane * ROWE;
   float* Vrow = Vs + lane * ROWE;
   const uint32_t t0 = c.tlane + TC_E_BASE;
+  tc_wait_st();  // the forward's s'(1-s) stores (D, TC_SP_PARK)
   __syncwarp();
   // ---- dwE[j] = sum_p Ebar_p e2[p][j] (Vs still holds e2) ----
   {
@@ -598,15 +626,16 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
   __syncwarp();
 #pragma unroll
   for (int j16 = 0; j16 < NE; j16 += 16) {
-    float vbar[16];
+    float vbar[16], sp[16];
+    tc_ld16(t0 + E_D + j16, sp);  // s'(1-s) of layer 2 as the forward formed it (1 - s = e s); D is written next by the
+    tc_wait_ld(sp);               // reverse MMA below
 #pragma unroll
     for (int j4 = 0; j4 < 16; j4 += 4) {
-      const float4 ev = LD4(&Vrow[(j16 + j4) ^ sx]), wEv = LD4(&w.wE[j16 + j4]);
-      const float ea[4] = {ev.x, ev.y, ev.z, ev.w}, wEa[4] = {wEv.x, wEv.y, wEv.z, wEv.w};
+      const float4 wEv = LD4(&w.wE[j16 + j4]);
+      const float wEa[4] = {wEv.x, wEv.y, wEv.z, wEv.w};
 #pragma unroll
       for (int i = 0; i < 4; i += 2) {
-        const float2 e = make_float2(ea[i], ea[i + 1]);
-        const float2 vb = f2mul(f2mul(f2bc(Ebar), make_float2(wEa[i], wEa[i + 1])), f2fma(f2neg(e), e, e));
+        const float2 vb = f2mul(f2mul(f2bc(Ebar), make_float2(wEa[i], wEa[i + 1])), make_float2(sp[j4 + i], sp[j4 + i + 1]));
         vbar[j4 + i] = vb.x; vbar[j4 + i + 1] = vb.y;
       }
       ST4(&Vrow[(j16 + j4) ^ sx], vbar[j4], vbar[j4 + 1], vbar[j4 + 2], vbar[j4 + 3]);
@@ -663,18 +692,16 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
   TL(11);
 #pragma unroll
   for (int k16 = 0; k16 < NE; k16 += 16) {
-    float eb[16];
+    float eb[16], sp1[16];
     tc_ld16(t0 + E_D + k16, eb);
-    tc_wait_ld(eb);
+    tc_ld16(c.tlane + TC_SP_PARK + k16, sp1);  // s'(1-s) of layer 1 as the forward formed it (1 - s = e s)
+    tc_wait_ld(eb); tc_wait_ld(sp1);
 #pragma unroll
     for (int k4 = 0; k4 < 16; k4 += 4) {
-      const float4 ev = LD4(&E1row[(k16 + k4) ^ sx]);
-      const float ea[4] = {ev.x, ev.y, ev.z, ev.w};
       float ub[4];
 #pragma unroll
       for (int i = 0; i < 4; i += 2) {
-        const float2 e = make_float2(ea[i], ea[i + 1]);
-        const float2 u = f2mul(make_float2(eb[k4 + i], eb[k4 + i + 1]), f2fma(f2neg(e), e, e));
+        const float2 u = f2mul(make_float2(eb[k4 + i], eb[k4 + i + 1]), make_float2(sp1[k4 + i], sp1[k4 + i + 1]));
         ub[i] = u.x; ub[i + 1] = u.y;
       }
       ST4(&Vrow[(k16 + k4) ^ sx], ub[0], ub[1], ub[2], ub[3]);
@@ -685,8 +712,9 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
     float ch[32];
 #pragma unroll
     for (int i = 0; i < NL; i += 2) {
-      const float2 s2 = sigm2_pre(f2fma(f2bc(R), make_float2(w.WgLs[i], w.WgLs[i + 1]), make_float2(w.bgLs[i], w.bgLs[i + 1])));
-      const float2 ub = gate_grads ? f2mul(f2mul(f2bc(gbar), make_float2(w.wg[i], w.wg[i + 1])), f2fma(f2neg(s2), s2, s2)) : f2bc(0.0f);
+      float2 om;
+      const float2 s2 = sigm2_pre(f2fma(f2bc(R), make_float2(w.WgLs[i], w.WgLs[i + 1]), make_float2(w.bgLs[i], w.bgLs[i + 1])), om);
+      const float2 ub = gate_grads ? f2mul(f2mul(f2bc(gbar), make_float2(w.wg[i], w.wg[i + 1])), f2mul(om, s2)) : f2bc(0.0f);
       const float2 ur = f2mul(ub, f2bc(R));
       const float2 gs = gate_grads ? f2mul(f2bc(gbar), s2) : f2bc(0.0f);
       ch[i] = ur.x; ch[i + 1] = ur.y;

@@ -91,6 +91,16 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, float (&v)[16]) {
 #pragma unroll
   for (int i = 0; i < 16; i++) v[i] = __uint_as_float(r[i]);
 }
+__device__ __forceinline__ void tc_st4f(uint32_t taddr, float a, float b, float c, float d) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(__float_as_uint(a)),
+               "r"(__float_as_uint(b)), "r"(__float_as_uint(c)), "r"(__float_as_uint(d)));
+}
+__device__ __forceinline__ void tc_st16f(uint32_t taddr, const float (&x)[16]) {
+  uint32_t v[16];
+#pragma unroll
+  for (int i = 0; i < 16; i++) v[i] = __float_as_uint(x[i]);
+  tc_st16(taddr, v);
+}
 __device__ __forceinline__ void tc_st8(uint32_t taddr, const uint32_t (&v)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]),
                "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]));
@@ -131,9 +141,11 @@ __device__ __forceinline__ void tc_st_split16(uint32_t t_hi, uint32_t t_lo, cons
 //   MLP role r (r = 0,1): columns [192 r, 192 r + 192)
 //     forward : A = s hi|s' hi|s'' hi|s lo|s' lo|s'' lo (6 x 16)   D = V0 (16) | V1,V2 (32) | P00,P01,P11 (48)
 //     reverse : A = vbar hi (4 x 16) | vbar lo (4 x 16)            D = hbar (4 x 16)
-//   E-net role: columns [384, 480): A = e1 / vbar hi (32) | lo (32), D (32)
+//   E-net role: columns [384, 480): A = e1 / vbar hi (32) | lo (32), D (32); between the forward's read of D and the
+//               reverse MMA, D holds s'(1-s) of layer 2 for the reverse sweep
+//   E-net role, forward to reverse: columns [480, 512): s'(1-s) of layer 1 for the reverse sweep
 // ---------------------------------------------------------------------------------------------
-constexpr uint32_t TC_MLP_COLS = 192, TC_E_BASE = 384;
+constexpr uint32_t TC_MLP_COLS = 192, TC_E_BASE = 384, TC_SP_PARK = 480;
 constexpr uint32_t F_S_HI = 0, F_SP_HI = 16, F_SPP_HI = 32, F_S_LO = 48, F_SP_LO = 64, F_SPP_LO = 80;
 constexpr uint32_t F_V0 = 96, F_V12 = 112, F_P = 144;
 constexpr uint32_t B_VB_HI = 0, B_VB_LO = 64, B_HB = 128;
