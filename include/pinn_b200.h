@@ -77,9 +77,9 @@ const char* pinn_last_error(pinn_handle* h);
 int64_t pinn_launch_count(pinn_handle* h);
 
 /* The library carries ONE implementation of the fused step kernel, PINN_ENGINE_TCGEN05 (skinny mat-vecs as M=128 TF32
- * tcgen05.mma with activations in tensor memory, 3xTF32); pinn_set_engine(PINN_ENGINE_FFMA) returns PINN_ENOTSUP.  The
- * FFMA engine (the same mat-vecs as FFMA chains, the round-1 baseline of DESIGN.md section 3) only exists in the separate
- * A/B build made by tools/build_ab.sh (-DPINN_AB_BUILD), where the two calls below - and nothing else - select it. */
+ * tcgen05.mma with activations in tensor memory, 3xTF32).  pinn_set_engine returns 0 for PINN_ENGINE_TCGEN05,
+ * PINN_ENOTSUP for PINN_ENGINE_FFMA (the round-1 engine of DESIGN.md section 3, no longer part of the library) and
+ * PINN_EINVAL for any other value; pinn_get_engine returns PINN_ENGINE_TCGEN05. */
 #define PINN_ENGINE_FFMA 0
 #define PINN_ENGINE_TCGEN05 1
 int pinn_set_engine(pinn_handle* h, int engine);

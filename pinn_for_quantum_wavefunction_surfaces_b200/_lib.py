@@ -199,7 +199,7 @@ class Handle:
     ENGINES = {"ffma": 0, "tcgen05": 1}
 
     def set_engine(self, name):
-        """'tcgen05' (default) or 'ffma': which implementation of the fused step kernel runs."""
+        """'tcgen05', the one implementation of the fused step kernel the library carries; 'ffma' raises PinnError."""
         self.check(self.L.pinn_set_engine(self.h, self.ENGINES[name]), "pinn_set_engine")
 
     def get_engine(self):

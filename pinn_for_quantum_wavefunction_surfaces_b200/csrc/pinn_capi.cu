@@ -1,7 +1,6 @@
 // C ABI of the PINN hot path (see include/pinn_b200.h for the contract).
 #include <chrono>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -11,10 +10,6 @@
 #include "pinn_train.h"
 
 std::string g_create_err;
-
-// upload block of the *_host entry: theta as float (padded to 1536) followed by the 3 loss weights
-constexpr int HOST_IN_THETA = 1536;
-constexpr size_t HOST_IN_BYTES = HOST_IN_THETA * sizeof(float) + 4 * sizeof(double);
 
 static const int kOffsets[17] = {O_W1, O_B1, O_W2, O_B2, O_WO, O_BO, O_WE1, O_BE1, O_WE2, O_BE2, O_WE, O_BE,
                                  O_WGL, O_BGL, O_WG, O_BG, NTHETA};
@@ -50,25 +45,12 @@ int pinn_create(int device, pinn_handle** out) {
   pinn_handle* h = new pinn_handle();
   h->device = device;
   h->sm_count = prop.multiProcessorCount;
-#ifdef PINN_AB_BUILD  // A/B builds only (tools/build_ab.sh): the product has one engine and reads no environment
-  if (const char* e = getenv("PINN_B200_ENGINE")) {
-    if (!strcmp(e, "ffma")) h->engine = PINN_ENGINE_FFMA;
-    else if (!strcmp(e, "tcgen05")) h->engine = PINN_ENGINE_TCGEN05;
-  }
-  if (const char* e = getenv("PINN_B200_HOST_ZEROCOPY")) h->host_zero_copy = strcmp(e, "0") != 0;
-  if (const char* e = getenv("PINN_B200_HOST_INLINE")) h->host_inline_params = strcmp(e, "0") != 0;
-  CREATE_CU(cudaMalloc(&h->wts, sizeof(Wts)));
-#endif
-  // theta (1536 float) and the 3 loss weights share one block so that the *_host entry uploads both with one copy
-  CREATE_CU(cudaMalloc(&h->theta_dev, HOST_IN_BYTES));
-  h->weights_dev = reinterpret_cast<double*>(h->theta_dev + HOST_IN_THETA);
+  CREATE_CU(cudaMalloc(&h->theta_dev, NTHETA * sizeof(float)));
   CREATE_CU(cudaHostAlloc(&h->out_pinned, NPART * sizeof(double), cudaHostAllocMapped));
   CREATE_CU(cudaHostGetDevicePointer(&h->out_mapped, h->out_pinned, 0));
-  CREATE_CU(cudaMallocHost(&h->theta_pinned, HOST_IN_BYTES));
-  h->weights_pinned = reinterpret_cast<double*>(h->theta_pinned + HOST_IN_THETA);
+  CREATE_CU(cudaMallocHost(&h->theta_pinned, NTHETA * sizeof(float)));
   CREATE_CU(cudaStreamCreateWithFlags(&h->s_copy, cudaStreamNonBlocking));
   CREATE_CU(cudaStreamCreateWithFlags(&h->s_main, cudaStreamNonBlocking));
-  CREATE_CU(cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
   for (int c = 0; c < 4; c++) CREATE_CU(cudaEventCreateWithFlags(&h->ev_chunk[c], cudaEventDisableTiming));
   // the workspace of the *_host entry's stream holds the rows of up to 4 chunk launches
   if (!ws_for(h, h->s_main, 4 * h->sm_count)) {
@@ -224,15 +206,11 @@ int pinn_destroy(pinn_handle* h) {
   DevGuard dev_guard(h->device);
   dp_release(h);
   cudaDeviceSynchronize();
-#ifdef PINN_AB_BUILD
-  cudaFree(h->wts);
-#endif
   for (pinn_workspace& w : h->ws) ws_free(w);
   cudaFree(h->theta_dev); cudaFree(h->stage_dev);
   cudaFreeHost(h->out_pinned); cudaFreeHost(h->theta_pinned);
   if (h->s_copy) cudaStreamDestroy(h->s_copy);
   if (h->s_main) cudaStreamDestroy(h->s_main);
-  if (h->ev_copy) cudaEventDestroy(h->ev_copy);
   for (int c = 0; c < 4; c++) if (h->ev_chunk[c]) cudaEventDestroy(h->ev_chunk[c]);
   for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
   delete h;
@@ -244,16 +222,12 @@ int64_t pinn_launch_count(pinn_handle* h) { return h ? h->launches : 0; }
 
 int pinn_set_engine(pinn_handle* h, int engine) {
   if (!h) return PINN_EINVAL;
+  if (engine == PINN_ENGINE_TCGEN05) return 0;
   std::lock_guard<std::mutex> lk(h->mu);
-  if (engine != PINN_ENGINE_FFMA && engine != PINN_ENGINE_TCGEN05) return fail(h, PINN_EINVAL, "pinn_set_engine: unknown engine");
-#ifndef PINN_AB_BUILD
-  if (engine != PINN_ENGINE_TCGEN05)
-    return fail(h, PINN_ENOTSUP, "pinn_set_engine: this library carries the tcgen05 engine only (the FFMA engine exists in A/B builds, tools/build_ab.sh)");
-#endif
-  h->engine = engine;
-  return 0;
+  if (engine == PINN_ENGINE_FFMA) return fail(h, PINN_ENOTSUP, "pinn_set_engine: this library carries the tcgen05 engine only");
+  return fail(h, PINN_EINVAL, "pinn_set_engine: unknown engine");
 }
-int pinn_get_engine(pinn_handle* h) { return h ? h->engine : PINN_EINVAL; }
+int pinn_get_engine(pinn_handle* h) { return h ? PINN_ENGINE_TCGEN05 : PINN_EINVAL; }
 
 int pinn_host_timing(pinn_handle* h, double* out4) {
   if (!h || !out4) return PINN_EINVAL;
@@ -405,41 +379,6 @@ int pinn_dp_shutdown(pinn_handle* h) {
   return 0;
 }
 
-static int variant_coef(int variant, VariantCoef* vc, int* nev) {
-  if (variant == PINN_VARIANT_POC) { *vc = {1.0f, -0.5f, -1.0f, -1.0f}; *nev = 2; return 0; }
-  if (variant == PINN_VARIANT_TRAINPY) { *vc = {2.0f, 1.0f, 1.0f, 1.0f}; *nev = 1; return 0; }
-  return PINN_EINVAL;
-}
-
-static int grid_for(pinn_handle* h, long long n) {
-  // one persistent CTA per SM; a CTA works on super-tiles of 128 points
-  const long long want = (n + 127) / 128;
-  return (int)(want < h->sm_count ? (want < 1 ? 1 : want) : h->sm_count);
-}
-
-// The step kernel builds its operand images from p.theta itself (A/B builds: the FFMA engine reads an image prepared by
-// a small kernel).
-static int enqueue_prep(pinn_handle* h, const float* theta, StepParams& p, cudaStream_t st) {
-  p.theta = theta;
-#ifdef PINN_AB_BUILD
-  p.wts = h->wts;
-  if (h->engine == PINN_ENGINE_TCGEN05) return 0;
-  CU(h, launch_prep(theta, h->wts, st));
-  h->launches++;
-#else
-  (void)st;
-#endif
-  return 0;
-}
-
-static cudaError_t launch_step_any(pinn_handle* h, int nev, bool train, const StepParams& p, int grid, cudaStream_t st) {
-#ifdef PINN_AB_BUILD
-  if (h->engine != PINN_ENGINE_TCGEN05) return launch_step(nev, train, p, grid, st);
-#endif
-  (void)h;
-  return launch_step_tc(nev, train, p, grid, st);
-}
-
 // Enqueue the fused step kernel for points [first, first + cnt) of a batch; its per-CTA rows go to partial rows
 // [row0, row0 + *rows).  The handle mutex is held by the caller.
 static int enqueue_step_chunk(pinn_handle* h, pinn_workspace* ws, int nev, StepParams p, int64_t first, int64_t cnt, int row0,
@@ -464,17 +403,17 @@ static int enqueue_step_chunk(pinn_handle* h, pinn_workspace* ws, int nev, StepP
     e1 = h->ev_pool[h->ev_used++];
     CU(h, cudaEventRecord(e0, st));
   }
-  CU(h, launch_step_any(h, nev, true, p, grid, st));
+  CU(h, launch_step_tc(nev, true, p, grid, st));
   if (e1) CU(h, cudaEventRecord(e1, st));
   h->launches++;
   *rows = grid;
   return 0;
 }
 
-// The training evaluation on device buffers.  theta / weights: device pointers, or (tcgen05 engine, used by the *_host
-// entry) NULL with theta_inline / weights_inline = HOST arrays that travel inside the kernel parameters.
 }  // extern "C"
 
+// The training evaluation on device buffers (or mapped page-locked columns): the set-count kernels when no loss weights
+// are given, one step launch per chunk of the plan, one reduction over the partial rows of all chunks.
 int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
   std::lock_guard<std::mutex> lk(h->mu);
   StepParams p{};
@@ -484,28 +423,26 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
   if (!c.x || !c.y || !c.z || !c.R || (!c.theta && !c.theta_inline && !c.theta_tensors) || !c.sums || !c.dtheta)
     return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: NULL pointer argument");
   if (c.in_dtype != PINN_F32 && c.in_dtype != PINN_F64) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: bad in_dtype");
+  const int nchunk = c.nchunk ? c.nchunk : 1;
   DevGuard dev_guard(h->device);
-  pinn_workspace* ws = ws_for(h, st, h->sm_count);
+  pinn_workspace* ws = ws_for(h, st, nchunk * h->sm_count);
   if (!ws) return PINN_EINVAL;
   if (int rc = dp_serialize(h, st)) return rc;
   p.x = c.x; p.y = c.y; p.z = c.z; p.R = c.R; p.mask = c.mask; p.n = c.n; p.in_f64 = c.in_dtype == PINN_F64;
-  p.bcut = c.bcutoff; p.partials = ws->partials; p.E_out = static_cast<float*>(c.E_out); p.E_f64 = c.E_f64;
+  p.bcut = c.bcutoff; p.E_out = static_cast<float*>(c.E_out); p.E_f64 = c.E_f64;
   p.base_grads = (c.grad_mask & 0x003Fu) != 0;
   p.gate_grads = (c.grad_mask & 0xF000u) != 0;
   const double* weights = c.weights;
   if (c.theta_inline) {
     p.theta_inline = c.theta_inline;
   } else if (c.theta_tensors) {
-#ifdef PINN_AB_BUILD
-    if (h->engine != PINN_ENGINE_TCGEN05) return fail(h, PINN_ENOTSUP, "the FFMA engine takes a packed theta only");
-#endif
     for (int k = 0; k < 16; k++) {
       if (!c.theta_tensors[k]) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd_tensors: NULL parameter tensor");
       p.theta_tensors[k] = c.theta_tensors[k];
     }
     p.theta_from_tensors = 1; p.tensors_f64 = c.tensors_f64; p.tensors_in_out = c.tensors_in_out;
   } else {
-    if (int rc = enqueue_prep(h, c.theta, p, st)) return rc;
+    p.theta = c.theta;
   }
   if (c.weights_inline) {
     p.weights_inline = c.weights_inline;
@@ -515,10 +452,15 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
     weights = ws->weights;
   }
   p.weights = weights;
-  int grid = 0;
-  int rc = enqueue_step_chunk(h, ws, nev, p, 0, c.n, 0, &grid, st);
-  if (rc) return rc;
-  CU(h, launch_reduce(ws->partials, grid, weights, c.weights_inline, c.grad_mask, c.dtheta, c.sums, p.E_out, c.n,
+  int rows = 0;
+  for (int k = 0; k < nchunk; k++) {
+    const LossCall::Chunk ck = c.nchunk ? c.chunk[k] : LossCall::Chunk{0, c.n, nullptr};
+    if (ck.ready) CU(h, cudaStreamWaitEvent(st, ck.ready, 0));
+    int r = 0;
+    if (int rc = enqueue_step_chunk(h, ws, nev, p, ck.first, ck.count, rows, &r, st)) return rc;
+    rows += r;
+  }
+  CU(h, launch_reduce(ws->partials, rows, weights, c.weights_inline, c.grad_mask, c.dtheta, c.sums, p.E_out, c.n,
                       h->dp_on ? h->dp : DpArgs(), st, c.adam, c.adam_ticket, c.presample, c.E_f64, c.dtheta_in_out));
   h->launches++;
   return 0;
@@ -586,9 +528,8 @@ int pinn_fields(pinn_handle* h, int variant, int64_t n, const void* x, const voi
   DevGuard dev_guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   p.x = x; p.y = y; p.z = z; p.R = R; p.n = n; p.in_f64 = in_dtype == PINN_F64;
-  p.psi = psi; p.lap = lap; p.hpsi = hpsi; p.res = res; p.E_out = E;
-  if (int rc = enqueue_prep(h, theta, p, st)) return rc;
-  CU(h, launch_step_any(h, nev, false, p, grid_for(h, n), st));
+  p.psi = psi; p.lap = lap; p.hpsi = hpsi; p.res = res; p.E_out = E; p.theta = theta;
+  CU(h, launch_step_tc(nev, false, p, grid_for(h, n), st));
   h->launches++;
   return 0;
 }
@@ -611,7 +552,7 @@ int pinn_loss_fwd_bwd_host(pinn_handle* h, int variant, int64_t n, const void* x
   // step kernel requests the coordinates of its next super-tile one tile ahead, which hides the PCIe latency, and
   // the 16 B/point crossing the bus overlap the whole kernel instead of preceding it.  Pageable inputs are staged.
   const void* mapped[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-  const bool zero_copy = h->host_zero_copy && map_pinned(x, &mapped[0]) && map_pinned(y, &mapped[1]) &&
+  const bool zero_copy = map_pinned(x, &mapped[0]) && map_pinned(y, &mapped[1]) &&
                          map_pinned(z, &mapped[2]) && map_pinned(R, &mapped[3]) && (!mask || map_pinned(mask, &mapped[4]));
   const size_t col = zero_copy ? 0 : ((size_t)n * es + 255) & ~(size_t)255;
   const size_t mcol = zero_copy ? 0 : ((size_t)n + 255) & ~(size_t)255;
@@ -631,92 +572,55 @@ int pinn_loss_fwd_bwd_host(pinn_handle* h, int variant, int64_t n, const void* x
   char* base = (char*)h->stage_dev;
   cudaStream_t st = h->s_main;
   for (int i = 0; i < NTHETA; i++) h->theta_pinned[i] = (float)theta_host[i];
-  const double* wdev = nullptr;
-  if (weights_host) {
-    memcpy(h->weights_pinned, weights_host, 3 * sizeof(double));
-    wdev = h->weights_dev;
-  }
-  // tcgen05 engine with known weights: theta and the weights ride in the kernel parameters, nothing is uploaded first
-  const bool inline_params = weights_host && h->engine == PINN_ENGINE_TCGEN05 && h->host_inline_params;
-  if (!inline_params)
-    CU(h, cudaMemcpyAsync(h->theta_dev, h->theta_pinned, weights_host ? HOST_IN_BYTES : NTHETA * sizeof(float),
-                          cudaMemcpyHostToDevice, st));
-  const float* th_dev = inline_params ? nullptr : h->theta_dev;
-  const float* th_inl = inline_params ? h->theta_pinned : nullptr;
-  const double* w_inl = inline_params ? h->weights_pinned : nullptr;
-  if (inline_params) wdev = nullptr;
-  // the 8 sums and 1521 gradients are written by the reduction kernel straight into mapped page-locked memory
-  double* outp = h->out_mapped;
-  uint8_t* mdev = mask ? (uint8_t*)(base + 4 * col) : nullptr;
   float* edev = (float*)(base + 4 * col + mcol);
-  // With the weights known up front the batch is processed in up to 4 chunks so that the copy of chunk k+1 (copy stream)
-  // overlaps the kernel of chunk k.  Chunks are whole rounds of super-tiles (sm_count x 128 points) so that no launch
-  // ends on a partial wave; the first chunk is short (2 rounds) to start computing early.
-  // Without weights the set sizes must be counted over the whole batch first: one chunk.
-  const int64_t unit = (int64_t)h->sm_count * 128;
-  const int64_t rounds = (n + unit - 1) / unit;
-  int nchunk = 1;
-  int64_t first[4] = {0, 0, 0, 0}, cnt[4] = {n, 0, 0, 0};
-  if (weights_host && rounds >= 8) {
-    nchunk = 4;
-    const int64_t rest = rounds - 2;
-    const int64_t r[4] = {2, rest / 3, rest / 3, rest - 2 * (rest / 3)};
-    int64_t at = 0;
-    for (int c = 0; c < 4; c++) {
-      first[c] = at;
-      cnt[c] = (c == 3) ? n - at : r[c] * unit;
-      at += cnt[c];
-    }
-  }
-  if (zero_copy) nchunk = 1;
-  const void* src[4] = {x, y, z, R};
-  for (int c = 0; c < nchunk && !zero_copy; c++) {
-    cudaStream_t sc = nchunk == 1 ? st : h->s_copy;
-    for (int k = 0; k < 4; k++)
-      CU(h, cudaMemcpyAsync(base + k * col + first[c] * es, (const char*)src[k] + first[c] * es, (size_t)cnt[c] * es,
-                            cudaMemcpyHostToDevice, sc));
-    if (mask) CU(h, cudaMemcpyAsync(mdev + first[c], mask + first[c], (size_t)cnt[c], cudaMemcpyHostToDevice, sc));
-    if (nchunk > 1) CU(h, cudaEventRecord(h->ev_chunk[c], sc));
+  LossCall c;
+  c.variant = variant; c.n = n; c.in_dtype = in_dtype; c.grad_mask = grad_mask; c.bcutoff = bcutoff; c.E_out = edev;
+  // the 8 sums and 1521 gradients are written by the reduction kernel straight into mapped page-locked memory
+  c.sums = h->out_mapped; c.dtheta = h->out_mapped + 8;
+  // With known weights theta and the weights ride in the kernel parameters and nothing is uploaded first.  Without them
+  // theta is uploaded, and the set sizes are counted on the device.
+  if (weights_host) {
+    c.theta_inline = h->theta_pinned;
+    c.weights_inline = weights_host;
+  } else {
+    CU(h, cudaMemcpyAsync(h->theta_dev, h->theta_pinned, NTHETA * sizeof(float), cudaMemcpyHostToDevice, st));
+    c.theta = h->theta_dev;
   }
   if (zero_copy) {
-    LossCall c;
-    c.variant = variant; c.n = n; c.x = mapped[0]; c.y = mapped[1]; c.z = mapped[2]; c.R = mapped[3]; c.in_dtype = in_dtype;
-    c.mask = (const uint8_t*)mapped[4]; c.theta = th_dev; c.weights = wdev; c.theta_inline = th_inl; c.weights_inline = w_inl;
-    c.grad_mask = grad_mask; c.bcutoff = bcutoff; c.sums = outp; c.dtheta = outp + 8; c.E_out = edev;
-    int rc = loss_fwd_bwd_impl(h, c, st);
-    if (rc) return rc;
-  } else if (nchunk == 1) {
-    LossCall c;
-    c.variant = variant; c.n = n; c.x = base; c.y = base + col; c.z = base + 2 * col; c.R = base + 3 * col; c.in_dtype = in_dtype;
-    c.mask = mdev; c.theta = th_dev; c.weights = wdev; c.theta_inline = th_inl; c.weights_inline = w_inl;
-    c.grad_mask = grad_mask; c.bcutoff = bcutoff; c.sums = outp; c.dtheta = outp + 8; c.E_out = edev;
-    int rc = loss_fwd_bwd_impl(h, c, st);
-    if (rc) return rc;
+    c.x = mapped[0]; c.y = mapped[1]; c.z = mapped[2]; c.R = mapped[3]; c.mask = (const uint8_t*)mapped[4];
   } else {
-    std::lock_guard<std::mutex> lk(h->mu);
-    StepParams p{};
-    int nev = 0;
-    if (variant_coef(variant, &p.vc, &nev)) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd_host: unknown variant");
-    pinn_workspace* ws = ws_for(h, st, 4 * h->sm_count);
-    if (!ws) return PINN_EINVAL;
-    if (int rc = dp_serialize(h, st)) return rc;
-    p.x = base; p.y = base + col; p.z = base + 2 * col; p.R = base + 3 * col; p.mask = mdev;
-    p.in_f64 = in_dtype == PINN_F64; p.bcut = bcutoff; p.E_out = edev; p.weights = wdev;
-    p.base_grads = (grad_mask & 0x003Fu) != 0;
-    p.gate_grads = (grad_mask & 0xF000u) != 0;
-    if (inline_params) { p.theta_inline = th_inl; p.weights_inline = w_inl; }
-    else if (int rc = enqueue_prep(h, h->theta_dev, p, st)) return rc;
-    int rows = 0;
-    for (int c = 0; c < nchunk; c++) {
-      CU(h, cudaStreamWaitEvent(st, h->ev_chunk[c], 0));
-      int r = 0;
-      int rc = enqueue_step_chunk(h, ws, nev, p, first[c], cnt[c], rows, &r, st);
-      if (rc) return rc;
-      rows += r;
+    uint8_t* mdev = mask ? (uint8_t*)(base + 4 * col) : nullptr;
+    c.x = base; c.y = base + col; c.z = base + 2 * col; c.R = base + 3 * col; c.mask = mdev;
+    // With the weights known up front the batch is processed in 4 chunks so that the copy of chunk k+1 (copy stream)
+    // overlaps the kernel of chunk k.  Chunks are whole rounds of super-tiles (sm_count x 128 points) so that no launch
+    // ends on a partial wave; the first chunk is short (2 rounds) to start computing early.
+    // Without weights the set sizes must be counted over the whole batch first: one chunk, copied on the main stream.
+    const int64_t unit = (int64_t)h->sm_count * 128;
+    const int64_t rounds = (n + unit - 1) / unit;
+    c.nchunk = 1;
+    c.chunk[0] = {0, n, nullptr};
+    if (weights_host && rounds >= 8) {
+      c.nchunk = 4;
+      const int64_t rest = rounds - 2;
+      const int64_t r[4] = {2, rest / 3, rest / 3, rest - 2 * (rest / 3)};
+      int64_t at = 0;
+      for (int k = 0; k < 4; k++) {
+        c.chunk[k] = {at, k == 3 ? n - at : r[k] * unit, h->ev_chunk[k]};
+        at += c.chunk[k].count;
+      }
     }
-    CU(h, launch_reduce(ws->partials, rows, wdev, w_inl, grad_mask, outp + 8, outp, edev, n, h->dp_on ? h->dp : DpArgs(), st));
-    h->launches++;
+    const void* src[4] = {x, y, z, R};
+    for (int k = 0; k < c.nchunk; k++) {
+      const LossCall::Chunk& ck = c.chunk[k];
+      cudaStream_t sc = ck.ready ? h->s_copy : st;
+      for (int j = 0; j < 4; j++)
+        CU(h, cudaMemcpyAsync(base + j * col + ck.first * es, (const char*)src[j] + ck.first * es, (size_t)ck.count * es,
+                              cudaMemcpyHostToDevice, sc));
+      if (mask) CU(h, cudaMemcpyAsync(mdev + ck.first, mask + ck.first, (size_t)ck.count, cudaMemcpyHostToDevice, sc));
+      if (ck.ready) CU(h, cudaEventRecord(ck.ready, sc));
+    }
   }
+  if (int rc = loss_fwd_bwd_impl(h, c, st)) return rc;
   if (E_out_host) CU(h, cudaMemcpyAsync(E_out_host, edev, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
   const auto t_submitted = std::chrono::steady_clock::now();
   CU(h, cudaStreamSynchronize(st));

@@ -21,8 +21,8 @@ enum : int {
   S_RES2 = 1521, S_PSI1 = 1522, S_PSI2 = 1523, S_E = 1524, S_CNT1 = 1525, S_CNT2 = 1526
 };
 
-// Weights as the kernels want them, built once per step by prep_weights_kernel and
-// bulk-copied (TMA, cp.async.bulk) into shared memory by every CTA.
+// Weights as the step kernel wants them: every CTA builds this image in its shared memory from theta
+// (build_weight_image, pinn_device.cuh).
 struct alignas(128) Wts {
   float w0[NH], w1[NH], b1[NH];          // W1[:,0], W1[:,1], b1
   float ww00[NH], ww01[NH], ww11[NH];    // w0^2, w0*w1, w1^2  (second-order channel)
@@ -42,19 +42,15 @@ struct alignas(128) Wts {
   float BWT[2][NH * NH];                 // n = k        : W2[j][k], K index = j          (reverse sweep)
   float BE[2][NE * NE];                  // n = j        : WE2[j][k]
   float BET[2][NE * NE];                 // n = k        : WE2[j][k], K index = j
-  // ---- FFMA engine only (pinn_kernels.cu); the tcgen05 kernel does not stage these ----
-  float W2[NH * NH];                     // [j][k]  forward rows
-  float W2T[NH * NH];                    // [k][j]  reverse-sweep rows
-  float WE2[NE * NE];                    // [j][k]
-  float WE2T[NE * NE];                   // [k][j]
 };
 // offset (floats) of element (n,k) of an N x K operand in the canonical K-major no-swizzle layout:
 // 16-byte K chunks strided by LBO = 128*(N/8) bytes, 8-row groups strided by SBO = 128 bytes
 __host__ __device__ constexpr int umma_off(int n, int k, int N) {
   return (k / 4) * (32 * (N / 8)) + (n / 8) * 32 + (n % 8) * 4 + (k % 4);
 }
-static_assert(sizeof(Wts) % 16 == 0, "Wts must be a multiple of 16 bytes for cp.async.bulk");
-static_assert(offsetof(Wts, BS) % 128 == 0 && offsetof(Wts, W2) % 16 == 0, "operand images must stay aligned");
+static_assert(sizeof(Wts) == 32640, "Wts: 480 layer floats + the six hi/lo operand images");
+static_assert(offsetof(Wts, BS) % 128 == 0 && sizeof(Wts) % 128 == 0,
+              "operand images and the shared-memory buffers behind the image must stay aligned");
 
 // entry i of the canonical theta -> index inside ITS tensor when that tensor is stored in train.py's (in,out) layout
 // (x @ A + b, train.py:4-5) instead of nn.Linear's (out,in); only W1 (16,2), W2 (16,16) and WE2 (32,32) differ
@@ -75,10 +71,5 @@ __host__ __device__ inline void theta_locate(int i, int& k, int& off) {
 struct VariantCoef {  // res = cL*lap(psi) + cV*(1/r1+1/r2)*psi + cE*E*psi ; N = sN * sum(evals) + bo
   float sN, cL, cV, cE;
 };
-
-__device__ __forceinline__ float sigmoidf_fast(float u) {
-  // 1/(1+exp(-u)) with MUFU.EX2 + MUFU.RCP (approx, ~2 ulp); saturates correctly at +-inf
-  return __frcp_rn(1.0f + __expf(-u)) ;
-}
 
 }  // namespace pinn

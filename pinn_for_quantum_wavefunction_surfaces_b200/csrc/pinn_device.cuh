@@ -1,4 +1,4 @@
-// Device helpers shared by the FFMA step kernel (pinn_kernels.cu) and the tcgen05 step kernel (pinn_step_tc.cu).
+// Device helpers of the tcgen05 step kernel (pinn_step_tc.cu) and the kernels around it (pinn_reduce.cu, pinn_train.cu).
 #pragma once
 #include "pinn_common.cuh"
 #include "pinn_launch.h"
@@ -7,19 +7,17 @@ namespace pinn {
 
 // Per-point stash rows live in shared memory, one row per lane (= point): 64 floats for an MLP warp
 // (4 Taylor channels x 16), 32 for the E-net warp.  Rows are NOT padded; instead the column index is
-// XOR-swizzled with 8*(row&3), which makes the mma fragment loads (rows t / t+4, columns g / g+8)
-// conflict free and keeps float4 groups intact.
+// XOR-swizzled (swz_tc), which keeps float4 groups intact.
 constexpr int ROWH = 64;
 constexpr int ROWE = 32;
 constexpr int EVAL_STASH = 2 * 32 * ROWH;  // floats: Hs + Gs
 constexpr int ENET_STASH = 2 * 32 * ROWE;  // floats: E1s + Vs
 
-__device__ __forceinline__ int swz(int row) { return (row & 3) << 3; }
-// Swizzle of the tcgen05 engine's stash (pinn_step_tc.cu): the 16-byte chunk index of a row is XOR-ed with
+// Swizzle of the stash: the 16-byte chunk index of a row is XOR-ed with
 // s(row) = ((row & 3) << 1) | ((row >> 2) & 1).  Eight consecutive rows get eight different values, so the 128-bit
 // accesses of a row by its own lane (quarter-warp = 8 lanes per phase) are conflict-free, and rows r, r+1, r+2, r+3 differ
 // in the upper two bits, which keeps the scalar mma.sync fragment loads (8 columns x 4 rows per instruction)
-// conflict-free as with swz().  Returned in floats (multiple of 4).
+// conflict-free.  Returned in floats (multiple of 4).
 __host__ __device__ constexpr int swz_tc(int row) { return ((((row & 3) << 1) | ((row >> 2) & 1)) << 2); }
 
 // ---------------------------------------------------------------------------------------------
@@ -30,14 +28,6 @@ __device__ __forceinline__ float rcp_approx(float x) {
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
 }
-// sigmoid = 1 / (1 + 2^(-u log2 e)): FMUL + MUFU.EX2 + FADD + MUFU.RCP (the .ftz forms skip the denormal fix-up code;
-// saturates to 0 / 1 for large |u|)
-__device__ __forceinline__ float sigm(float u) {
-  float e;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(u * -1.4426950408889634f));
-  return rcp_approx(1.0f + e);
-}
-
 constexpr float NEG_LOG2E = -1.4426950408889634f;
 __device__ __forceinline__ float ex2_approx(float x) {
   float e;
@@ -53,7 +43,7 @@ __device__ __forceinline__ void named_barrier(int id, int nthreads) {
 
 // 3xTF32: x = hi + lo.  The tensor cores read the upper 19 bits of an fp32 operand (they truncate; measured with
 // tools/microbench/umma_ts.cu).
-//  * weights (split once per step by prep_weights_kernel): split_tf32_rn - hi is x ROUNDED to nearest TF32 (add half an
+//  * weights (split once per CTA by build_weight_image): split_tf32_rn - hi is x ROUNDED to nearest TF32 (add half an
 //    ulp, clear the low 13 bits), lo = x - hi is exact in fp32 and gets half an ulp added so that the hardware truncation
 //    rounds it to nearest as well: |lo| <= 2^-11 |x| with random sign.
 //  * forward-sweep activations: split_tf32_rn3 - the same rounded hi, lo = x - hi left as it is (three instructions): the
@@ -89,43 +79,6 @@ __device__ __forceinline__ void mma_3xtf32(float (&c)[4], const uint32_t (&ah)[4
   mma_tf32(c, ah, bh0, bh1);
 }
 
-// Column sum over the 32 rows (points) of a swizzled stash: lane sums column `col`.
-template <int ROW>
-__device__ __forceinline__ float colsum(const float* __restrict__ base, int col) {
-  // four row-phase pointers (the swizzle depends on row & 3 only); fully unrolled so that every load is
-  // [pointer + immediate] and no per-row address arithmetic is left
-  const float* p0 = base + col;
-  const float* p1 = base + ROW + (col ^ 8);
-  const float* p2 = base + 2 * ROW + (col ^ 16);
-  const float* p3 = base + 3 * ROW + (col ^ 24);
-  float s0 = 0.0f, s1 = 0.0f, s2 = 0.0f, s3 = 0.0f;
-#pragma unroll
-  for (int p = 0; p < 32; p += 4) {
-    s0 += p0[p * ROW]; s1 += p1[p * ROW]; s2 += p2[p * ROW]; s3 += p3[p * ROW];
-  }
-  return (s0 + s1) + (s2 + s3);
-}
-// Weighted column sums: returns sum_p base[p][col] and sum_p wgt_p * base[p][col] (wgt = per-lane value of row p)
-template <int ROW>
-__device__ __forceinline__ void colsum_w(const float* __restrict__ base, int col, float wgt, float& plain, float& weighted) {
-  const float* p0 = base + col;
-  const float* p1 = base + ROW + (col ^ 8);
-  const float* p2 = base + 2 * ROW + (col ^ 16);
-  const float* p3 = base + 3 * ROW + (col ^ 24);
-  float s0 = 0.0f, s1 = 0.0f, t0 = 0.0f, t1 = 0.0f;
-#pragma unroll
-  for (int p = 0; p < 32; p += 4) {
-    const float v0 = p0[p * ROW], v1 = p1[p * ROW], v2 = p2[p * ROW], v3 = p3[p * ROW];
-    s0 += v0; s1 += v1; s0 += v2; s1 += v3;
-    t0 = fmaf(__shfl_sync(0xffffffffu, wgt, p + 0), v0, t0);
-    t1 = fmaf(__shfl_sync(0xffffffffu, wgt, p + 1), v1, t1);
-    t0 = fmaf(__shfl_sync(0xffffffffu, wgt, p + 2), v2, t0);
-    t1 = fmaf(__shfl_sync(0xffffffffu, wgt, p + 3), v3, t1);
-  }
-  plain = s0 + s1;
-  weighted = t0 + t1;
-}
-
 // packed float32x2 arithmetic (sm_100 FFMA2 / FMUL2 / FADD2): one instruction for two independent values, each rounded
 // exactly like its scalar counterpart
 __device__ __forceinline__ float2 f2bc(float x) { return make_float2(x, x); }
@@ -134,7 +87,7 @@ __device__ __forceinline__ float2 f2mul(float2 a, float2 b) { return __fmul2_rn(
 __device__ __forceinline__ float2 f2add(float2 a, float2 b) { return __fadd2_rn(a, b); }
 __device__ __forceinline__ float2 f2fma(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
 
-// Packed column sums (FADD2 / FFMA2: half the instructions of the scalar versions above).  Lane = 16 * half + pair
+// Packed column sums (FADD2 / FFMA2).  Lane = 16 * half + pair
 // sums the 16 rows [16 half, 16 half + 16) of the two adjacent columns col2, col2 + 1 (col2 even).  The two halves are
 // separate accumulators until the kernel's final fold.
 template <int ROW>
@@ -220,24 +173,10 @@ __device__ __forceinline__ Geom geom_from_raw(const RawPt& r) {
 }
 __device__ __forceinline__ Geom load_geom(const StepParams& p, long long i) { return geom_from_raw(load_raw(p, i)); }
 
-// N sigmoids stage by stage (all EX2, then all RCP) so that the MUFU latencies overlap inside one warp
-template <int N>
-__device__ __forceinline__ void sigm_n(const float (&u)[N], float (&s)[N]) {
-  float e[N];
-#pragma unroll
-  for (int i = 0; i < N; i++) asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e[i]) : "f"(u[i] * -1.4426950408889634f));
-#pragma unroll
-  for (int i = 0; i < N; i++) e[i] = 1.0f + e[i];
-#pragma unroll
-  for (int i = 0; i < N; i++) s[i] = rcp_approx(e[i]);
-}
-
 // ---------------------------------------------------------------------------------------------
-// theta (1521 scalars, state_dict order) -> the weight image the kernels read (Wts).  Run by `nt` threads (t = 0..nt-1):
-// by prep_weights_kernel into global memory for the FFMA engine (FULL = true: also the plain mat-vec rows), and by every
-// CTA of the tcgen05 kernel straight into its shared memory (FULL = false: only what lies in front of Wts::W2).
+// theta (1521 scalars, state_dict order) -> the weight image the step kernel reads (Wts).  Run by `nt` threads
+// (t = 0..nt-1) of every CTA, straight into its shared memory.
 // ---------------------------------------------------------------------------------------------
-template <bool FULL>
 __device__ __forceinline__ void build_weight_image(const float* __restrict__ th, Wts* __restrict__ out, int t, int nt) {
   for (int i = t; i < NH; i += nt) {
     const float a = th[O_W1 + 2 * i], b = th[O_W1 + 2 * i + 1];
@@ -262,18 +201,6 @@ __device__ __forceinline__ void build_weight_image(const float* __restrict__ th,
     out->bgLs[i] = in ? th[O_BGL + i] * NEG_LOG2E : 0.0f;
   }
   if (t == 0) { out->bo = th[O_BO]; out->bE = th[O_BE]; out->bg = th[O_BG]; out->pad0 = 0.0f; }
-  if (FULL) {
-    for (int i = t; i < NH * NH; i += nt) {
-      const int j = i / NH, k = i % NH;
-      out->W2[i] = th[O_W2 + i];
-      out->W2T[k * NH + j] = th[O_W2 + i];
-    }
-    for (int i = t; i < NE * NE; i += nt) {
-      const int j = i / NE, k = i % NE;
-      out->WE2[i] = th[O_WE2 + i];
-      out->WE2T[k * NE + j] = th[O_WE2 + i];
-    }
-  }
   // ---- tcgen05 operand images: value -> (hi, lo) TF32 pair, round-to-nearest split ----
   auto put = [](float* hi, float* lo, int off, float v) {
     uint32_t h, l;
@@ -352,9 +279,6 @@ __device__ __forceinline__ float2 sigm2_pre(const float2 up, float2& om) {
 __device__ __forceinline__ float2 one_minus_sigm2_pre(const float2 up, const float2 s) {
   return one_minus_sigm2(make_float2(ex2_approx(up.x), ex2_approx(up.y)), s);
 }
-
-// one sigmoid whose argument already carries the factor -log2(e)
-__device__ __forceinline__ float sigm_pre(float up) { return rcp_approx(1.0f + ex2_approx(up)); }
 
 // Q = al11 v1^2 + al12 v1 v2 + al22 v2^2 for two hidden units.  (A 5-operation form v1 (al11 v1 + al12 v2) + al22 v2^2, a
 // packed accumulation of N and D, and a non-volatile mma.sync were measured together in round 2: +0.1 % - inside the

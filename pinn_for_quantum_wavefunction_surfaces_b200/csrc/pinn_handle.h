@@ -32,20 +32,14 @@ struct pinn_handle {
   int sm_count = 0;
   std::vector<pinn_workspace> ws;  // one per stream that has called in (guarded by mu)
   uint64_t ws_clock = 0;
-#ifdef PINN_AB_BUILD
-  Wts* wts = nullptr;              // FFMA engine (A/B builds only): prepared weight image
-#endif
-  float* theta_dev = nullptr;      // upload block of the *_host entry: 1536 float ...
-  double* weights_dev = nullptr;   // ... followed by the 3 loss weights
   // *_host entry
+  float* theta_pinned = nullptr;   // theta as float: kernel parameters, or the source of the upload below
+  float* theta_dev = nullptr;      // theta uploaded for calls without loss weights
   void* stage_dev = nullptr;       // coordinates + mask
   size_t stage_bytes = 0;
   double* out_pinned = nullptr;    // mapped page-locked: the reduction kernel of the *_host entry writes it directly
   double* out_mapped = nullptr;    // its device alias
-  float* theta_pinned = nullptr;
-  double* weights_pinned = nullptr;
   cudaStream_t s_copy = nullptr, s_main = nullptr;
-  cudaEvent_t ev_copy = nullptr;
   cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr};  // *_host entry: copy of chunk c complete
   // data-parallel exchange (pinn_dp_*): own buffer, the peers' buffers as mapped on this device, and whether calls reduce
   unsigned char* dp_buf = nullptr;
@@ -56,11 +50,6 @@ struct pinn_handle {
   bool dp_opened[DP_MAX_WORLD] = {false, false, false, false, false, false, false, false};  // peer[r] came from cudaIpcOpenMemHandle
   double host_us[4] = {0, 0, 0, 0};   // last pinn_loss_fwd_bwd_host call: submit, wait, copy-out, total (microseconds)
   int64_t launches = 0;
-  // The product library has ONE engine (tcgen05) and no run-time knobs.  -DPINN_AB_BUILD (tools/build_ab.sh) adds the
-  // FFMA engine and two environment switches of the *_host entry for A/B measurements.
-  int engine = PINN_ENGINE_TCGEN05;
-  bool host_inline_params = true;     // *_host entry: theta + loss weights inside the kernel parameters
-  bool host_zero_copy = true;         // pinn_loss_fwd_bwd_host reads page-locked inputs in place
   bool profiling = false;          // pinn_profile_begin/collect: CUDA events around the fused step kernel
   std::vector<cudaEvent_t> ev_pool;
   size_t ev_used = 0;
@@ -109,8 +98,29 @@ struct LossCall {
   const pinn::AdamParams* adam = nullptr;       // optimizer step fused behind the reduction (the trainer)
   unsigned long long* adam_ticket = nullptr;
   const pinn::SampleParams* presample = nullptr;  // the trainer's next batch drawn by extra blocks of the reduction kernel
+  // Chunk plan: the batch as up to 4 step launches over points [first, first + count), each enqueued after the stream has
+  // waited for its event (NULL: no wait; the *_host entry records there that the chunk's copy is complete).  The partial
+  // rows of all chunks go to ONE reduction.  nchunk = 0: one launch over the whole batch.
+  struct Chunk {
+    int64_t first, count;
+    cudaEvent_t ready;
+  };
+  int nchunk = 0;
+  Chunk chunk[4] = {};
 };
 int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st);
+
+// VariantCoef and number of MLP evaluations (1 or 2) of a PINN_VARIANT_*; PINN_EINVAL for an unknown variant
+inline int variant_coef(int variant, VariantCoef* vc, int* nev) {
+  if (variant == PINN_VARIANT_POC) { *vc = {1.0f, -0.5f, -1.0f, -1.0f}; *nev = 2; return 0; }
+  if (variant == PINN_VARIANT_TRAINPY) { *vc = {2.0f, 1.0f, 1.0f, 1.0f}; *nev = 1; return 0; }
+  return PINN_EINVAL;
+}
+// Grid of a step-kernel launch over n points: one persistent CTA per SM, a CTA works on super-tiles of 128 points
+inline int grid_for(const pinn_handle* h, long long n) {
+  const long long want = (n + 127) / 128;
+  return (int)(want < h->sm_count ? (want < 1 ? 1 : want) : h->sm_count);
+}
 
 // The workspace of stream `st` with room for at least `rows` partial rows (created / grown on first use; the handle mutex
 // is held by the caller).  NULL + error message on failure.

@@ -29,7 +29,10 @@ struct GridDesc {
 struct StepParams {
   const void *x, *y, *z, *R;
   const uint8_t* mask;
-  const Wts* wts;         // A/B builds, FFMA engine: weight image built by prep_weights_kernel
+  // 8 unused bytes.  Without them every member behind moves up by 8 bytes, and ptxas schedules the training kernel
+  // <2,true,false> differently (5866 instead of 5874 SASS instructions): measured 0.2 % slower, 0.11085 vs 0.11062 ms
+  // per 2^18-point step (tools/ab_time.py, 5 interleaved rounds, B200 at 1000 W).
+  const void* unused_slot;
   const float* theta;     // the raw parameter vector; every CTA builds its own operand images in shared memory
   const double* weights;  // {w_pde, w_bc1, w_bc2}
   double* partials;       // [gridDim.x][NPART]
@@ -77,11 +80,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #endif
 
-#ifdef PINN_AB_BUILD  // FFMA engine (pinn_step_ffma.cu), A/B builds only
-cudaError_t launch_step(int nev, bool train, const StepParams& p, int grid, cudaStream_t st);
-cudaError_t launch_prep(const float* theta, Wts* out, cudaStream_t st);
-#endif
-// tcgen05 engine (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM
+// the fused step kernel (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st);
 cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, cudaStream_t st);
 // sums the rows_per_R rows of every R in a fixed order -> out [nR][8]; a row with R <= 0 (or NaN) is all NaN

@@ -1,6 +1,6 @@
 // Collocation sampler + clamp + boundary sets (train.py:26-39; poc/main.py:124-156, 390-393) as device code shared by
 // sample_kernel (pinn_train.cu) and by the sampler blocks that ride in the reduction kernel of the previous step
-// (pinn_kernels.cu: the batch of step t+1 is drawn while step t is reduced).
+// (pinn_reduce.cu: the batch of step t+1 is drawn while step t is reduced).
 #pragma once
 #include "pinn_device.cuh"
 #include "pinn_train.h"

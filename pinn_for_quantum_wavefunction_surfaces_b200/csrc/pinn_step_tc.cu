@@ -1,14 +1,13 @@
 // Fused PINN residual-and-gradient kernel, tcgen05 engine (B200, sm_100a).
 //
-// Same mathematics and the same role decomposition as pinn_kernels.cu (oracle/closed_form.py is the
-// specification; poc/main.py:247-303, 82-120, 341-355 and train.py:41-57 are what it replaces), but the
-// four mat-vec families of a tile
+// oracle/closed_form.py is the specification; poc/main.py:247-303, 82-120, 341-355 and train.py:41-57 are what it
+// replaces.  The four mat-vec families of a tile
 //     base-MLP layer 2 forward      V = W2 h        (4 Taylor channels)
 //     base-MLP layer 2 reverse      hbar = W2^T vbar (4 channels)
 //     E-net layer 2 forward / reverse (32 x 32)
 // run on the 5th-generation tensor cores instead of FFMA chains:
 //   * a CTA works on a SUPER-TILE of 128 collocation points: 4 groups x 32 points, thread = point =
-//     TMEM lane.  Warps are specialised by role as before (one warpgroup per MLP evaluation, one for
+//     TMEM lane.  Warps are specialised by role (one warpgroup per MLP evaluation, one for
 //     E-net + gate); the 4 warps of a role form the 128 rows of an M=128 tcgen05.mma.
 //   * every thread writes its row of the A operand (activations, split x = hi + lo with hi = the 19 bits
 //     the tensor core reads) straight from registers into TENSOR MEMORY with tcgen05.st; the B operands
@@ -61,7 +60,7 @@ __host__ __device__ constexpr int tc_group_stash_floats() { return NEV * EVAL_ST
 constexpr int GEO_BYTES = 2 * 128 * 12 * 4;
 template <int NEV>
 __host__ __device__ constexpr size_t tc_smem_bytes() {
-  return WTS_TC_BYTES + 64 /*mbarriers + tmem base*/ + sizeof(float2) * 4 * 2 * 3 * 32 + sizeof(float) * 4 * tc_group_stash_floats<NEV>() +
+  return sizeof(Wts) + 64 /*mbarriers + tmem base*/ + sizeof(float2) * 4 * 2 * 3 * 32 + sizeof(float) * 4 * tc_group_stash_floats<NEV>() +
          COORD_STAGES * COORD_STAGE_BYTES + GEO_BYTES;
 }
 
@@ -79,11 +78,6 @@ __device__ __forceinline__ void cp_async8(uint32_t dst, const void* src) {
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-// all but the newest COORD_AHEAD - 1 groups have landed
-__device__ __forceinline__ void cp_async_wait_next() {
-  if (COORD_AHEAD == 1) asm volatile("cp.async.wait_group 0;" ::: "memory");
-  else asm volatile("cp.async.wait_group 1;" ::: "memory");
-}
 
 // issued by the E-net warp of a group for the group's 32 points (slot = 32 * group + lane of the super-tile)
 __device__ __forceinline__ void coord_stage_issue(const StepParams& p, unsigned char* buf, int slot, long long i) {
@@ -775,12 +769,12 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
   const StepParams& p = q.p;
   constexpr int G = 4;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  Wts& w = *reinterpret_cast<Wts*>(smem_raw);  // only the first WTS_TC_BYTES are staged / valid
-  uint64_t* mbars = reinterpret_cast<uint64_t*>(smem_raw + WTS_TC_BYTES);  // [0]: weight copy, [1..3]: roles
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_raw + WTS_TC_BYTES + 32);
-  uint64_t* cfull = reinterpret_cast<uint64_t*>(smem_raw + WTS_TC_BYTES + 40);  // [COORD_STAGES]: bulk coordinate copies landed
-  float2* mbox = reinterpret_cast<float2*>(smem_raw + WTS_TC_BYTES + 64);
-  float* stash = reinterpret_cast<float*>(smem_raw + WTS_TC_BYTES + 64 + sizeof(float2) * G * 2 * 3 * 32);
+  Wts& w = *reinterpret_cast<Wts*>(smem_raw);
+  uint64_t* mbars = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Wts));  // [0]: weight copy, [1..3]: roles
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem_raw + sizeof(Wts) + 32);
+  uint64_t* cfull = reinterpret_cast<uint64_t*>(smem_raw + sizeof(Wts) + 40);  // [COORD_STAGES]: bulk coordinate copies landed
+  float2* mbox = reinterpret_cast<float2*>(smem_raw + sizeof(Wts) + 64);
+  float* stash = reinterpret_cast<float*>(smem_raw + sizeof(Wts) + 64 + sizeof(float2) * G * 2 * 3 * 32);
   unsigned char* cstage = smem_raw + tc_smem_bytes<NEV>() - COORD_STAGES * COORD_STAGE_BYTES - GEO_BYTES;
   float4* geo = reinterpret_cast<float4*>(smem_raw + tc_smem_bytes<NEV>() - GEO_BYTES);  // [2][128][3]
 
@@ -793,8 +787,8 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
   // CTA 0 times itself (SM cycles and nanoseconds, entry to the end of its tile loop): the effective SM clock of the launch,
   // read back by pinn_step_kernel_clock.  It is lower than the clock nvidia-smi samples while the tensor pipe is in use.
   // (start values parked in two free slots of the 64-byte barrier block, not in registers that would stay live)
-  uint32_t* clk0_slot = reinterpret_cast<uint32_t*>(smem_raw + WTS_TC_BYTES + 36);
-  unsigned long long* ns0_slot = reinterpret_cast<unsigned long long*>(smem_raw + WTS_TC_BYTES + 56);
+  uint32_t* clk0_slot = reinterpret_cast<uint32_t*>(smem_raw + sizeof(Wts) + 36);
+  unsigned long long* ns0_slot = reinterpret_cast<unsigned long long*>(smem_raw + sizeof(Wts) + 56);
   if (blockIdx.x == 0 && tid == 0) {
     unsigned long long ns0;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns0));
@@ -827,7 +821,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
   // Launches on device-resident batches keep the per-lane cp.async stage and carry no bulk code at all: with it the step on
   // HBM-resident inputs measured 1.7 % slower (0.1166 vs 0.1146 ms, tools/ab_time.py on one box, whichever warp issues and
   // whoever waits), against 3 % gained when the coordinates cross PCIe.
-  const bool cbulk = INLINE && TRAIN && COORD_AHEAD == 1 && !p.grid.on &&
+  const bool cbulk = INLINE && TRAIN && !p.grid.on &&
                      ((((uintptr_t)p.x | (uintptr_t)p.y | (uintptr_t)p.z | (uintptr_t)p.R | (uintptr_t)p.mask) & 15u) == 0);
   auto tile_bulk = [&](long long st) { return INLINE && cbulk && (st * 128 + 128 <= p.n); };
   const bool bulk_issuer = stager && grp == 0 && lane == 0;  // in the warp that SYNCS on the E-net role barrier (see below)
@@ -837,11 +831,6 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
     const long long i0 = (long long)blockIdx.x * 128 + slot;
     coord_stage_issue(p, cstage, slot, i0 < p.n ? i0 : p.n - 1);
     cp_async_commit();
-    if (COORD_AHEAD == 2) {  // and the second one
-      const long long i1 = i0 + (long long)gridDim.x * 128;
-      if ((long long)blockIdx.x + gridDim.x < ((p.n + 127) >> 7)) coord_stage_issue(p, cstage + COORD_STAGE_BYTES, slot, i1 < p.n ? i1 : p.n - 1);
-      cp_async_commit();
-    }
   }
 
   // ---- weights: theta arrives in shared memory by ONE TMA bulk copy (6080 of its 6084 bytes; bulk copies move multiples
@@ -885,7 +874,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       for (int i = tid; i < NTHETA; i += blockDim.x) th_s[i] = p.theta[i];
     }
     __syncthreads();
-    build_weight_image<false>(th_s, &w, tid, blockDim.x);
+    build_weight_image(th_s, &w, tid, blockDim.x);
     // the tensor cores read the operand images through the async proxy
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     __syncthreads();
@@ -935,7 +924,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
     const long long nsuper = (p.n + 127) >> 7;
     int it = 0;
     if (stager) {  // the first super-tile's coordinates (requested before the weight image was built)
-      cp_async_wait_next();
+      cp_async_wait_all();
       if (tile_bulk(blockIdx.x)) mbar_wait(smem_u32(&cfull[0]), 0u);
     }
     __syncthreads();
@@ -1006,17 +995,17 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
           g.R = 0.0f;  // only the E-net warp uses R
         }
       }
-      if (stager) {  // coordinates COORD_AHEAD super-tiles ahead: in flight while this one (and the next) is computed
-        const long long in = pidx + (long long)COORD_AHEAD * gridDim.x * 128;
-        const long long stn = st + (long long)COORD_AHEAD * gridDim.x;
+      if (stager) {  // coordinates of the next super-tile: in flight while this one is computed
+        const long long in = pidx + (long long)gridDim.x * 128;
+        const long long stn = st + gridDim.x;
         if (stn < nsuper) {
-          unsigned char* nbuf = cstage + ((it + COORD_AHEAD) % COORD_STAGES) * COORD_STAGE_BYTES;
+          unsigned char* nbuf = cstage + ((it + 1) % COORD_STAGES) * COORD_STAGE_BYTES;
           if (tile_bulk(stn)) {
             // (training launches only.)  The target buffer was read at the top of the previous super-tile; this thread
             // sits in the E-net role's issuing warp and has since SYNCED on the role barriers of that tile (the other
             // three warps only signal there), i.e. all four E-net warps - the only readers of the stage in training
             // launches - had read their coordinates.
-            if (bulk_issuer) coord_stage_issue_bulk(p, nbuf, &cfull[(it + COORD_AHEAD) % COORD_STAGES], stn);
+            if (bulk_issuer) coord_stage_issue_bulk(p, nbuf, &cfull[(it + 1) % COORD_STAGES], stn);
           } else {
             coord_stage_issue(p, nbuf, slot, in < p.n ? in : p.n - 1);
           }
@@ -1043,7 +1032,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       }
       TL(5);
       if (stager) {  // the NEXT tile's coordinates have landed; the barrier publishes them to the group
-        cp_async_wait_next();
+        cp_async_wait_all();
         // bulk copies complete on the stage's mbarrier: the E-net warps (the role with slack) wait for it here, off the MLP
         // warps' critical path, and the group barrier hands the data on (use number (it+1)/2 of that stage -> parity)
         const long long stn = st + (long long)gridDim.x;

@@ -153,15 +153,7 @@ constexpr uint32_t E_A_HI = 0, E_A_LO = 32, E_D = 64;
 
 constexpr int COORD_COL_BYTES = 128 * 8;                      // one coordinate column of a super-tile (float64 worst case)
 constexpr int COORD_STAGE_BYTES = 4 * COORD_COL_BYTES + 128 * 4;  // + one word per point for the set mask
-#ifndef PINN_COORD_AHEAD
-#define PINN_COORD_AHEAD 1
-#endif
-constexpr int COORD_AHEAD = PINN_COORD_AHEAD;                     // super-tiles the coordinate stage runs ahead (1 or 2)
-constexpr int COORD_STAGES = COORD_AHEAD + 1;
-static_assert(COORD_AHEAD == 1 || COORD_AHEAD == 2, "cp.async.wait_group needs an immediate");
-
-constexpr size_t WTS_TC_BYTES = offsetof(Wts, W2);  // everything the tcgen05 kernel stages
-static_assert(WTS_TC_BYTES % 128 == 0, "staged weight image must keep the buffers behind it aligned");
+constexpr int COORD_STAGES = 2;  // the coordinate stage runs one super-tile ahead
 
 struct TcCtx {
   uint32_t tbase;      // TMEM base address of the allocation

@@ -190,9 +190,7 @@ int pinn_grid_reduce(pinn_handle* h, int variant, const float* theta, int nx, in
   if (nx < 2 || ny < 2 || nz < 2) return fail(h, PINN_EINVAL, "pinn_grid_reduce: every axis needs at least 2 points");
   StepParams p{};
   int nev = 0;
-  if (variant == PINN_VARIANT_POC) { p.vc = {1.0f, -0.5f, -1.0f, -1.0f}; nev = 2; }
-  else if (variant == PINN_VARIANT_TRAINPY) { p.vc = {2.0f, 1.0f, 1.0f, 1.0f}; nev = 1; }
-  else return fail(h, PINN_EINVAL, "pinn_grid_reduce: unknown variant");
+  if (variant_coef(variant, &p.vc, &nev)) return fail(h, PINN_EINVAL, "pinn_grid_reduce: unknown variant");
   DevGuard dev_guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   pinn_workspace* ws = ws_for(h, st, h->sm_count);
@@ -204,8 +202,7 @@ int pinn_grid_reduce(pinn_handle* h, int variant, const float* theta, int nx, in
   p.grid.y0 = lim[2]; p.grid.dy = (lim[3] - lim[2]) / (ny - 1);
   p.grid.z0 = lim[4]; p.grid.dz = (lim[5] - lim[4]) / (nz - 1);
   p.grid.R = R; p.grid.wx = wx; p.grid.wy = wy; p.grid.wz = wz; p.grid.partials = ws->grid_partials;
-  const long long tiles = (p.n + 127) / 128;
-  const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+  const int grid = grid_for(h, p.n);
   CU(h, launch_step_tc(nev, false, p, grid, st));  // the dense-grid mode lives in the tcgen05 kernel
   CU(h, launch_grid_finish(ws->grid_partials, grid, out, st));
   h->launches += 2;
@@ -220,9 +217,7 @@ int pinn_spheroidal_reduce(pinn_handle* h, int variant, const float* theta, int 
   if (nR < 1 || ns < 1 || nnu < 1) return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: nR, ns and nnu must be at least 1");
   StepParams p{};
   int nev = 0;
-  if (variant == PINN_VARIANT_POC) { p.vc = {1.0f, -0.5f, -1.0f, -1.0f}; nev = 2; }
-  else if (variant == PINN_VARIANT_TRAINPY) { p.vc = {2.0f, 1.0f, 1.0f, 1.0f}; nev = 1; }
-  else return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: unknown variant");
+  if (variant_coef(variant, &p.vc, &nev)) return fail(h, PINN_EINVAL, "pinn_spheroidal_reduce: unknown variant");
   // every R owns whole super-tiles; the kernel's index arithmetic is 32-bit
   const long long tiles_per_R = ((long long)ns * nnu + 127) / 128;
   const long long tiles = tiles_per_R * nR;
@@ -239,7 +234,7 @@ int pinn_spheroidal_reduce(pinn_handle* h, int variant, const float* theta, int 
   p.grid.ns = ns; p.grid.nnu = nnu; p.grid.tiles_per_R = (int)tiles_per_R;
   p.grid.Rs = R; p.grid.s = s; p.grid.ws = ws; p.grid.nu = nu; p.grid.wnu = wnu;
   p.grid.partials = wk->sph_partials;
-  const int grid = (int)(tiles < h->sm_count ? tiles : h->sm_count);
+  const int grid = grid_for(h, p.n);
   CU(h, launch_step_tc(nev, false, p, grid, st));
   CU(h, launch_sph_finish(wk->sph_partials, nR, (int)tiles_per_R * 4, R, out, st));
   h->launches += 2;

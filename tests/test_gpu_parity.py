@@ -34,7 +34,7 @@ TRAINED_LBC_BAR = 1.5e-4    # Lbc ~ 9e-10 = psi^2 of a 2e-5 cancellation of O(0.
 
 
 def test_one_engine_no_dispatch():
-    """The product library carries the tcgen05 engine only; the FFMA engine lives in the A/B build (tools/build_ab.sh)."""
+    """The library carries the tcgen05 engine only: asking for the FFMA engine is refused and changes nothing."""
     h = pk.Handle.get(0)
     assert h.get_engine() == "tcgen05"
     with pytest.raises(pk.PinnError):

@@ -1,5 +1,5 @@
 """Tiny driver for ncu: a few training-step launches on one 2^18-point batch.
-   python tools/prof_step.py [tcgen05|ffma] [variant 0|1] [launches] [finetune 0|1]"""
+   python tools/prof_step.py [variant 0|1] [launches] [finetune 0|1]"""
 import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -7,13 +7,10 @@ sys.path.insert(0, ROOT)
 import pinn_for_quantum_wavefunction_surfaces_b200 as pk
 from oracle import ref_autograd as ra
 
-engine = sys.argv[1] if len(sys.argv) > 1 else "tcgen05"
-variant = int(sys.argv[2]) if len(sys.argv) > 2 else 0
-launches = int(sys.argv[3]) if len(sys.argv) > 3 else 4
-finetune = int(sys.argv[4]) if len(sys.argv) > 4 else 0
+variant = int(sys.argv[1]) if len(sys.argv) > 1 else 0
+launches = int(sys.argv[2]) if len(sys.argv) > 2 else 4
+finetune = int(sys.argv[3]) if len(sys.argv) > 3 else 0
 dev = torch.device("cuda:0")
-if engine != "tcgen05":  # "ffma": A/B build only (PINN_B200_LIBRARY=tools/dbg/libpinn_b200_ab.so)
-    pk.Handle.get(0).set_engine(engine)
 n = 1 << 18
 g = torch.Generator().manual_seed(5)
 x, y, z, R, i1, i2 = ra.sample_box(n, "poc" if variant == 0 else "trainpy", g)
@@ -30,4 +27,4 @@ for i in range(launches):
     pk.loss_and_grad_raw(variant, *xs, th, None, w, pk.FINE_TUNE_GRAD_MASK if finetune else 0xFFFF, sums=sums, dtheta=dth)
 e1.record()
 torch.cuda.synchronize()
-print("engine %s variant %d: last step %.4f ms, Ltot %.6e" % (engine, variant, e0.elapsed_time(e1), float(sums[0])))
+print("variant %d: last step %.4f ms, Ltot %.6e" % (variant, e0.elapsed_time(e1), float(sums[0])))

@@ -34,10 +34,6 @@ def case(variant, theta, n, seed):
         print("   %-18s max|ref| %.3e  err/max|ref_tensor| %.2e  err/max|grad| %.2e" % (
             nm, np.abs(b).max(), np.abs(a - b).max() / max(np.abs(b).max(), 1e-300), np.abs(a - b).max() / gmax))
 
-ENGINE = sys.argv[1] if len(sys.argv) > 1 else "tcgen05"   # "ffma" needs the A/B build (PINN_B200_LIBRARY=tools/dbg/libpinn_b200_ab.so)
-if ENGINE != "tcgen05":
-    pk.Handle.get(0).set_engine(ENGINE)
-print("engine:", pk.Handle.get(0).get_engine())
 ck = np.load(os.path.join(gd, "checkpoints.npz"))
 rng = np.random.default_rng(1)
 tp = np.load(os.path.join(gd, "trainpy_n2048.npz"))

@@ -20,7 +20,6 @@ from oracle import ref_autograd as ra
 variant = int(sys.argv[1]) if len(sys.argv) > 1 else 0
 dev = torch.device("cuda:0")
 h = pk.Handle.get(0)
-h.set_engine("tcgen05")
 n = 1 << 18
 g = torch.Generator().manual_seed(5)
 x, y, z, R, i1, i2 = ra.sample_box(n, "poc", g)
