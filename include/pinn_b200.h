@@ -17,7 +17,10 @@
  *    calls, so every *device* entry point is CUDA-graph capturable once one plain
  *    call has been made on the capturing stream.  pinn_spheroidal_reduce also keeps
  *    room for the largest sweep it has run on the stream: a capture of it needs one
- *    plain call at least as large (nR * ceil(ns*nnu/128)) first.
+ *    plain call at least as large (nR * ceil(ns*nnu/128)) first.  Likewise a training
+ *    call with more points than any earlier call on its stream grows the row workspace
+ *    (past 148 x 256 x 128 = 4.8e6 points a training launch gets one row per 256
+ *    super-tiles per SM): capture only after a plain call at least as large.
  *  - every call takes the stream explicitly (as a void* holding a cudaStream_t) and
  *    selects the handle's device itself, so it may be called from any host thread
  *    (torch runs autograd.Function.backward on its own thread).  Calls on ONE stream

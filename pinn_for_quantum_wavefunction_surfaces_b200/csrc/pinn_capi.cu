@@ -390,7 +390,7 @@ static int enqueue_step_chunk(pinn_handle* h, pinn_workspace* ws, int nev, StepP
   if (p.E_out) p.E_out += first;
   p.n = cnt;
   p.partials = ws->partials + (size_t)row0 * NPART;
-  const int grid = grid_for(h, cnt);
+  const int grid = train_grid_for(h, cnt);
   if (row0 + grid > ws->rows) return fail(h, PINN_EINVAL, "internal: partial-row workspace exceeded");
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (h->profiling) {
@@ -424,8 +424,10 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
     return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: NULL pointer argument");
   if (c.in_dtype != PINN_F32 && c.in_dtype != PINN_F64) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: bad in_dtype");
   const int nchunk = c.nchunk ? c.nchunk : 1;
+  int need_rows = 0;  // one partial row per CTA of every chunk launch
+  for (int k = 0; k < nchunk; k++) need_rows += train_grid_for(h, c.nchunk ? c.chunk[k].count : c.n);
   DevGuard dev_guard(h->device);
-  pinn_workspace* ws = ws_for(h, st, nchunk * h->sm_count);
+  pinn_workspace* ws = ws_for(h, st, need_rows);
   if (!ws) return PINN_EINVAL;
   if (int rc = dp_serialize(h, st)) return rc;
   p.x = c.x; p.y = c.y; p.z = c.z; p.R = c.R; p.mask = c.mask; p.n = c.n; p.in_f64 = c.in_dtype == PINN_F64;

@@ -121,6 +121,17 @@ inline int grid_for(const pinn_handle* h, long long n) {
   const long long want = (n + 127) / 128;
   return (int)(want < h->sm_count ? (want < 1 ? 1 : want) : h->sm_count);
 }
+// Grid of a TRAINING launch: the step kernel keeps its gradient and loss sums in float32 registers over every super-tile
+// a CTA works on, and their error grows with that count (DESIGN.md section 4).  Past TRAIN_TILES_MAX super-tiles per CTA
+// the launch gets sm_count * ceil(T / TRAIN_TILES_MAX) CTAs instead (T = super-tiles per CTA at one CTA per SM); the
+// CTAs beyond one per SM run as later waves, each into its own partial row.  Up to 148 x 256 x 128 = 4.8e6 points a
+// launch keeps one CTA per SM.
+constexpr long long TRAIN_TILES_MAX = 256;
+inline int train_grid_for(const pinn_handle* h, long long n) {
+  const long long per_cta = ((n + 127) / 128 + h->sm_count - 1) / h->sm_count;
+  if (per_cta <= TRAIN_TILES_MAX) return grid_for(h, n);
+  return (int)((long long)h->sm_count * ((per_cta + TRAIN_TILES_MAX - 1) / TRAIN_TILES_MAX));
+}
 
 // The workspace of stream `st` with room for at least `rows` partial rows (created / grown on first use; the handle mutex
 // is held by the caller).  NULL + error message on failure.
