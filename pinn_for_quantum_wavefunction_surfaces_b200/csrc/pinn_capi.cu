@@ -79,7 +79,7 @@ void ws_release(pinn_handle* h, cudaStream_t st) {
     }
 }
 
-static bool stream_is_capturing(cudaStream_t st) {
+bool stream_is_capturing(cudaStream_t st) {
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) { cudaGetLastError(); return false; }
   return cap != cudaStreamCaptureStatusNone;
@@ -169,37 +169,7 @@ bool ws_sph_rows(pinn_handle* h, pinn_workspace* w, cudaStream_t st, int rows) {
   return true;
 }
 
-// With the data-parallel exchange enabled the handle's exchange buffers carry one sequence of steps: calls must reach the
-// device in one order on all ranks.  A call on another stream than the previous exchanging call first waits (on the
-// host) for that stream to drain.
-static int dp_serialize(pinn_handle* h, cudaStream_t st) {
-  if (!h->dp_on || h->dp.world <= 1) return 0;
-  if (h->dp_stream_set && h->dp_stream != st) {
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) { cudaGetLastError(); cap = cudaStreamCaptureStatusNone; }
-    if (cap != cudaStreamCaptureStatusNone)
-      return fail(h, PINN_EINVAL, "data-parallel exchange: the previous exchanging call used another stream; cannot switch streams under capture");
-    CU(h, cudaStreamSynchronize(h->dp_stream));
-  }
-  h->dp_stream = st;
-  h->dp_stream_set = true;
-  return 0;
-}
-
 extern "C" {
-
-static void dp_release(pinn_handle* h) {
-  for (int r = 0; r < DP_MAX_WORLD; r++) {
-    if (h->dp_opened[r] && h->dp.peer[r]) cudaIpcCloseMemHandle(h->dp.peer[r]);
-    h->dp_opened[r] = false;
-    h->dp.peer[r] = nullptr;
-  }
-  if (h->dp_buf) cudaFree(h->dp_buf);
-  h->dp_buf = nullptr;
-  h->dp = DpArgs();
-  h->dp_on = false;
-  h->dp_stream_set = false;
-}
 
 int pinn_destroy(pinn_handle* h) {
   if (!h) return 0;
@@ -268,115 +238,6 @@ static bool map_pinned(const void* p, const void** dev) {
   if (a.type != cudaMemoryTypeHost || !a.devicePointer) return false;
   *dev = a.devicePointer;
   return true;
-}
-
-// ---------------------------------------------------------------------------------------------
-// data-parallel exchange over NVLink peer memory (include/pinn_b200.h: pinn_dp_*)
-// ---------------------------------------------------------------------------------------------
-int pinn_dp_init(pinn_handle* h, int rank, int world, void* ipc_handle_out) {
-  if (!h) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (world < 1 || world > DP_MAX_WORLD || rank < 0 || rank >= world)
-    return fail(h, PINN_EINVAL, "pinn_dp_init: need 0 <= rank < world <= 8");
-  DevGuard dev_guard(h->device);
-  dp_release(h);
-  CU(h, cudaMalloc(&h->dp_buf, DP_BUFFER_BYTES));
-  CU(h, cudaMemset(h->dp_buf, 0, DP_BUFFER_BYTES));
-  CU(h, cudaDeviceSynchronize());
-  h->dp.rank = rank;
-  h->dp.world = world;
-  h->dp.peer[rank] = h->dp_buf;
-  if (ipc_handle_out) {
-    static_assert(sizeof(cudaIpcMemHandle_t) == PINN_DP_HANDLE_BYTES, "IPC handle size");
-    cudaIpcMemHandle_t ih;
-    CU(h, cudaIpcGetMemHandle(&ih, h->dp_buf));
-    memcpy(ipc_handle_out, &ih, sizeof(ih));
-  }
-  return 0;
-}
-
-int pinn_dp_connect(pinn_handle* h, const void* all_handles) {
-  if (!h || !all_handles) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (!h->dp_buf) return fail(h, PINN_EINVAL, "pinn_dp_connect: call pinn_dp_init first");
-  DevGuard dev_guard(h->device);
-  for (int r = 0; r < h->dp.world; r++) {
-    if (r == h->dp.rank) continue;
-    cudaIpcMemHandle_t ih;
-    memcpy(&ih, (const char*)all_handles + (size_t)r * PINN_DP_HANDLE_BYTES, sizeof(ih));
-    void* ptr = nullptr;
-    CU(h, cudaIpcOpenMemHandle(&ptr, ih, cudaIpcMemLazyEnablePeerAccess));
-    h->dp.peer[r] = (unsigned char*)ptr;
-    h->dp_opened[r] = true;
-  }
-  h->dp_on = true;
-  return 0;
-}
-
-int pinn_dp_connect_local(pinn_handle* h, pinn_handle* const* peers) {
-  if (!h || !peers) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (!h->dp_buf) return fail(h, PINN_EINVAL, "pinn_dp_connect_local: call pinn_dp_init first");
-  DevGuard dev_guard(h->device);
-  for (int r = 0; r < h->dp.world; r++) {
-    if (r == h->dp.rank) continue;
-    pinn_handle* q = peers[r];
-    if (!q || !q->dp_buf || q->dp.world != h->dp.world || q->dp.rank != r)
-      return fail(h, PINN_EINVAL, "pinn_dp_connect_local: peer handle is not initialised for this rank/world");
-    if (q->device != h->device) {
-      int can = 0;
-      CU(h, cudaDeviceCanAccessPeer(&can, h->device, q->device));
-      if (!can) return fail(h, PINN_ENOTSUP, "pinn_dp_connect_local: no peer access between the two devices");
-      cudaError_t e = cudaDeviceEnablePeerAccess(q->device, 0);
-      if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
-      else if (e != cudaSuccess) return fail(h, (int)e, "cudaDeviceEnablePeerAccess");
-    }
-    h->dp.peer[r] = q->dp_buf;
-  }
-  h->dp_on = true;
-  return 0;
-}
-
-int pinn_dp_enable(pinn_handle* h, int on) {
-  if (!h) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (on) {
-    for (int r = 0; r < h->dp.world; r++)
-      if (!h->dp.peer[r]) return fail(h, PINN_EINVAL, "pinn_dp_enable: the exchange is not connected");
-    if (h->dp.world < 1) return fail(h, PINN_EINVAL, "pinn_dp_enable: the exchange is not initialised");
-  }
-  h->dp_on = on != 0;
-  return 0;
-}
-
-int pinn_dp_set_timeout(pinn_handle* h, double seconds) {
-  if (!h) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (!(seconds > 0.0) || seconds > 3600.0) return fail(h, PINN_EINVAL, "pinn_dp_set_timeout: need 0 < seconds <= 3600");
-  if (h->dp.world < 1) return fail(h, PINN_EINVAL, "pinn_dp_set_timeout: the exchange is not initialised");
-  h->dp.timeout_cycles = (long long)(seconds * 2.0e9);  // SM cycles at ~2 GHz: a bound, not a stopwatch
-  return 0;
-}
-
-int pinn_dp_status(pinn_handle* h, int64_t* exchanges) {
-  if (!h) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (!h->dp_buf) return fail(h, PINN_EINVAL, "pinn_dp_status: the exchange is not initialised");
-  DevGuard dev_guard(h->device);
-  unsigned long long ctl[3];
-  CU(h, cudaMemcpy(ctl, h->dp_buf + DP_ROWS_BYTES, sizeof(ctl), cudaMemcpyDeviceToHost));
-  if (exchanges) *exchanges = (int64_t)ctl[0];
-  if (ctl[2]) return fail(h, PINN_ETIMEDOUT, "pinn_dp: a peer did not deliver its partial sums within the time-out");
-  return 0;
-}
-
-int pinn_dp_shutdown(pinn_handle* h) {
-  if (!h) return PINN_EINVAL;
-  std::lock_guard<std::mutex> lk(h->mu);
-  DevGuard dev_guard(h->device);
-  CU(h, cudaDeviceSynchronize());
-  dp_release(h);
-  return 0;
 }
 
 // Enqueue the fused step kernel for points [first, first + cnt) of a batch; its per-CTA rows go to partial rows
@@ -463,7 +324,7 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
     rows += r;
   }
   CU(h, launch_reduce(ws->partials, rows, weights, c.weights_inline, c.grad_mask, c.dtheta, c.sums, p.E_out, c.n,
-                      h->dp_on ? h->dp : DpArgs(), st, c.adam, c.adam_ticket, c.presample, c.E_f64, c.dtheta_in_out));
+                      dp_active(h), st, c.adam, c.adam_ticket, c.presample, c.E_f64, c.dtheta_in_out));
   h->launches++;
   return 0;
 }

@@ -227,26 +227,9 @@ __device__ __forceinline__ void build_weight_image(const float* __restrict__ th,
   }
 }
 
-// system-scope accesses of the data-parallel exchange (peer memory over NVLink)
-__device__ __forceinline__ void st_relaxed_sys_v2(unsigned int* p, unsigned int a, unsigned int b) {
-  asm volatile("st.relaxed.sys.global.v2.u32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ uint2 ld_relaxed_sys_v2(const unsigned int* p) {
-  uint2 v;
-  asm volatile("ld.relaxed.sys.global.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p) : "memory");
-  return v;
-}
 __device__ __forceinline__ double ld_acquire_gpu(const double* p) {
   double v;
   asm volatile("ld.acquire.gpu.global.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_release_sys(unsigned long long* p, unsigned long long v) {
-  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
   return v;
 }
 

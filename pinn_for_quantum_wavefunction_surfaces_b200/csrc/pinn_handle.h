@@ -7,9 +7,20 @@
 
 #include "../../include/pinn_b200.h"
 #include "pinn_common.cuh"
+#include "pinn_dp.cuh"
 #include "pinn_launch.h"
 
 using namespace pinn;
+
+// The handle's data-parallel exchange (pinn_dp.cu)
+struct DpState {
+  unsigned char* buf = nullptr;  // own exchange buffer
+  DpArgs args;                   // rank, world, every rank's buffer as mapped on this device, time-out
+  bool on = false;               // calls exchange
+  cudaStream_t stream = nullptr;  // the exchange buffers carry ONE sequence of steps: the stream of the last exchanging call
+  bool stream_set = false;
+  bool opened[DP_MAX_WORLD] = {false, false, false, false, false, false, false, false};  // args.peer[r] came from cudaIpcOpenMemHandle
+};
 
 // Scratch memory of the calls ENQUEUED ON ONE STREAM.  Kernels of one stream run in order, so they may share it; calls
 // that arrive on different streams (torch's current stream, the *_host entry's private stream, every trainer's own
@@ -41,13 +52,7 @@ struct pinn_handle {
   double* out_mapped = nullptr;    // its device alias
   cudaStream_t s_copy = nullptr, s_main = nullptr;
   cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr};  // *_host entry: copy of chunk c complete
-  // data-parallel exchange (pinn_dp_*): own buffer, the peers' buffers as mapped on this device, and whether calls reduce
-  unsigned char* dp_buf = nullptr;
-  DpArgs dp;
-  bool dp_on = false;
-  cudaStream_t dp_stream = nullptr;  // the exchange buffers carry ONE sequence of steps: the stream of the last exchanging call
-  bool dp_stream_set = false;
-  bool dp_opened[DP_MAX_WORLD] = {false, false, false, false, false, false, false, false};  // peer[r] came from cudaIpcOpenMemHandle
+  DpState dp;
   double host_us[4] = {0, 0, 0, 0};   // last pinn_loss_fwd_bwd_host call: submit, wait, copy-out, total (microseconds)
   int64_t launches = 0;
   bool profiling = false;          // pinn_profile_begin/collect: CUDA events around the fused step kernel
@@ -140,6 +145,15 @@ pinn_workspace* ws_for(pinn_handle* h, cudaStream_t st, int rows);
 // any earlier call on the stream, which is refused under CUDA-graph capture.  false + error message on failure.
 bool ws_sph_rows(pinn_handle* h, pinn_workspace* w, cudaStream_t st, int rows);
 void ws_release(pinn_handle* h, cudaStream_t st);
+bool stream_is_capturing(cudaStream_t st);
+
+// pinn_dp.cu.  dp_active: the exchange arguments of a call (world <= 1 unless the exchange is on with world > 1).
+// dp_serialize: before a call that may exchange is enqueued on `st`, mutex held.  dp_read_status: this rank's control
+// block, read synchronously (the exchange must be initialised).
+DpArgs dp_active(const pinn_handle* h);
+int dp_serialize(pinn_handle* h, cudaStream_t st);
+int dp_read_status(pinn_handle* h, int64_t* exchanges, bool* failed);
+void dp_release(pinn_handle* h);
 
 extern std::string g_create_err;
 

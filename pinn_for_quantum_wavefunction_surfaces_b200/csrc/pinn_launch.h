@@ -86,31 +86,11 @@ cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, c
 // sums the rows_per_R rows of every R in a fixed order -> out [nR][8]; a row with R <= 0 (or NaN) is all NaN
 cudaError_t launch_sph_finish(const double* partials, int nR, int rows_per_R, const double* Rs, double* out, cudaStream_t st);
 cudaError_t launch_count(const StepParams& p, unsigned long long* counts, double* weights, cudaStream_t st);
-// Data-parallel exchange fused into the reduction kernel (SURVEY.md 8e): every rank owns one exchange buffer that all
-// peers of the box can write through NVLink peer memory (cudaIpc / peer access).
-//   rows [2 slots][DP_MAX_WORLD][NPART] x 16 B : rank r deposits its reduced row in slot (step & 1), index r, of EVERY
-//        rank; each float64 is two 8-byte words {32 data bits, 32-bit step number} (pinn_reduce.cu: reduce_partials_kernel)
-//   ctl  8 x u64 {exchanges completed, blocks done, status, set-count exchanges completed, ...}
-//   cnt  [2 slots][DP_MAX_WORLD][2] x 8 B : the sampler's boundary-set sizes, same {data, step} words (pinn_train.cu)
-constexpr int DP_MAX_WORLD = 8;
-// How long a rank polls for a peer's contribution before it declares the run failed (SM cycles, ~30 s): long enough for any
-// host-side skew between the ranks' launches (one rank writing a checkpoint, drawing a batch on the CPU ...), short
-// enough that a dead peer does not hang the GPU.
-constexpr long long DP_TIMEOUT_CYCLES = 60000000000ll;
-constexpr int DP_BLOCKS = NPART / 32;
-constexpr size_t DP_ROWS_BYTES = 2ull * DP_MAX_WORLD * NPART * 16;
-constexpr size_t DP_CTL_BYTES = 64;
-constexpr size_t DP_CNT_BYTES = 2ull * DP_MAX_WORLD * 2 * 8;
-constexpr size_t DP_BUFFER_BYTES = DP_ROWS_BYTES + DP_CTL_BYTES + DP_CNT_BYTES;
-struct DpArgs {
-  int world = 0;  // <= 1: no exchange
-  int rank = 0;
-  unsigned char* peer[DP_MAX_WORLD] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // exchange buffers, [rank] = own
-  long long timeout_cycles = DP_TIMEOUT_CYCLES;  // pinn_dp_set_timeout
-};
 // weights: device pointer, or NULL with weights_inline (host, 3 double) carried in the kernel parameters
+// dp: the data-parallel exchange fused into the reduction (pinn_dp.cuh)
 // adam (optional): the optimizer step of the device-resident trainer fused behind the reduction (pinn_train.h)
 // presample (optional): extra blocks of the same launch draw the trainer's next batch (pinn_sample.cuh)
+struct DpArgs;
 struct AdamParams;
 struct SampleParams;
 // E_f64: E_out holds float64; dtheta_in_out: the 2-D tensors of dtheta are written in train.py's (in,out) layout

@@ -33,16 +33,13 @@ __global__ void weights_from_counts_kernel(const unsigned long long* counts, lon
 // ---------------------------------------------------------------------------------------------
 // add the partial rows (fixed order, double) -> dtheta, sums
 // block = 1024 threads = 32 entries x 32 row-slices (every thread has at most 5 independent loads in flight: one
-// round trip to L2 instead of a chain of 19)
+// round trip to L2 instead of a chain of 19); RED_BLOCKS blocks of 32 entries cover a row
 //
-// With dp.world > 1 the kernel is also the data-parallel all-reduce, in the style of a low-latency (LL) protocol: every
-// float64 travels as two 8-byte words {32 data bits, 32-bit step number}; 8-byte stores are single-copy atomic, so a
-// reader that sees the step number of this exchange in both words has the value - no fence, no separate flag, one
-// NVLink one-way latency.  Thread (r, e) of block b stores the block's reduced entry e into slot `rank` of peer r's
-// exchange buffer and then polls slot r of its own buffer; the `world` values are added in rank order, so every rank
-// computes bit-identical sums.  No NCCL launch, no extra kernel.  Two slots alternate by step parity: a peer can be at
-// most one exchange ahead (it needs this rank's next contribution to go further).
+// With dp.world > 1 the kernel is also the data-parallel all-reduce (pinn_dp.cuh): thread (r, e) of block b sends the
+// block's reduced entry e to peer r and receives peer r's; the `world` values are added in rank order.  No NCCL launch,
+// no extra kernel.
 // ---------------------------------------------------------------------------------------------
+constexpr int RED_BLOCKS = NPART / 32;
 constexpr int RED_SLICES = 32;
 static_assert(RED_SLICES >= DP_MAX_WORLD, "one row-slice of threads per data-parallel peer");
 struct RedWeights {  // loss weights by value (the *_host entry) instead of through device memory
@@ -56,7 +53,7 @@ struct AdamFuse {
   AdamParams a;
   unsigned long long* ticket;  // device, zero between launches
 };
-// The batch of the NEXT step drawn by extra blocks of this launch (blocks DP_BLOCKS .. gridDim.x-1), into the trainer's
+// The batch of the NEXT step drawn by extra blocks of this launch (blocks RED_BLOCKS .. gridDim.x-1), into the trainer's
 // other batch buffer: the sampler overlaps the reduction / optimizer step instead of standing between two kernels.
 struct SampleFuse {
   int on;
@@ -70,10 +67,10 @@ __global__ void __launch_bounds__(RED_SLICES * 32) reduce_partials_kernel(const 
                                                               const float* __restrict__ E_out, long long n, const DpArgs dp,
                                                               const AdamFuse ad, const SampleFuse sf, const int E_f64,
                                                               const int dtheta_in_out) {
-  if (blockIdx.x >= DP_BLOCKS) {
+  if (blockIdx.x >= RED_BLOCKS) {
     // sampler blocks: they touch nothing the step kernel in front reads or writes (other batch buffer), so they do not
     // wait for it; the reduction blocks below do, which also keeps this grid from completing early
-    if (sf.on) sample_block(sf.s, blockIdx.x - DP_BLOCKS, gridDim.x - DP_BLOCKS);
+    if (sf.on) sample_block(sf.s, blockIdx.x - RED_BLOCKS, gridDim.x - RED_BLOCKS);
     return;
   }
   __shared__ double sh[RED_SLICES][33];
@@ -92,19 +89,15 @@ __global__ void __launch_bounds__(RED_SLICES * 32) reduce_partials_kernel(const 
   sh[sl][e] = s;
   __syncthreads();
   unsigned int step = 0;
-  size_t slot = 0;
-  // A peer that never delivers (time-out below) poisons the run: ctl[2] is set and stays set, this and every later
-  // launch then skips the polling (no 30 s stall per step) AND the fused optimizer step, so the parameters stay what they
-  // were before the failed exchange; pinn_dp_status / pinn_trainer_read report PINN_ETIMEDOUT.
+  // A peer that never delivers poisons the run (DP_FAILED stays set): this and every later launch then skips the polling
+  // (no 30 s stall per step) AND the fused optimizer step, so the parameters stay what they were before the failed
+  // exchange; pinn_dp_status / pinn_trainer_read report PINN_ETIMEDOUT.
   __shared__ volatile int dp_failed_s;
   if (threadIdx.x == 0) dp_failed_s = 0;
   if (dp.world > 1) {
-    unsigned char* own = dp.peer[dp.rank];
-    unsigned long long* ctl = reinterpret_cast<unsigned long long*>(own + DP_ROWS_BYTES);
-    if (threadIdx.x == 0) dp_failed_s = ld_acquire_sys(&ctl[2]) != 0ull;
-    const unsigned long long step64 = ld_acquire_sys(&ctl[0]) + 1;  // ctl[0] = exchanges completed on this rank
+    if (threadIdx.x == 0) dp_failed_s = dp_has_failed(dp);
+    const unsigned long long step64 = dp_next_step(dp, DP_EXCHANGES);
     step = (unsigned int)step64;
-    slot = (size_t)(step64 & 1ull) * DP_MAX_WORLD;
     if (sl == 0) {
       double t = 0.0;
 #pragma unroll
@@ -118,38 +111,16 @@ __global__ void __launch_bounds__(RED_SLICES * 32) reduce_partials_kernel(const 
       if (r == dp.rank) {
         v = tot[e];
       } else {
-        const unsigned long long bits = (unsigned long long)__double_as_longlong(tot[e]);
-        unsigned int* dst = reinterpret_cast<unsigned int*>(dp.peer[r]) + ((slot + dp.rank) * NPART + idx) * 4;
-        st_relaxed_sys_v2(dst, (unsigned int)bits, step);
-        st_relaxed_sys_v2(dst + 2, (unsigned int)(bits >> 32), step);
-        const unsigned int* src = reinterpret_cast<const unsigned int*>(own) + ((slot + r) * NPART + idx) * 4;
-        const long long t0 = clock64();
-        uint2 lo = make_uint2(0u, 0u), hi = lo;
-        bool ok = false;
-        while (!dp_failed_s) {
-          lo = ld_relaxed_sys_v2(src);
-          hi = ld_relaxed_sys_v2(src + 2);
-          if (lo.y == step && hi.y == step) { ok = true; break; }
-          if (clock64() - t0 > dp.timeout_cycles) {  // a peer never arrived; report instead of hanging the GPU
-            for (int q = 0; q < dp.world; q++)  // tell everybody: the peers stop updating their replicas as well
-              st_release_sys(reinterpret_cast<unsigned long long*>(dp.peer[q] + DP_ROWS_BYTES) + 2, 1ull);
-            dp_failed_s = 1;
-            break;
-          }
-        }
-        v = ok ? __longlong_as_double((long long)(((unsigned long long)hi.x << 32) | lo.x)) : 0.0;
+        dp_send(dp_row(dp.peer[r], step, dp.rank, idx), (unsigned long long)__double_as_longlong(tot[e]), step);
+        unsigned long long bits = 0;
+        if (dp_recv(dp, dp_row(dp.peer[dp.rank], step, r, idx), step, dp_failed_s, bits))
+          v = __longlong_as_double((long long)bits);
       }
     }
     __syncthreads();  // every thread is done with sh / tot of the local pass
     sh[sl][e] = v;    // slices >= world contribute 0; the fixed-order sum below is the sum over ranks
     __syncthreads();
-    if (threadIdx.x == 0) {  // the last block of the launch closes the exchange (the next launch is stream-ordered behind it)
-      __threadfence();
-      if (atomicAdd(&ctl[1], 1ull) == (unsigned long long)DP_BLOCKS - 1) {
-        ctl[1] = 0ull;
-        st_release_sys(&ctl[0], step64);
-      }
-    }
+    if (threadIdx.x == 0) dp_block_done(dp, step64, RED_BLOCKS);
   }
   if (sl == 0) {
     double t = 0.0;
@@ -198,27 +169,13 @@ __global__ void __launch_bounds__(RED_SLICES * 32) reduce_partials_kernel(const 
       for (int i = 0; i < RED_SLICES; i++) local += sh[i][j];
       double g = local;
       if (dp.world > 1) {
-        const unsigned char* own = dp.peer[dp.rank];
         g = 0.0;
         for (int r = 0; r < dp.world; r++) {
           double v = local;
-          if (r != dp.rank) {  // the peer's block SB deposits this entry in our buffer; only read here
-            const unsigned int* src = reinterpret_cast<const unsigned int*>(own) + ((slot + r) * NPART + S_RES2 + j) * 4;
-            const long long t0 = clock64();
-            uint2 lo = make_uint2(0u, 0u), hi = lo;
-            bool ok = false;
-            while (!dp_failed_s) {
-              lo = ld_relaxed_sys_v2(src);
-              hi = ld_relaxed_sys_v2(src + 2);
-              if (lo.y == step && hi.y == step) { ok = true; break; }
-              if (clock64() - t0 > dp.timeout_cycles) {
-                for (int q = 0; q < dp.world; q++)
-                  st_release_sys(reinterpret_cast<unsigned long long*>(dp.peer[q] + DP_ROWS_BYTES) + 2, 1ull);
-                dp_failed_s = 1;
-                break;
-              }
-            }
-            v = ok ? __longlong_as_double((long long)(((unsigned long long)hi.x << 32) | lo.x)) : 0.0;
+          if (r != dp.rank) {  // the peer's block SB sent this entry to our buffer; only received here
+            unsigned long long bits = 0;
+            const bool ok = dp_recv(dp, dp_row(dp.peer[dp.rank], step, r, S_RES2 + j), step, dp_failed_s, bits);
+            v = ok ? __longlong_as_double((long long)bits) : 0.0;
           }
           g += v;
         }
@@ -239,7 +196,7 @@ __global__ void __launch_bounds__(RED_SLICES * 32) reduce_partials_kernel(const 
   __syncthreads();
   if (threadIdx.x == 0) {
     __threadfence();
-    flag_s = atomicAdd(ad.ticket, 1ull) == (unsigned long long)DP_BLOCKS - 1;
+    flag_s = atomicAdd(ad.ticket, 1ull) == (unsigned long long)RED_BLOCKS - 1;
     if (flag_s) {  // every block has updated its parameters and read the step / best loss; the loss sums are visible
       __threadfence();
       const double sv[8] = {ld_acquire_gpu(&sums[0]), ld_acquire_gpu(&sums[1]), ld_acquire_gpu(&sums[2]), ld_acquire_gpu(&sums[3]),
@@ -275,7 +232,7 @@ cudaError_t launch_reduce(const double* partials, int nrows, const double* weigh
   if (presample) { sf.on = 1; sf.s = *presample; }
   RedWeights wi{};
   if (weights_inline) { wi.w[0] = weights_inline[0]; wi.w[1] = weights_inline[1]; wi.w[2] = weights_inline[2]; wi.use = 1; }
-  return launch_pdl(reduce_partials_kernel, dim3(DP_BLOCKS + (presample ? PRESAMPLE_BLOCKS : 0)), dim3(RED_SLICES * 32), 0, st,
+  return launch_pdl(reduce_partials_kernel, dim3(RED_BLOCKS + (presample ? PRESAMPLE_BLOCKS : 0)), dim3(RED_SLICES * 32), 0, st,
                     partials, nrows, weights, wi, grad_mask, dtheta, sums, E_out, n, dp, ad, sf, E_f64, dtheta_in_out);
 }
 

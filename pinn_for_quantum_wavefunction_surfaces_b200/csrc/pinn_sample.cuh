@@ -26,9 +26,9 @@ __host__ __device__ inline void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t
 __device__ __forceinline__ float u01(uint32_t r) { return (float)(r >> 8) * 5.9604644775390625e-08f; }  // [0,1), 24 bits
 
 // weights {1/n, 1/|set1|, 1/|set2|} of the reference's means (empty set -> inf -> NaN loss, as in the reference),
-// and the batch counter moves on.  Run by one warp of the block of sample_kernel that finishes last.  Data-parallel runs (dp.world > 1) first add the set sizes of all ranks:
-// lane r stores this rank's two counts into peer r's exchange buffer as {count, step} words and polls its own buffer
-// for peer r's (same protocol as the gradient sum in reduce_partials_kernel), lane 0 adds them in rank order.
+// and the batch counter moves on.  Run by one warp of the block of sample_kernel that finishes last.  Data-parallel runs
+// (dp.world > 1) first add the set sizes of all ranks: lane r sends this rank's two counts (32 bits each) to peer r and
+// receives peer r's (pinn_dp.cuh), lane 0 adds them in rank order.
 __device__ __forceinline__ void sample_finish(const SampleParams& s) {
   __shared__ unsigned long long c[DP_MAX_WORLD][2];
   const DpArgs& dp = s.dp;
@@ -38,35 +38,19 @@ __device__ __forceinline__ void sample_finish(const SampleParams& s) {
   unsigned long long c1 = atomicAdd(&s.counts[0], 0ull), c2 = atomicAdd(&s.counts[1], 0ull);  // L2 values of the other blocks' atomics
   long long ntot = n;
   if (dp.world > 1) {
-    unsigned char* own = dp.peer[dp.rank];
-    unsigned long long* ctl = reinterpret_cast<unsigned long long*>(own + DP_ROWS_BYTES);
-    const unsigned long long step64 = ld_acquire_sys(&ctl[3]) + 1;
+    const unsigned long long step64 = dp_next_step(dp, DP_COUNT_EXCHANGES);
     const unsigned int step = (unsigned int)step64;
-    const size_t slot = (size_t)(step64 & 1ull) * DP_MAX_WORLD;
     if (lane < dp.world) {
       const int r = lane;
       if (r == dp.rank) {
         c[r][0] = c1; c[r][1] = c2;
       } else {
-        unsigned int* dst = reinterpret_cast<unsigned int*>(dp.peer[r] + DP_ROWS_BYTES + DP_CTL_BYTES) + (slot + dp.rank) * 4;
-        st_relaxed_sys_v2(dst, (unsigned int)c1, step);
-        st_relaxed_sys_v2(dst + 2, (unsigned int)c2, step);
-        const unsigned int* src = reinterpret_cast<const unsigned int*>(own + DP_ROWS_BYTES + DP_CTL_BYTES) + (slot + r) * 4;
-        const long long t0 = clock64();
-        uint2 a = make_uint2(0u, 0u), b = a;
-        // ctl[2] != 0: an earlier exchange of this run already failed (a peer never delivered) - do not wait again
-        bool failed = ld_acquire_sys(&ctl[2]) != 0ull;
-        while (!failed) {
-          a = ld_relaxed_sys_v2(src);
-          b = ld_relaxed_sys_v2(src + 2);
-          if (a.y == step && b.y == step) break;
-          if (clock64() - t0 > dp.timeout_cycles) {
-            for (int q = 0; q < dp.world; q++)  // every rank stops updating its replica (see reduce_partials_kernel)
-              st_release_sys(reinterpret_cast<unsigned long long*>(dp.peer[q] + DP_ROWS_BYTES) + 2, 1ull);
-            failed = true;
-          }
-        }
-        c[r][0] = failed ? 0ull : a.x; c[r][1] = failed ? 0ull : b.x;
+        dp_send(dp_cnt(dp.peer[r], step, dp.rank), (c2 << 32) | (unsigned int)c1, step);
+        // an earlier exchange of this run already failed (a peer never delivered): do not wait again
+        bool failed = dp_has_failed(dp);
+        unsigned long long v = 0;
+        const bool ok = dp_recv(dp, dp_cnt(dp.peer[dp.rank], step, r), step, failed, v);
+        c[r][0] = ok ? (unsigned int)v : 0ull; c[r][1] = ok ? v >> 32 : 0ull;
       }
     }
     __syncwarp();
@@ -74,7 +58,7 @@ __device__ __forceinline__ void sample_finish(const SampleParams& s) {
       c1 = 0; c2 = 0;
       for (int r = 0; r < dp.world; r++) { c1 += c[r][0]; c2 += c[r][1]; }
       ntot = n * dp.world;
-      st_release_sys(&ctl[3], step64);
+      dp_complete(dp, DP_COUNT_EXCHANGES, step64);
     }
   }
   if (lane == 0) {

@@ -3,6 +3,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "pinn_dp.cuh"
 #include "pinn_launch.h"
 #include <cmath>
 

@@ -1,6 +1,7 @@
 // C ABI of the rows next to the hot path (include/pinn_b200.h, "training loop" and "analysis" sections):
 // sampler, fused Adam, the device-resident trainer (CUDA-graph replay of sample -> loss -> Adam), the E(R)/gate
 // curve and the dense-grid quadrature sums.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 
@@ -45,10 +46,9 @@ static SampleParams sampler_params(pinn_trainer* t, int buf) {
   s.x = t->x[buf]; s.y = t->y[buf]; s.z = t->z[buf]; s.R = t->R[buf]; s.mask = t->mask[buf]; s.counts = t->counts[buf];
   // data-parallel: rank r draws points [r n, (r+1) n) of the global batch of world*n points, so the union over the
   // ranks is exactly the batch a single GPU would draw for n_global = world*n
-  const bool dp_run = h->dp_on && h->dp.world > 1;
-  s.index_offset = dp_run ? (long long)h->dp.rank * c.n : 0;
+  s.dp = dp_active(h);
+  s.index_offset = (long long)s.dp.rank * c.n;
   s.weights = t->weights[buf]; s.ticket = t->counts[buf] + 2; s.reset_counts = 1;
-  if (dp_run) s.dp = h->dp;
   return s;
 }
 
@@ -67,7 +67,7 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool presample_next
   a.theta = t->theta; a.m = t->m; a.v = t->v; a.grad = t->grad; a.sums = t->sums; a.theta32 = t->theta32;
   a.step = t->step; a.best_loss = t->best_loss; a.best_theta = t->best_theta; a.best_step = t->best_step;
   a.hist = t->hist; a.hist_cap = c.history_capacity;
-  a.n = c.n * ((h->dp_on && h->dp.world > 1) ? h->dp.world : 1);  // mean E of the history is over the global batch
+  a.n = c.n * std::max(1, dp_active(h).world);  // mean E of the history is over the global batch
   a.lr = c.lr; a.beta1 = c.beta1; a.beta2 = c.beta2; a.eps = c.eps; a.best_after = (double)c.best_after;
   a.grad_mask = c.grad_mask; a.best_mode = c.best_mode; a.hist_mean_E = c.history_mean_E;
   a.step_base = (unsigned long long)t->step_base;
@@ -446,9 +446,9 @@ int pinn_trainer_read(pinn_trainer* t, double* theta, double* m, double* v, doub
     const int64_t rows = history_rows < t->cfg.history_capacity ? history_rows : t->cfg.history_capacity;
     if (rows > 0) CU(h, cudaMemcpy(history, t->hist, (size_t)rows * 4 * 8, cudaMemcpyDeviceToHost));
   }
-  if (h->dp_on && h->dp.world > 1 && h->dp_buf) {  // a data-parallel run whose exchange failed stopped updating: say so
-    unsigned long long failed = 0;
-    CU(h, cudaMemcpy(&failed, h->dp_buf + DP_ROWS_BYTES + 2 * sizeof(unsigned long long), sizeof(failed), cudaMemcpyDeviceToHost));
+  if (dp_active(h).world > 1) {  // a data-parallel run whose exchange failed stopped updating: say so
+    bool failed = false;
+    if (int rc = dp_read_status(h, nullptr, &failed)) return rc;
     if (failed)
       return fail(h, PINN_ETIMEDOUT, "pinn_trainer_read: a data-parallel peer did not deliver its partial sums; the optimizer "
                                      "steps from the failed exchange on were skipped (values read are those before it)");
