@@ -253,6 +253,33 @@ int pinn_sample(pinn_handle* h, int64_t n, uint64_t seed, uint64_t batch, const 
                 float* x, float* y, float* z, float* R, uint8_t* mask, uint64_t* counts, double* weights, void* stream);
 
 /*
+ * Residual-adaptive collocation (RAD, Wu et al., CMAME 403, 2023): the n points of a batch drawn from `pool` uniform
+ * candidates with probability proportional to the PDE residual.
+ *  1. The pool is pinn_sample(pool, seed, batch, box, cutoff, bcutoff) bit for bit (pool_x .. pool_mask); pool_res is
+ *     its residual at theta (device float32 [1521]), the bits pinn_fields writes to `res`.
+ *  2. Weights, in float64: q_i = |res_i|^k (0 where res_i is not finite), Q = sum q_i; w_i = q_i * pool / Q + c when
+ *     Q > 0 and finite, else w_i = 1 (uniform).  pool_cdf (device float64 [pool]) = inclusive prefix sum of w, with a
+ *     fixed association order (block sums, then a sequential fold of the block totals): the same bits on every call, and
+ *     never decreasing.
+ *  3. Systematic resampling: u0 = word 0 of Philox4x32-10(counter = {pool_lo, pool_hi, batch_lo, batch_hi}, key = seed)
+ *     * 2^-32, the point just past the pool in its own stream.  Output j takes the first i with
+ *     pool_cdf[i] > ((double)j + u0) / (double)n * pool_cdf[pool-1] (evaluated exactly as written; no such i: pool-1).
+ *     Candidate i is therefore taken floor(n P_i) or ceil(n P_i) times, P_i = w_i / sum w.
+ *  4. x, y, z, R, mask = the pool's at the selected indices; idx (device int64 [n], may be NULL) = those indices;
+ *     counts (device 2 x uint64) = set sizes of the batch; weights (device 3 double) = {1/n, 1/count1, 1/count2} as
+ *     pinn_sample forms them.
+ * Eight launches: the batch index, the pool's set-size reset, the pool's sampler, the pool's residual (inference
+ * instance of the step kernel), four selection kernels.  All buffers are the caller's, so the call can be captured in a
+ * CUDA graph once it has run on the stream outside a capture.  PINN_EINVAL, with nothing launched, for n <= 0,
+ * pool < n, k or c negative or not finite, a NULL pointer other than idx, or an unknown variant.
+ */
+int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed, uint64_t batch,
+                         const float box[8], float cutoff, float bcutoff, float k, float c, float* pool_x, float* pool_y,
+                         float* pool_z, float* pool_R, uint8_t* pool_mask, float* pool_res, double* pool_cdf, float* x,
+                         float* y, float* z, float* R, uint8_t* mask, int64_t* idx, uint64_t* counts, double* weights,
+                         void* stream);
+
+/*
  * One optimizer step of torch.optim.Adam (no weight decay, no amsgrad) over the 1521 float64 parameters, fused with
  * the reference loops' bookkeeping (train.py:58-72; poc/main.py:403-417).  All pointers are device memory.
  *  theta, m, v   in/out float64 [1521];  grad: dLtot/dtheta;  sums: the 8 sums of pinn_loss_fwd_bwd
@@ -302,6 +329,16 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
 int pinn_trainer_read(pinn_trainer* t, double* theta, double* m, double* v, double* best_theta, double* scalars, double* history,
                       int64_t history_rows);
 int pinn_trainer_batch(pinn_trainer* t, float** x, float** y, float** z, float** R, uint8_t** mask);
+/* Residual-adaptive batches (pinn_sample_adaptive) for this trainer: every step that resamples draws its batch from
+ * pool_factor * n candidates, at the float32 parameters the previous step's Adam update left, with the trainer's seed and
+ * batch index (one index per draw).  The draw is enqueued in front of that step's step kernel: 6 launches more per
+ * resampling step (8 in all), and no batch is drawn inside the reduction kernel while adaptive sampling is on.
+ * use_graph = 1 replays the whole adaptive step as one graph of its own (same bits as plain launches).  The history and
+ * the best-model record are evaluated on the adaptive batches, so Ltot is not comparable with a uniform run's.
+ * pool_factor = 0 (the default) turns it off and frees the pool; the buffers of pool_factor * n points are allocated
+ * here, never in pinn_trainer_run.  PINN_EINVAL for pool_factor < 0, or k or c negative or not finite; PINN_ENOTSUP while
+ * the data-parallel exchange is on (pinn_trainer_run also refuses an adaptive trainer then). */
+int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c);
 void* pinn_trainer_stream(pinn_trainer* t);
 
 /*

@@ -25,12 +25,12 @@ from .ops import (PinnLossPoc, PinnLossTrainPy, loss_poc, loss_trainpy, fields, 
                   indices_to_mask, HostStep)
 from .patch import patch_nn_ion, run_train_py, trainpy_patched_source
 from . import analysis, convert, trainer
-from .trainer import Trainer, AdamState, adam_step, sample, train_trainpy, train_poc, init_trainpy, init_poc
+from .trainer import Trainer, AdamState, adam_step, sample, sample_adaptive, train_trainpy, train_poc, init_trainpy, init_poc
 
 __all__ = [
     "N_THETA", "POC_TENSOR_NAMES", "TRAINPY_TENSOR_NAMES", "pack_poc", "unpack_poc", "pack_trainpy",
     "unpack_trainpy", "FINE_TUNE_GRAD_MASK", "lib", "Handle", "PinnError", "library_path", "bind_host_to_device_numa", "PinnLossPoc",
     "PinnLossTrainPy", "loss_poc", "loss_trainpy", "fields", "loss_and_grad_raw", "indices_to_mask", "HostStep",
     "patch_nn_ion", "run_train_py", "trainpy_patched_source", "analysis", "convert", "trainer", "Trainer", "AdamState",
-    "adam_step", "sample", "train_trainpy", "train_poc", "init_trainpy", "init_poc",
+    "adam_step", "sample", "sample_adaptive", "train_trainpy", "train_poc", "init_trainpy", "init_poc",
 ]

@@ -11,9 +11,9 @@ EXPORTS = [
     "pinn_version", "pinn_theta_size", "pinn_theta_offsets", "pinn_create", "pinn_destroy", "pinn_last_error",
     "pinn_launch_count", "pinn_set_engine", "pinn_get_engine", "pinn_profile_begin", "pinn_profile_collect", "pinn_loss_fwd_bwd", "pinn_fields", "pinn_loss_fwd_bwd_host",
     "pinn_loss_fwd_bwd_tensors", "pinn_mask_from_index_sets", "pinn_measure_fp32_peak", "pinn_step_kernel_clock",
-    "pinn_sample", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_spheroidal_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
+    "pinn_sample", "pinn_sample_adaptive", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_spheroidal_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
     "pinn_trainer_load_state", "pinn_trainer_set_batch", "pinn_trainer_run", "pinn_trainer_read", "pinn_trainer_batch",
-    "pinn_trainer_stream",
+    "pinn_trainer_stream", "pinn_trainer_set_adaptive",
     "pinn_host_timing", "pinn_dp_init", "pinn_dp_connect", "pinn_dp_connect_local", "pinn_dp_enable", "pinn_dp_status", "pinn_dp_set_timeout", "pinn_dp_shutdown",
 ]
 
@@ -92,6 +92,9 @@ def lib():
         u64, f64 = ctypes.c_uint64, ctypes.c_double
         L.pinn_sample.argtypes = [vp, i64, u64, u64, ctypes.POINTER(f32), f32, f32, vp, vp, vp, vp, vp, vp, vp, vp]
         L.pinn_sample.restype = i32
+        L.pinn_sample_adaptive.argtypes = [vp, i32, vp, i64, i64, u64, u64, ctypes.POINTER(f32), f32, f32, f32, f32,
+                                           vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+        L.pinn_sample_adaptive.restype = i32
         L.pinn_adam_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, f64, f64, f64, f64, u32,
                                      i32, i64, i32, vp]
         L.pinn_adam_step.restype = i32
@@ -118,6 +121,8 @@ def lib():
         L.pinn_trainer_batch.restype = i32
         L.pinn_trainer_stream.argtypes = [vp]
         L.pinn_trainer_stream.restype = vp
+        L.pinn_trainer_set_adaptive.argtypes = [vp, i32, f32, f32]
+        L.pinn_trainer_set_adaptive.restype = i32
         L.pinn_host_timing.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
         L.pinn_host_timing.restype = i32
         L.pinn_dp_init.argtypes = [vp, i32, i32, vp]

@@ -49,6 +49,23 @@ struct AdamParams {
 cudaError_t launch_sample(const SampleParams& s, bool zero_counts, cudaStream_t st);
 cudaError_t launch_adam(const AdamParams& a, cudaStream_t st);
 
+// Residual-adaptive selection (pinn_adaptive.cu): n points out of a pool of N drawn by launch_sample, with the pool's
+// residuals.  Four launches; out.counts and out.ticket need not be zero.
+struct AdaptiveParams {
+  long long pool;                                 // N
+  double k, c;                                    // w_i = |res_i|^k * N / sum_j |res_j|^k + c
+  const float *px, *py, *pz, *pR, *res;           // device [N]: the pool and its residuals
+  const uint8_t* pmask;
+  double* cdf;                                    // device [N]: inclusive prefix sum of w
+  double* part;                                   // device [adaptive_scratch_doubles(N)]
+  const unsigned long long* pool_batch;           // device: the batch counter as the pool's draw left it (one past the pool)
+  long long* idx;                                 // device [n] pool index of every output point, or NULL
+  SampleParams out;                               // the batch: n, seed, x..mask, counts, weights, ticket, batch_counter
+                                                  // (moved on by sample_finish: point it at a scratch word), reset_counts
+};
+long long adaptive_scratch_doubles(long long pool);
+cudaError_t launch_adaptive_select(const AdaptiveParams& a, cudaStream_t st);
+
 // The update of one parameter (torch.optim.Adam: lerp first moment, bias corrections, eps outside the square root; no
 // weight decay, no amsgrad), shared by adam_kernel and by the optimizer step fused into the reduction kernel.
 // t = optimizer steps done before this one.

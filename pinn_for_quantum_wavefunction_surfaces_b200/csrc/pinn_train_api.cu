@@ -2,6 +2,7 @@
 // sampler, fused Adam, the device-resident trainer (CUDA-graph replay of sample -> loss -> Adam), the E(R)/gate
 // curve and the dense-grid quadrature sums.
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 
@@ -34,7 +35,33 @@ struct pinn_trainer {
   int64_t steps_issued = 0;
   int64_t step_base = 0;  // optimizer steps done when the run (re)started (pinn_trainer_load_state)
   bool have_batch = false;
+  // residual-adaptive sampling (pinn_trainer_set_adaptive): pool_factor * n candidates per resampling step; off at 0
+  int pool_factor = 0;
+  float ad_k = 1.0f, ad_c = 1.0f;
+  float *px = nullptr, *py = nullptr, *pz = nullptr, *pR = nullptr, *pres = nullptr;
+  uint8_t* pmask = nullptr;
+  double *pcdf = nullptr, *pweights = nullptr, *ppart = nullptr;
+  unsigned long long* pcounts = nullptr;  // {|set1|, |set2|, ticket} of the pool's draw, [3] scratch batch word of the selection
+  cudaGraphExec_t graph_ad[2] = {nullptr, nullptr};  // [cur]: adaptive draw + step
+  bool ad_warmed = false;  // one plain adaptive step has run (the inference kernel's attributes are set)
 };
+
+// Launches of one adaptive draw on top of the pool's sampler: the pool's residual and the four selection kernels
+constexpr int ADAPTIVE_LAUNCHES = 6;
+
+// Pool of pool.n points (launch_sample), its residual at theta (the inference instance of the step kernel), then the
+// selection of a.out.n points (pinn_adaptive.cu).  The handle mutex is held by the caller.
+static int adaptive_enqueue(pinn_handle* h, int nev, const VariantCoef& vc, const float* theta, const SampleParams& pool,
+                            bool zero_pool_counts, const AdaptiveParams& a, cudaStream_t st) {
+  CU(h, launch_sample(pool, zero_pool_counts, st));
+  StepParams p{};
+  p.vc = vc; p.x = pool.x; p.y = pool.y; p.z = pool.z; p.R = pool.R; p.n = pool.n; p.theta = theta;
+  p.res = const_cast<float*>(a.res);
+  CU(h, launch_step_tc(nev, false, p, grid_for(h, pool.n), st));
+  CU(h, launch_adaptive_select(a, st));
+  h->launches += ADAPTIVE_LAUNCHES + (zero_pool_counts ? 1 : 0);
+  return 0;
+}
 
 static SampleParams sampler_params(pinn_trainer* t, int buf) {
   pinn_handle* h = t->h;
@@ -54,7 +81,7 @@ static SampleParams sampler_params(pinn_trainer* t, int buf) {
 
 // One optimizer step on buffer t->cur.  sample_now: draw its batch first with the stand-alone sampler kernel (the first
 // resampling step of a run); presample_next: the reduction kernel also draws the batch of the NEXT step into the other buffer.
-static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool presample_next, cudaStream_t st) {
+static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool adaptive_now, bool presample_next, cudaStream_t st) {
   pinn_handle* h = t->h;
   const pinn_train_config& c = t->cfg;
   const int b = t->cur;
@@ -62,6 +89,24 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool presample_next
     const SampleParams s = sampler_params(t, b);
     CU(h, launch_sample(s, false, st));
     h->launches += 1;
+  }
+  if (adaptive_now) {
+    // the pool takes the trainer's batch index (and moves it on); the selection writes buffer b like the sampler would
+    SampleParams pool = sampler_params(t, b);
+    pool.n = (long long)t->pool_factor * c.n; pool.index_offset = 0;
+    pool.x = t->px; pool.y = t->py; pool.z = t->pz; pool.R = t->pR; pool.mask = t->pmask;
+    pool.counts = t->pcounts; pool.ticket = t->pcounts + 2; pool.weights = t->pweights;
+    AdaptiveParams a{};
+    a.pool = pool.n; a.k = t->ad_k; a.c = t->ad_c;
+    a.px = t->px; a.py = t->py; a.pz = t->pz; a.pR = t->pR; a.pmask = t->pmask; a.res = t->pres;
+    a.cdf = t->pcdf; a.part = t->ppart; a.pool_batch = t->batch; a.idx = nullptr;
+    a.out = sampler_params(t, b);
+    a.out.index_offset = 0; a.out.batch_counter = t->pcounts + 3;
+    VariantCoef vc;
+    int nev = 0;
+    variant_coef(c.variant, &vc, &nev);
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (int rc = adaptive_enqueue(h, nev, vc, t->theta32, pool, false, a, st)) return rc;
   }
   AdamParams a{};
   a.theta = t->theta; a.m = t->m; a.v = t->v; a.grad = t->grad; a.sums = t->sums; a.theta32 = t->theta32;
@@ -84,12 +129,12 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool presample_next
   return 0;
 }
 
-static int trainer_capture(pinn_trainer* t, bool presample_next, cudaGraphExec_t* out) {
+static int trainer_capture(pinn_trainer* t, bool adaptive_now, bool presample_next, cudaGraphExec_t* out) {
   pinn_handle* h = t->h;
   cudaGraph_t g = nullptr;
   CU(h, cudaStreamBeginCapture(t->st, cudaStreamCaptureModeThreadLocal));
   const int64_t launches_before = h->launches;
-  int rc = trainer_enqueue(t, false, presample_next, t->st);
+  int rc = trainer_enqueue(t, false, adaptive_now, presample_next, t->st);
   h->launches = launches_before;  // capture does not launch; replays are counted in pinn_trainer_run
   cudaError_t e = cudaStreamEndCapture(t->st, &g);
   if (rc) { if (g) cudaGraphDestroy(g); return rc; }
@@ -98,6 +143,19 @@ static int trainer_capture(pinn_trainer* t, bool presample_next, cudaGraphExec_t
   cudaGraphDestroy(g);
   if (e != cudaSuccess) return fail(h, (int)e, "cudaGraphInstantiate");
   return 0;
+}
+
+// Pool buffers and the adaptive graphs (the stream is idle)
+static void trainer_free_adaptive(pinn_trainer* t) {
+  for (cudaGraphExec_t& g : t->graph_ad)
+    if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+  cudaFree(t->px); cudaFree(t->py); cudaFree(t->pz); cudaFree(t->pR); cudaFree(t->pres); cudaFree(t->pmask);
+  cudaFree(t->pcdf); cudaFree(t->pweights); cudaFree(t->ppart); cudaFree(t->pcounts);
+  t->px = t->py = t->pz = t->pR = t->pres = nullptr;
+  t->pmask = nullptr;
+  t->pcdf = t->pweights = t->ppart = nullptr;
+  t->pcounts = nullptr;
+  t->pool_factor = 0;
 }
 
 extern "C" {
@@ -124,6 +182,50 @@ int pinn_sample(pinn_handle* h, int64_t n, uint64_t seed, uint64_t batch, const 
   CU(h, launch_sample(s, true, st));
   h->launches += 2;
   return 0;
+}
+
+int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed, uint64_t batch,
+                         const float box[8], float cutoff, float bcutoff, float k, float c, float* pool_x, float* pool_y,
+                         float* pool_z, float* pool_R, uint8_t* pool_mask, float* pool_res, double* pool_cdf, float* x,
+                         float* y, float* z, float* R, uint8_t* mask, int64_t* idx, uint64_t* counts, double* weights,
+                         void* stream) {
+  if (!h) return PINN_EINVAL;
+  std::lock_guard<std::mutex> lk(h->mu);
+  if (n <= 0 || pool < n) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: need 0 < n <= pool");
+  if (!(k >= 0.0f) || !std::isfinite(k) || !(c >= 0.0f) || !std::isfinite(c))
+    return fail(h, PINN_EINVAL, "pinn_sample_adaptive: k and c must be finite and >= 0");
+  if (!theta || !box || !pool_x || !pool_y || !pool_z || !pool_R || !pool_mask || !pool_res || !pool_cdf || !x || !y || !z ||
+      !R || !mask || !counts || !weights)
+    return fail(h, PINN_EINVAL, "pinn_sample_adaptive: NULL pointer argument");
+  VariantCoef vc;
+  int nev = 0;
+  if (variant_coef(variant, &vc, &nev)) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: unknown variant");
+  DevGuard dev_guard(h->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long scratch_rows = (adaptive_scratch_doubles(pool) + NPART - 1) / NPART;
+  if (scratch_rows > 0x7fffffffll) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: pool too large");
+  pinn_workspace* ws = ws_for(h, st, std::max(h->sm_count, (int)scratch_rows));
+  if (!ws) return PINN_EINVAL;
+  unsigned long long* batch_counter = ws->counts + 2;  // [0..1] the pool's set sizes, [2] its batch index, [3] block ticket
+  set_u64_kernel<<<1, 1, 0, st>>>(batch_counter, (unsigned long long)batch);
+  CU(h, cudaGetLastError());
+  h->launches += 1;
+  SampleParams ps{};
+  ps.n = pool; ps.seed = seed; ps.batch_counter = batch_counter;
+  ps.xL = box[0]; ps.xR = box[1]; ps.yL = box[2]; ps.yR = box[3]; ps.zL = box[4]; ps.zR = box[5]; ps.RL = box[6]; ps.RR = box[7];
+  ps.cutoff = cutoff; ps.bcutoff = bcutoff;
+  ps.x = pool_x; ps.y = pool_y; ps.z = pool_z; ps.R = pool_R; ps.mask = pool_mask; ps.counts = ws->counts;
+  ps.weights = ws->weights; ps.ticket = batch_counter + 1; ps.reset_counts = 0;
+  AdaptiveParams a{};
+  a.pool = pool; a.k = k; a.c = c;
+  a.px = pool_x; a.py = pool_y; a.pz = pool_z; a.pR = pool_R; a.pmask = pool_mask; a.res = pool_res;
+  a.cdf = pool_cdf; a.part = ws->partials; a.pool_batch = batch_counter; a.idx = reinterpret_cast<long long*>(idx);
+  a.out = ps;
+  a.out.n = n; a.out.x = x; a.out.y = y; a.out.z = z; a.out.R = R; a.out.mask = mask;
+  a.out.counts = (unsigned long long*)counts; a.out.weights = weights;
+  // rad_scan_kernel has read the pool's batch index by the time the selection's finish moves this word on again
+  a.out.batch_counter = batch_counter;
+  return adaptive_enqueue(h, nev, vc, theta, ps, true, a, st);
 }
 
 int pinn_adam_step(pinn_handle* h, double* theta, double* m, double* v, const double* grad, const double* sums, float* theta32,
@@ -306,6 +408,7 @@ int pinn_trainer_destroy(pinn_trainer* t) {
   for (int a = 0; a < 2; a++)
     for (int b = 0; b < 2; b++)
       if (t->graph[a][b]) cudaGraphExecDestroy(t->graph[a][b]);
+  trainer_free_adaptive(t);
   for (int b = 0; b < 2; b++) {
     cudaFree(t->x[b]); cudaFree(t->y[b]); cudaFree(t->z[b]); cudaFree(t->R[b]); cudaFree(t->mask[b]);
     cudaFree(t->weights[b]); cudaFree(t->counts[b]);
@@ -353,6 +456,41 @@ int pinn_trainer_load_state(pinn_trainer* t, const double* theta, const double* 
   for (int a = 0; a < 2; a++)
     for (int b = 0; b < 2; b++)
       if (t->graph[a][b]) { cudaGraphExecDestroy(t->graph[a][b]); t->graph[a][b] = nullptr; }
+  for (cudaGraphExec_t& g : t->graph_ad)
+    if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+  return 0;
+}
+
+int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  if (pool_factor < 0 || !(k >= 0.0f) || !std::isfinite(k) || !(c >= 0.0f) || !std::isfinite(c))
+    return fail(h, PINN_EINVAL, "pinn_trainer_set_adaptive: pool_factor, k and c must be finite and >= 0");
+  if (pool_factor > 0 && (int64_t)pool_factor > INT64_MAX / 8 / t->cfg.n)
+    return fail(h, PINN_EINVAL, "pinn_trainer_set_adaptive: pool_factor * n too large");
+  if (dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_set_adaptive: adaptive sampling is not available with the data-parallel exchange");
+  DevGuard dev_guard(h->device);
+  CU(h, cudaStreamSynchronize(t->st));
+  trainer_free_adaptive(t);
+  if (pool_factor == 0) return 0;
+  const size_t N = (size_t)pool_factor * (size_t)t->cfg.n;
+#define AD_CU(call)                                                            \
+  do {                                                                         \
+    cudaError_t e__ = (call);                                                  \
+    if (e__ != cudaSuccess) {                                                  \
+      trainer_free_adaptive(t);                                                \
+      return fail(h, (int)e__, "pinn_trainer_set_adaptive: " #call);           \
+    }                                                                          \
+  } while (0)
+  AD_CU(cudaMalloc(&t->px, N * 4)); AD_CU(cudaMalloc(&t->py, N * 4)); AD_CU(cudaMalloc(&t->pz, N * 4));
+  AD_CU(cudaMalloc(&t->pR, N * 4)); AD_CU(cudaMalloc(&t->pres, N * 4)); AD_CU(cudaMalloc(&t->pmask, N));
+  AD_CU(cudaMalloc(&t->pcdf, N * 8)); AD_CU(cudaMalloc(&t->pweights, 4 * 8));
+  AD_CU(cudaMalloc(&t->ppart, (size_t)adaptive_scratch_doubles((long long)N) * 8));
+  AD_CU(cudaMalloc(&t->pcounts, 32)); AD_CU(cudaMemset(t->pcounts, 0, 32));
+#undef AD_CU
+  t->pool_factor = pool_factor; t->ad_k = k; t->ad_c = c;
+  t->ad_warmed = false;
   return 0;
 }
 
@@ -389,30 +527,37 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
   if (steps < 0) return fail(h, PINN_EINVAL, "pinn_trainer_run: steps must be >= 0");
   if (!resample && !t->have_batch) return fail(h, PINN_EINVAL, "pinn_trainer_run: no batch yet (resample = 0 needs pinn_trainer_set_batch or an earlier sampled step)");
   DevGuard dev_guard(h->device);
+  const bool adaptive = t->pool_factor > 0;
+  if (adaptive && dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_run: adaptive sampling is not available with the data-parallel exchange");
   auto resamples = [&](int64_t tt) { return resample && (tt % t->cfg.sc_sampling == 0) && (tt < t->cfg.freeze_after); };
   for (int64_t k = 0; k < steps; k++) {
     const int64_t tt = t->steps_issued;
     const bool rs = resamples(tt);
     bool sample_now = false;
-    if (rs) {
+    // adaptive: the draw needs the parameters this step starts from, so it goes in front of the step, never in the
+    // reduction kernel of the step before
+    const bool adaptive_now = rs && adaptive;
+    if (rs && !adaptive) {
       if (t->next_ready) { t->cur ^= 1; t->next_ready = false; }  // drawn while the previous step was reduced
       else sample_now = true;
     }
-    const bool presample_next = (k + 1 < steps) && resamples(tt + 1);
-    if (use_graph && t->warmed && !sample_now) {
-      cudaGraphExec_t& g = t->graph[t->cur][presample_next ? 1 : 0];
+    const bool presample_next = !adaptive && (k + 1 < steps) && resamples(tt + 1);
+    if (use_graph && t->warmed && !sample_now && (!adaptive_now || t->ad_warmed)) {
+      cudaGraphExec_t& g = adaptive_now ? t->graph_ad[t->cur] : t->graph[t->cur][presample_next ? 1 : 0];
       if (!g) {
-        int rc = trainer_capture(t, presample_next, &g);
+        int rc = trainer_capture(t, adaptive_now, presample_next, &g);
         if (rc) return rc;
       }
       CU(h, cudaGraphLaunch(g, t->st));
-      h->launches += 2;
+      h->launches += adaptive_now ? 2 + ADAPTIVE_LAUNCHES : 2;
     } else {
-      // plain launches: the first step ever (one-time kernel attributes are set outside any capture) and steps that
-      // start with the stand-alone sampler
-      int rc = trainer_enqueue(t, sample_now, presample_next, t->st);
+      // plain launches: the first step ever and the first adaptive step (one-time kernel attributes are set outside any
+      // capture) and steps that start with the stand-alone sampler
+      int rc = trainer_enqueue(t, sample_now, adaptive_now, presample_next, t->st);
       if (rc) return rc;
       t->warmed = true;
+      if (adaptive_now) t->ad_warmed = true;
     }
     if (presample_next) t->next_ready = true;
     if (rs) t->have_batch = true;

@@ -5,6 +5,7 @@ The reference loops stay usable unchanged through `patch_nn_ion` / `run_train_py
 which parity runs need); this module is the fast path for runs that do not need that stream:
 
     sample(...)              <->  train.py:26-39; sampling()+radial()+torch.where  poc/main.py:124-156, 390-393
+    sample_adaptive(...)        residual-adaptive batches (RAD) drawn from a pool of sample() points
     adam_step(...)           <->  optimizer.step() + best/history bookkeeping      train.py:58-72; poc/main.py:403-417
     Trainer                  <->  train()                                          train.py:21-72; poc/main.py:359-430
     train_trainpy / train_poc   convenience drivers with the reference's defaults and return values
@@ -49,6 +50,40 @@ def sample(n, seed, batch, box=BOX_POC, cutoff=0.005, bcutoff=17.5, device=None)
     return out
 
 
+def sample_adaptive(variant, theta, n, pool_factor=4, k=1.0, c=1.0, seed=0, batch=0, box=None, cutoff=0.005, bcutoff=17.5,
+                    device=None):
+    """Residual-adaptive batch (pinn_sample_adaptive): n points out of pool_factor * n uniform candidates
+    (= sample(pool_factor * n, seed, batch)), candidate i taken with probability proportional to
+    |res_i|^k * N / sum |res|^k + c, res = the residual of `theta` (packed parameters) there, by systematic resampling.
+    -> dict(x, y, z, R, mask, counts, weights as sample(); idx int64 (n,) pool index of each point; pool = dict(x, y, z,
+    R, mask) of the candidates; res float32 and cdf float64 (N,), the candidates' residuals and weight prefix sums)."""
+    variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
+    if box is None:
+        box = BOX_POC if variant == 0 else BOX_TRAINPY
+    h = _handle(device)
+    dev = torch.device("cuda", h.device)
+    N = int(pool_factor) * int(n)
+    th = torch.as_tensor(np.asarray(theta) if not torch.is_tensor(theta) else theta).detach()
+    th = th.to(device=dev, dtype=torch.float32).contiguous()
+    col = lambda m, dt=torch.float32: torch.empty(m, dtype=dt, device=dev)
+    pool = {k_: col(N) for k_ in "xyzR"}
+    pool["mask"] = col(N, torch.uint8)
+    out = {k_: col(n) for k_ in "xyzR"}
+    out["mask"] = col(n, torch.uint8)
+    out["counts"] = torch.zeros(2, dtype=torch.int64, device=dev)
+    out["weights"] = col(3, torch.float64)
+    out["idx"] = col(n, torch.int64)
+    out["pool"], out["res"], out["cdf"] = pool, col(N), col(N, torch.float64)
+    b = (ctypes.c_float * 8)(*box)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    rc = h.L.pinn_sample_adaptive(h.h, variant, _ptr(th), n, N, seed, batch, b, cutoff, bcutoff, k, c,
+                                  *[_ptr(pool[k_]) for k_ in ("x", "y", "z", "R", "mask")], _ptr(out["res"]),
+                                  _ptr(out["cdf"]), *[_ptr(out[k_]) for k_ in ("x", "y", "z", "R", "mask", "idx", "counts",
+                                                                              "weights")], ctypes.c_void_p(stream))
+    h.check(rc, "pinn_sample_adaptive")
+    return out
+
+
 class AdamState:
     """Device state of the fused Adam step (float64, like the reference's parameters)."""
 
@@ -87,7 +122,7 @@ class Trainer:
 
     def __init__(self, variant, n, theta0, seed=12345, lr=8e-3, betas=(0.9, 0.999), eps=1e-8, box=None, cutoff=0.005,
                  bcutoff=17.5, grad_mask=0xFFFF, best_mode=None, best_after=0, sc_sampling=1, freeze_after=INT64_MAX,
-                 history_capacity=0, history_mean_E=None, device=None, handle=None):
+                 history_capacity=0, history_mean_E=None, device=None, handle=None, adaptive=None):
         variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
         self.h = handle if handle is not None else _handle(device)   # default: the cached per-device Handle
         if box is None:
@@ -109,6 +144,16 @@ class Trainer:
         self.h.check(rc, "pinn_trainer_create")
         self.t = tp
         self._step_base = 0
+        if adaptive:
+            self.set_adaptive(**adaptive)
+
+    def set_adaptive(self, pool_factor=4, k=1.0, c=1.0):
+        """Residual-adaptive batches (pinn_trainer_set_adaptive): every resampling step draws its n points from
+        pool_factor * n candidates in proportion to |res|^k / mean |res|^k + c at the current parameters; pool_factor=0
+        turns it off.  The history and best-model record are then evaluated on the adaptive batches, so Ltot is not
+        comparable with a uniform run's."""
+        self.h.check(self.h.L.pinn_trainer_set_adaptive(self.t, int(pool_factor), float(k), float(c)),
+                     "pinn_trainer_set_adaptive")
 
     def load_state(self, theta, m=None, v=None, step=0):
         """Resume: parameters, Adam moments (None = zeros) and the number of optimizer steps already done.  The resumed run
@@ -195,13 +240,15 @@ def init_poc(seed=0):
     return P.pack_poc(ts, dtype=torch.float64).numpy()
 
 
-def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_tune=False, use_graph=False, log_every=0):
+def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_tune=False, use_graph=False, log_every=0,
+                  adaptive=None):
     """train(params, lr, epochs) of train.py on the device.  Like the reference it evaluates epochs+1 losses, takes `epochs`
-    optimizer steps and returns the parameters of the best loss seen (train.py:58-69).  Returns (theta_best, info)."""
+    optimizer steps and returns the parameters of the best loss seen (train.py:58-69).  Returns (theta_best, info).
+    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive)."""
     if theta0 is None:
         theta0 = init_trainpy(seed)
     mask = P.FINE_TUNE_GRAD_MASK if fine_tune else 0xFFFF  # train.py:111 (commented) trains the E-net tensors only
-    tr = Trainer("trainpy", n, theta0, seed=seed, lr=lr, grad_mask=mask, history_capacity=epochs + 1)
+    tr = Trainer("trainpy", n, theta0, seed=seed, lr=lr, grad_mask=mask, history_capacity=epochs + 1, adaptive=adaptive)
     done = 0
     while done < epochs:
         k = min(log_every or epochs, epochs - done)
@@ -222,9 +269,10 @@ def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_t
     return best, info
 
 
-def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False):
+def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False, adaptive=None):
     """train(params, loadWeights, freezeUnits) of poc/main.py:359-430 on the device.  `params` uses the reference's keys
-    (set_params(), poc/main.py:14-45).  Returns (theta_last, theta_saved or None, lossDictionary like poc/main.py:422-427)."""
+    (set_params(), poc/main.py:14-45).  Returns (theta_last, theta_saved or None, lossDictionary like poc/main.py:422-427).
+    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive)."""
     pr = {"xL": -18, "xR": 18, "yL": -18, "yR": 18, "zL": -18, "zR": 18, "RxL": 0.2, "RxR": 4, "cutOff": 0.005,
           "BCcutoff": 17.5, "sc_sampling": 1, "n_train": 100000, "epochs": 5000, "lr": 8e-3}
     pr.update(params or {})
@@ -237,7 +285,7 @@ def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False):
     tr = Trainer("poc", int(pr["n_train"]), theta0, seed=seed, lr=pr["lr"], box=box, cutoff=pr["cutOff"],
                  bcutoff=pr["BCcutoff"], grad_mask=P.FINE_TUNE_GRAD_MASK if freezeUnits else 0xFFFF, best_mode=1,
                  best_after=best_after, sc_sampling=int(pr["sc_sampling"]), freeze_after=freeze_after,
-                 history_capacity=epochs, history_mean_E=False)
+                 history_capacity=epochs, history_mean_E=False, adaptive=adaptive)
     tr.run(epochs, use_graph=use_graph)
     r = tr.read()
     tr.close()
