@@ -16,7 +16,8 @@ def weights(res, k, c):
     k, c = float(np.float32(k)), float(np.float32(c))
     fin = np.isfinite(r)
     q = np.zeros_like(r)
-    q[fin] = np.abs(r[fin]) ** k
+    with np.errstate(over="ignore"):  # |res|^k past the float64 range is inf, as on the device
+        q[fin] = np.abs(r[fin]) ** k
     Q = q.sum()
     if not (Q > 0.0 and np.isfinite(Q)):
         return np.ones_like(r)

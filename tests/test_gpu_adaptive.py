@@ -11,6 +11,7 @@ import torch
 
 import pinn_for_quantum_wavefunction_surfaces_b200 as pk
 from oracle import adaptive as ad
+from oracle import layout
 from oracle import philox as ph
 
 pytestmark = pytest.mark.gpu
@@ -20,7 +21,12 @@ AD = dict(pool_factor=4, k=1.0, c=1.0)
 @pytest.fixture(scope="module")
 def thetas(golden_dir):
     ck = np.load(os.path.join(golden_dir, "checkpoints.npz"))
-    return {"trained": ck["ionHsym"], "init": pk.init_poc(0)}
+    tp = np.load(os.path.join(golden_dir, "trainpy_n2048.npz"))["theta"]  # train.py's init rule, seed 12345
+    # bo near the float32 maximum: q N overflows near the nuclei and stays finite far from them, so the residual is
+    # non-finite on part of every pool
+    huge = ck["ionHsym"].astype(np.float32)
+    huge[layout.offsets()[5]] = 3.0e38
+    return {"trained": ck["ionHsym"], "init": pk.init_poc(0), "trainpy_init": tp, "huge_bo": huge}
 
 
 def _np(t):
@@ -43,14 +49,26 @@ def _trainer_batch(tr, n):
     return [_np(c) for c in cols]
 
 
-@pytest.mark.parametrize("which", ["trained", "init"])
-@pytest.mark.parametrize("variant", ["poc", "trainpy"])
-def test_draw_against_the_oracle(variant, which, thetas):
-    n, seed, batch, k, c = 5000, 77, 9, 1.0, 1.0
+# (n, pool_factor, k, c) beyond the plain draw: one output; a pool equal to n; 513 scan blocks (three rounds of the
+# offset fold) and the grid-stride loop of the selection; non-integer k; c = 0; k = 1e30, where |res|^k is 0 or inf and
+# the draw falls back to uniform weights; and residuals that are not finite on part of the pool
+DRAWS = {"": (5000, 4, 1.0, 1.0), "n1": (1, 4, 1.0, 1.0), "pool_eq_n": (4097, 1, 1.0, 1.0),
+         "fold3": ((1 << 19) + 3, 4, 1.0, 1.0), "k0.5": (5000, 4, 0.5, 1.0), "k1.7": (5000, 4, 1.7, 1.0),
+         "c0": (5000, 4, 1.0, 0.0), "k1e30": (5000, 4, 1e30, 1.0), "nonfinite": (5000, 4, 1.0, 1.0)}
+DRAW_CASES = [pytest.param(variant, which, case, id="-".join([variant, which] + ([case] if case else [])))
+              for case in DRAWS
+              for which in {"k1e30": ["trained", "init", "trainpy_init", "huge_bo"], "nonfinite": ["trained"]}.get(case, ["trained", "init"])
+              for variant in ["poc", "trainpy"]]
+
+
+@pytest.mark.parametrize("variant, which, case", DRAW_CASES)
+def test_draw_against_the_oracle(variant, which, case, thetas):
+    n, pf, k, c = DRAWS[case]
+    seed, batch = 77, 9
     box = pk.trainer.BOX_POC if variant == "poc" else pk.trainer.BOX_TRAINPY
-    theta = thetas[which]
-    out = pk.sample_adaptive(variant, theta, n, pool_factor=4, k=k, c=c, seed=seed, batch=batch, box=box)
-    N = 4 * n
+    theta = thetas["huge_bo" if case == "nonfinite" else which]  # (huge_bo at k = 1e30: finite |res| > 1, Q = inf)
+    out = pk.sample_adaptive(variant, theta, n, pool_factor=pf, k=k, c=c, seed=seed, batch=batch, box=box)
+    N = pf * n
     # the pool is the uniform sampler's batch `batch` of N points, bit for bit
     x, y, z, R, mask, _ = ph.sample_batch(N, seed, batch, box=box)
     pool = {kk: _np(v) for kk, v in out["pool"].items()}
@@ -67,6 +85,18 @@ def test_draw_against_the_oracle(variant, which, thetas):
     want_cdf = np.cumsum(ad.weights(res, k, c))
     assert np.all(np.abs(cdf - want_cdf) <= 1e-12 * want_cdf)
     assert np.all(np.diff(cdf) >= 0.0)
+    r = np.abs(res.astype(np.float64))
+    if case == "k1e30":  # Q = 0 when every finite |res| < 1, inf when one exceeds 1: uniform either way
+        rmax = r[np.isfinite(r)].max()
+        print("k = 1e30, %s %s: max|res| %.3g -> Q = %s" % (which, variant, rmax, "inf" if rmax > 1 else "0"))
+        assert rmax != 1.0 and (rmax > 1.0) == (which == "huge_bo")
+        assert np.array_equal(cdf, np.arange(1, N + 1, dtype=np.float64))
+    if case == "nonfinite":  # the weight of a non-finite residual is c alone
+        fin = np.isfinite(res)
+        print("non-finite residuals: %d of %d" % ((~fin).sum(), N))
+        assert fin.any() and not fin.all()
+        step = np.diff(cdf, prepend=0.0)[~fin]
+        assert np.all(np.abs(step - c) <= 4 * np.spacing(cdf[~fin]))
     # selection: exactly the oracle's over the device's own cdf
     idx = _np(out["idx"])
     assert np.array_equal(idx, ad.select(cdf, n, ad.u0(N, seed, batch)))
@@ -76,12 +106,12 @@ def test_draw_against_the_oracle(variant, which, thetas):
     assert np.array_equal(m, pool["mask"][idx])
     c1, c2 = int((m & 1).sum()), int((m >> 1 & 1).sum())
     assert _np(out["counts"]).tolist() == [c1, c2]
-    assert _np(out["weights"]).tolist() == [1.0 / n, 1.0 / c1, 1.0 / c2]
+    with np.errstate(divide="ignore"):  # a set can be empty at n = 1: its weight is inf
+        assert _np(out["weights"]).tolist() == (1.0 / np.array([n, c1, c2], np.float64)).tolist()
 
 
-def test_counts_within_floor_and_ceil_at_2_18(thetas):
-    n = 1 << 18
-    out = pk.sample_adaptive("poc", thetas["trained"], n, pool_factor=4, k=1.0, c=1.0, seed=3, batch=1)
+def check_counts(thetas, n, pf, k, c):
+    out = pk.sample_adaptive("poc", thetas["trained"], n, pool_factor=pf, k=k, c=c, seed=3, batch=1)
     cdf = _np(out["cdf"])
     P = np.diff(cdf, prepend=0.0) / cdf[-1]
     cnt = np.bincount(_np(out["idx"]), minlength=cdf.size)
@@ -94,8 +124,18 @@ def test_counts_within_floor_and_ceil_at_2_18(thetas):
         r2 = np.sqrt((x + R) ** 2 + y ** 2 + z ** 2)
         return float(np.mean(np.minimum(r1, r2) < 4.0))
 
-    print("share within 4 bohr of a nucleus (trained weights, k=1, c=1): batch %.4f, pool %.4f"
-          % (near(out), near(out["pool"])))
+    print("share within 4 bohr of a nucleus (trained weights, n=%d, k=%g, c=%g): batch %.4f, pool %.4f"
+          % (n, k, c, near(out), near(out["pool"])))
+
+
+def test_counts_within_floor_and_ceil_at_2_18(thetas):
+    check_counts(thetas, 1 << 18, 4, 1.0, 1.0)
+
+
+@pytest.mark.parametrize("case", [c for c in DRAWS if c not in ("", "k1e30", "nonfinite")])
+def test_counts_within_floor_and_ceil_of_other_draws(case, thetas):
+    """The count bounds at the draws of DRAWS whose weights are not uniform."""
+    check_counts(thetas, *DRAWS[case])
 
 
 def test_two_calls_and_a_graph_replay_give_the_same_bits(thetas):

@@ -18,6 +18,7 @@ import torch
 import pinn_for_quantum_wavefunction_surfaces_b200 as pk
 from oracle import closed_form as cf
 from oracle import layout
+from oracle import pointwise as pw
 from oracle import ref_autograd as ra
 
 pytestmark = pytest.mark.gpu
@@ -121,6 +122,9 @@ def test_golden_reference_outputs_poc(golden_dir, ck):
         assert rel(f["lap"].cpu().numpy(), g[tag + "_lap"]) < 1e-5
         assert rel(f["hpsi"].cpu().numpy(), g[tag + "_hpsi"]) < 1e-5
         assert rel(f["E"].cpu().numpy(), g[tag + "_E"]) < 1e-5
+        keys = ("psi", "lap", "hpsi", "E")
+        pw.check("golden poc " + tag, {k: f[k].cpu().numpy() for k in keys}, {k: g[tag + "_" + k] for k in keys},
+                 pw.magnitudes("poc", ck[tag], *a64, rounded_weights=True), pw.C_KERNEL, a64)
 
 
 def test_golden_reference_outputs_trainpy(golden_dir):
@@ -137,6 +141,9 @@ def test_golden_reference_outputs_trainpy(golden_dir):
     f = pk.fields("trainpy", *[t(g[k]) for k in "xyzR"], t(g["theta"]))
     assert rel(f["psi"].cpu().numpy(), g["psi"]) < 1e-5
     assert rel(f["res"].cpu().numpy(), g["res"]) < 1e-5
+    a64 = [g[k] for k in "xyzR"]
+    pw.check("golden trainpy", {k: f[k].cpu().numpy() for k in ("psi", "res")}, {k: g[k].reshape(-1) for k in ("psi", "res")},
+             pw.magnitudes("trainpy", g["theta"], *a64, rounded_weights=True), pw.C_KERNEL, a64)
 
 
 @pytest.mark.parametrize("variant", [0, 1])
@@ -180,8 +187,12 @@ def test_fields_vs_oracle(variant, ck, init_theta):
         t = lambda a: torch.from_numpy(a).to(dev())
         out = pk.fields(variant, *[t(a) for a in a32], t(th32))
         torch.cuda.synchronize()
-        for k in ("psi", "lap", "res", "E", "hpsi"):
-            assert rel(out[k].cpu().numpy(), f[k]) < 1e-5, (k, rel(out[k].cpu().numpy(), f[k]))
+        got = {k: out[k].cpu().numpy() for k in pw.OUTPUTS}
+        for k in pw.OUTPUTS:
+            assert rel(got[k], f[k]) < 1e-5, (k, rel(got[k], f[k]))
+        a64 = [a.astype(np.float64) for a in a32]
+        name = "poc" if variant == 0 else "trainpy"
+        pw.check("fields %s" % name, got, f, pw.magnitudes(name, th32.astype(np.float64), *a64), pw.C_KERNEL, a64)
 
 
 def test_points_at_the_clamp_distance(init_theta):

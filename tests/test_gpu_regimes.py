@@ -9,7 +9,7 @@ entry has to be as accurate as a large one.
 Regimes are built from train.py's init vector by shifting one layer's biases (and shrinking a unit's weights where its
 input range would not fit in the band) so that every unit's pre-activation lies in the band for ANY point: the inputs of
 a layer are bounded (exp(-r) and sigmoids in [0, 1], R in the union of the two samplers' ranges [0.2, 4]), not only the
-points sampled here.  The CPU test checks the bands with the float64 oracle on the points the GPU tests use.
+points sampled here (oracle/regimes.py).  The CPU test checks the bands with the float64 oracle on the points the GPU tests use.
 """
 import ctypes
 import os
@@ -22,48 +22,13 @@ import torch
 import pinn_for_quantum_wavefunction_surfaces_b200 as pk
 from oracle import closed_form as cf
 from oracle import layout
+from oracle import pointwise as pw
 from oracle import ref_autograd as ra
+from oracle.regimes import BAND, LAYERS, REGIMES, unit_signs, regime_theta
 
 OFFS = layout.offsets() + [1521]
 N = 4096 + 37                     # the last 128-point super-tile is ragged
 SEED = 7
-BAND = (8.0, 12.0)
-HALF = 1.8                        # every unit is put in [10 - HALF, 10 + HALF] (or its negative): inside BAND with margin
-R_RANGE = (0.2, 4.0)              # poc samples R in [0.2, 4], train.py in [0.2, 3]
-
-# sigmoid layer: (weight tensor, bias tensor) in the canonical layout; inputs of the base and E-net second layers are
-# sigmoids, of the base first layer exp(-r1), exp(-r2), of the E-net and gate first layers R
-LAYERS = {"base_L1": (0, 1), "base_L2": (2, 3), "enet_L1": (6, 7), "enet_L2": (8, 9), "gate_L1": (12, 13)}
-INPUT_RANGE = {"base_L1": (0.0, 1.0), "base_L2": (0.0, 1.0), "enet_L1": R_RANGE, "enet_L2": (0.0, 1.0), "gate_L1": R_RANGE}
-
-
-def _unit_signs(layer, sign):
-    n = layout.POC_TENSORS[LAYERS[layer][1]][1][0]
-    if sign != "mixed":
-        return np.full(n, 1.0 if sign == "pos" else -1.0)
-    # the mixed regime saturates all five layers at once, two units in three on the positive side
-    return np.where(np.arange(n) % 3 == 2, -1.0, 1.0)
-
-
-REGIMES = {f"{layer}_{sign}": {layer: sign} for layer in LAYERS for sign in ("pos", "neg")}
-REGIMES["mixed"] = {layer: "mixed" for layer in LAYERS}
-
-
-def regime_theta(init, name):
-    """init (1521,) float64 -> the regime's weights, rounded to float32 (what the kernel is given)."""
-    P = [p.copy() for p in layout.unpack_poc(np.asarray(init, np.float64))]
-    for layer, sign in REGIMES[name].items():
-        iw, ib = LAYERS[layer]
-        W = P[iw].reshape(P[ib].size, -1)
-        lo_in, hi_in = INPUT_RANGE[layer]
-        lo = np.minimum(W * lo_in, W * hi_in).sum(1)          # range of W x over every admissible input x
-        hi = np.maximum(W * lo_in, W * hi_in).sum(1)
-        shrink = np.minimum(1.0, 2 * HALF / np.maximum(hi - lo, 1e-300))
-        W *= shrink[:, None]
-        mid = 0.5 * (lo + hi) * shrink
-        P[iw] = W.reshape(P[iw].shape)
-        P[ib] = 10.0 * _unit_signs(layer, sign) - mid
-    return layout.pack_poc(P).astype(np.float32)
 
 
 def sample(variant):
@@ -104,7 +69,7 @@ def test_regime_reaches_its_band(regime, variant, init_theta):
     th = regime_theta(init_theta, regime)
     u = preactivations(th, variant, sample(variant)[0])
     for layer, sign in REGIMES[regime].items():
-        s = _unit_signs(layer, sign)
+        s = unit_signs(layer, sign)
         us = u[layer] * s                                      # folded onto the positive side
         assert us.min() >= BAND[0] and us.max() <= BAND[1], (layer, us.min(), us.max())
     for layer in set(LAYERS) - set(REGIMES[regime]):           # the other layers stay where the init put them
@@ -180,6 +145,8 @@ def test_step_and_fields_at_saturated_sigmoids(regime, variant, init_theta):
     bad = {k: v for k, v in {**lerr, **ferr}.items() if not v < 1e-5}
     bad.update({k: v for k, v in errs.items() if not (v[0] < 1e-5 and v[1] < 1e-4)})
     assert not bad, bad
+    pw.check("fields %s %s" % (regime, name), {k: out[k].cpu().numpy() for k in pw.OUTPUTS}, f,
+             pw.magnitudes(name, th32.astype(np.float64), *a64), pw.C_KERNEL, a64)
 
 
 @pytest.mark.gpu

@@ -13,6 +13,7 @@ from oracle import layout
 from oracle import philox as ph
 from oracle import simpson as sp
 from oracle import train_loop as tl
+from oracle.regimes import REGIMES, regime_theta
 
 pytestmark = pytest.mark.gpu
 OFFS = layout.offsets() + [1521]
@@ -485,8 +486,41 @@ def test_calculate_E_R_against_the_papers_table(ck, golden_dir):
     assert np.all(np.isfinite(d["dEdR_HF"]))
 
 
+def enet_curve_reference(th32, R):
+    """E, dE/dR, d2E/dR2 and the gate in float64 with sigma' = e^-u / (1 + e^-u)^2 and sigma'' = e^-u (e^-u - 1) /
+    (1 + e^-u)^3: accurate where a sigmoid saturates, where s (1 - s) keeps only e^|u| 2^-53 of relative accuracy."""
+    P = layout.unpack_poc(th32.astype(np.float64))
+
+    def sig(u):
+        e = np.exp(-u)
+        return 1.0 / (1.0 + e), e / (1.0 + e) ** 2, e * (e - 1.0) / (1.0 + e) ** 3
+
+    w1 = P[6][:, 0]
+    s, sp, spp = sig(R[:, None] * w1 + P[7])
+    v, vp, vpp = s @ P[8].T + P[9], (sp * w1) @ P[8].T, (spp * w1 * w1) @ P[8].T
+    t, tp, tpp = sig(v)
+    wE = P[10][0]
+    g = sig(R[:, None] * P[12][:, 0] + P[13])[0] @ P[14][0] + P[15][0]
+    return dict(E=t @ wE + P[11][0], dE=(tp * vp) @ wE, d2E=(tpp * vp * vp + tp * vpp) @ wE, gate=g)
+
+
+@pytest.mark.parametrize("regime", [r for r in sorted(REGIMES) if r.startswith(("enet", "gate"))] + ["mixed"])
+def test_enet_curve_at_saturated_sigmoids(regime, init_theta):
+    """The E-net and gate layers saturated, u in [8, 12] or [-12, -8] (oracle/regimes.py), at the bars of
+    test_enet_curve_vs_autograd against the exp-form float64 reference."""
+    Rs = np.linspace(0.2, 4.0, 39)
+    th32 = regime_theta(init_theta, regime)
+    c, ref = pk.analysis.enet_curve(th32, Rs), enet_curve_reference(th32, Rs)
+    errs = {k: rel(c[k], ref[k]) for k in ("E", "dE", "d2E", "gate")}
+    print("%s: %s" % (regime, " ".join("%s %.1e" % kv for kv in errs.items())))
+    assert errs["E"] < 1e-12 and errs["dE"] < 1e-11 and errs["d2E"] < 1e-10 and errs["gate"] < 1e-12, errs
+
+
 def test_enet_curve_vs_autograd(ck):
+    Rs = np.linspace(0.2, 4.0, 39)
     th32 = ck["ionHsym_fineTune"].astype(np.float32)
+    c, ref = pk.analysis.enet_curve(th32, Rs), enet_curve_reference(th32, Rs)
+    assert rel(c["dE"], ref["dE"]) < 1e-11 and rel(c["d2E"], ref["d2E"]) < 1e-10
     R = torch.linspace(0.2, 4.0, 39, dtype=torch.float64, requires_grad=True)
     P = [torch.tensor(a.astype(np.float64)) for a in layout.unpack_poc(th32.astype(np.float64))]
     e = torch.sigmoid(R[:, None] * P[6][:, 0][None, :] + P[7][None, :])
