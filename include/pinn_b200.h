@@ -40,6 +40,7 @@
 #ifndef PINN_B200_H
 #define PINN_B200_H
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -340,6 +341,65 @@ int pinn_trainer_batch(pinn_trainer* t, float** x, float** y, float** z, float**
  * the data-parallel exchange is on (pinn_trainer_run also refuses an adaptive trainer then). */
 int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c);
 void* pinn_trainer_stream(pinn_trainer* t);
+
+/*
+ * L-BFGS: torch.optim.LBFGS.step(closure) of torch 2.11 (torch/optim/lbfgs.py with _strong_wolfe and _cubic_interpolate)
+ * in float64 on the device, decision for decision, as a machine that advances by ONE closure evaluation per launch and
+ * needs no host synchronisation inside a .step() call.  The closure is Ltot and its gradient at theta.
+ *
+ * The state is caller-owned device memory of pinn_lbfgs_state_bytes(history_size) bytes; all zero bytes is a fresh
+ * optimizer (torch's empty state), and d, t, the history, H_diag, prev_flat_grad, prev_loss, n_iter and func_evals
+ * persist in it across calls.  Keep history_size the same for the life of a state.  Its first 8 doubles are the status:
+ *   [0] n_iter (torch's state["n_iter"])   [1] func_evals (state["func_evals"])   [2] evaluations in this call
+ *   [3] done (1 once the call has finished)  [4] reason (PINN_LBFGS_*)   [5] loss (torch's `loss` when it finished)
+ *   [6] iterations in this call            [7] step length of the point requested last (0 for the first evaluation)
+ * A call:  pinn_lbfgs_begin requests an evaluation at theta (it writes theta32 = (float)theta).  Then, until done: evaluate
+ * the loss and gradient at the requested point (sums[0] = loss, grad = its 1521 doubles; a frozen entry has gradient 0, as
+ * torch's _gather_flat_grad gives for a parameter without .grad) and call pinn_lbfgs_advance, which consumes it and
+ * writes the next point to evaluate into theta (float64) and theta32, or finishes: theta = torch's final iterate.  After
+ * done, pinn_lbfgs_advance changes nothing.  A call takes at most max_eval evaluations, or max_eval + 1 with the line
+ * search (torch's line search always evaluates its first trial, even when max_eval has been reached).
+ * Every reduction has a fixed order: the same inputs give the same bits on every run and under graph replay.
+ * All pointers are device memory; PINN_EINVAL, with nothing launched, for a NULL pointer or a bad config.
+ */
+typedef struct pinn_lbfgs_config {
+  double lr;                /* torch: lr = 1 */
+  int max_iter;             /* 20; >= 1 */
+  int max_eval;             /* <= 0: torch's default max_iter * 5 / 4 */
+  int history_size;         /* 100; >= 1 */
+  int line_search;          /* 0: line_search_fn = None (fixed step); 1: "strong_wolfe" */
+  double tolerance_grad;    /* 1e-7 */
+  double tolerance_change;  /* 1e-9 (the line search keeps its own 1e-9, like torch) */
+} pinn_lbfgs_config;
+/* status[4]: why the call finished, in the order torch tests */
+#define PINN_LBFGS_RUNNING 0
+#define PINN_LBFGS_OPTIMAL_AT_START 1         /* max|g| <= tolerance_grad at the first evaluation */
+#define PINN_LBFGS_DIRECTIONAL_DERIVATIVE 2   /* g.d > -tolerance_change */
+#define PINN_LBFGS_MAX_ITER 3
+#define PINN_LBFGS_MAX_EVAL 4
+#define PINN_LBFGS_TOLERANCE_GRAD 5           /* max|g| <= tolerance_grad after a step */
+#define PINN_LBFGS_STEP_CHANGE 6              /* lack of progress: max|t d| <= tolerance_change */
+#define PINN_LBFGS_LOSS_CHANGE 7              /* lack of progress: |loss - prev_loss| < tolerance_change */
+#define PINN_LBFGS_SLOTS_EXHAUSTED 8          /* safety stop: more evaluations than the call can take (not expected) */
+size_t pinn_lbfgs_state_bytes(int history_size); /* 0 for history_size < 1 */
+int pinn_lbfgs_begin(pinn_handle* h, void* state, const pinn_lbfgs_config* cfg, const double* theta, float* theta32,
+                     void* stream);
+int pinn_lbfgs_advance(pinn_handle* h, void* state, const double* sums, const double* grad, double* theta, float* theta32,
+                       void* stream);
+/* One .step() call of the trainer on its current batch (resample = 1: the trainer's sampler draws the next batch first;
+ * 0: the batch is kept, PINN_EINVAL if there is none yet).  Each evaluation is the step kernel at theta32, the reduction
+ * (no Adam, no batch drawn) and the L-BFGS kernel, with the trainer's grad_mask.  use_graph = 0 enqueues every slot the
+ * call may take (max_eval, + 1 with the line search): slots after termination change no state, but their step kernels
+ * still run.  use_graph = 1 replays one evaluation as the body of a CUDA conditional WHILE node, and the L-BFGS kernel
+ * ends the loop when the call finishes, so nothing runs past the end.  The first L-BFGS evaluation of a trainer runs as
+ * plain launches.  Adam's moments and step counter, the best-model record and the history are not touched, so Adam can
+ * run again afterwards; pinn_trainer_load_state resets the L-BFGS state.  The state is allocated on first use and again
+ * (fresh) when history_size changes, in this call.  PINN_ENOTSUP with the data-parallel exchange on, and for resample = 1
+ * with adaptive sampling on. */
+int pinn_trainer_run_lbfgs(pinn_trainer* t, const pinn_lbfgs_config* cfg, int resample, int use_graph);
+/* Synchronise; status: the 8 doubles above (all 0 before the first call); trace: up to `rows` rows of the last call,
+ * one per evaluation: {Ltot, Lpde, Lbc, step length of the point}.  Either may be NULL. */
+int pinn_trainer_read_lbfgs(pinn_trainer* t, double* status, double* trace, int64_t rows);
 
 /*
  * E(R) of the E-net with its first and second derivative (autograd in poc/main.py:1324-1332) and the gate g(R)

@@ -11,7 +11,8 @@ call sites:
 * ``fields``          - fused ``parametricPsi`` + ``hamiltonian`` (poc/main.py:321, 118)
 * ``patch_nn_ion``    - monkey-patches an ``NN_ion`` class so the reference training loop runs unchanged
 * ``run_train_py``    - runs the reference ``train.py`` with lines 41-57 routed through the kernel
-* ``trainer``         - device-resident loop: Philox sampler, fused Adam, CUDA-graph replay (train.py:21-72; poc/main.py:359-430)
+* ``trainer``         - device-resident loop: Philox sampler, fused Adam, CUDA-graph replay (train.py:21-72; poc/main.py:359-430),
+  and a device-resident torch.optim.LBFGS (``Trainer.run_lbfgs``, ``LBFGSState``)
 * ``analysis``        - dense-grid energies / Hellmann-Feynman force / E(R) curve (poc/main.py:438-517, 639-676; energy.py)
 * ``convert``         - ``model.bin`` and ``.pt`` containers <-> packed parameters
 
@@ -25,12 +26,12 @@ from .ops import (PinnLossPoc, PinnLossTrainPy, loss_poc, loss_trainpy, fields, 
                   indices_to_mask, HostStep)
 from .patch import patch_nn_ion, run_train_py, trainpy_patched_source
 from . import analysis, convert, trainer
-from .trainer import Trainer, AdamState, adam_step, sample, sample_adaptive, train_trainpy, train_poc, init_trainpy, init_poc
+from .trainer import Trainer, AdamState, adam_step, LBFGSState, lbfgs_begin, lbfgs_advance, sample, sample_adaptive, train_trainpy, train_poc, init_trainpy, init_poc
 
 __all__ = [
     "N_THETA", "POC_TENSOR_NAMES", "TRAINPY_TENSOR_NAMES", "pack_poc", "unpack_poc", "pack_trainpy",
     "unpack_trainpy", "FINE_TUNE_GRAD_MASK", "lib", "Handle", "PinnError", "library_path", "bind_host_to_device_numa", "PinnLossPoc",
     "PinnLossTrainPy", "loss_poc", "loss_trainpy", "fields", "loss_and_grad_raw", "indices_to_mask", "HostStep",
     "patch_nn_ion", "run_train_py", "trainpy_patched_source", "analysis", "convert", "trainer", "Trainer", "AdamState",
-    "adam_step", "sample", "sample_adaptive", "train_trainpy", "train_poc", "init_trainpy", "init_poc",
+    "adam_step", "LBFGSState", "lbfgs_begin", "lbfgs_advance", "sample", "sample_adaptive", "train_trainpy", "train_poc", "init_trainpy", "init_poc",
 ]

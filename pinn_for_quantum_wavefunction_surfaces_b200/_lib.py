@@ -13,7 +13,8 @@ EXPORTS = [
     "pinn_loss_fwd_bwd_tensors", "pinn_mask_from_index_sets", "pinn_measure_fp32_peak", "pinn_step_kernel_clock",
     "pinn_sample", "pinn_sample_adaptive", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_spheroidal_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
     "pinn_trainer_load_state", "pinn_trainer_set_batch", "pinn_trainer_run", "pinn_trainer_read", "pinn_trainer_batch",
-    "pinn_trainer_stream", "pinn_trainer_set_adaptive",
+    "pinn_trainer_stream", "pinn_trainer_set_adaptive", "pinn_lbfgs_state_bytes", "pinn_lbfgs_begin", "pinn_lbfgs_advance",
+    "pinn_trainer_run_lbfgs", "pinn_trainer_read_lbfgs",
     "pinn_host_timing", "pinn_dp_init", "pinn_dp_connect", "pinn_dp_connect_local", "pinn_dp_enable", "pinn_dp_status", "pinn_dp_set_timeout", "pinn_dp_shutdown",
 ]
 
@@ -27,6 +28,13 @@ class TrainConfig(ctypes.Structure):
                 ("zL", ctypes.c_float), ("zR", ctypes.c_float), ("RL", ctypes.c_float), ("RR", ctypes.c_float),
                 ("cutoff", ctypes.c_float), ("bcutoff", ctypes.c_float), ("grad_mask", ctypes.c_uint32),
                 ("lr", ctypes.c_double), ("beta1", ctypes.c_double), ("beta2", ctypes.c_double), ("eps", ctypes.c_double)]
+
+
+class LBFGSConfig(ctypes.Structure):
+    """pinn_lbfgs_config of include/pinn_b200.h"""
+    _fields_ = [("lr", ctypes.c_double), ("max_iter", ctypes.c_int), ("max_eval", ctypes.c_int),
+                ("history_size", ctypes.c_int), ("line_search", ctypes.c_int), ("tolerance_grad", ctypes.c_double),
+                ("tolerance_change", ctypes.c_double)]
 
 
 class PinnError(RuntimeError):
@@ -123,6 +131,16 @@ def lib():
         L.pinn_trainer_stream.restype = vp
         L.pinn_trainer_set_adaptive.argtypes = [vp, i32, f32, f32]
         L.pinn_trainer_set_adaptive.restype = i32
+        L.pinn_lbfgs_state_bytes.argtypes = [i32]
+        L.pinn_lbfgs_state_bytes.restype = ctypes.c_size_t
+        L.pinn_lbfgs_begin.argtypes = [vp, vp, ctypes.POINTER(LBFGSConfig), vp, vp, vp]
+        L.pinn_lbfgs_begin.restype = i32
+        L.pinn_lbfgs_advance.argtypes = [vp, vp, vp, vp, vp, vp, vp]
+        L.pinn_lbfgs_advance.restype = i32
+        L.pinn_trainer_run_lbfgs.argtypes = [vp, ctypes.POINTER(LBFGSConfig), i32, i32]
+        L.pinn_trainer_run_lbfgs.restype = i32
+        L.pinn_trainer_read_lbfgs.argtypes = [vp, vp, vp, i64]
+        L.pinn_trainer_read_lbfgs.restype = i32
         L.pinn_host_timing.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
         L.pinn_host_timing.restype = i32
         L.pinn_dp_init.argtypes = [vp, i32, i32, vp]

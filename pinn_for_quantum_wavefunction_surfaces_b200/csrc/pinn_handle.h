@@ -114,6 +114,8 @@ struct LossCall {
   Chunk chunk[4] = {};
 };
 int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st);
+// pinn_lbfgs.cu: torch's defaults for an unset max_eval, then the checks every L-BFGS entry makes (PINN_EINVAL + message)
+int lbfgs_resolve_config(pinn_handle* h, const pinn_lbfgs_config* in, pinn_lbfgs_config* out);
 
 // VariantCoef and number of MLP evaluations (1 or 2) of a PINN_VARIANT_*; PINN_EINVAL for an unknown variant
 inline int variant_coef(int variant, VariantCoef* vc, int* nev) {

@@ -3,6 +3,7 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "../../include/pinn_b200.h"
 #include "pinn_dp.cuh"
 #include "pinn_launch.h"
 #include <cmath>
@@ -114,6 +115,17 @@ __device__ inline void adam_bookkeeping(const AdamParams& a, unsigned long long 
   if (take_best) { *a.best_loss = Ltot; *a.best_step = (long long)t; }
   *a.step = t + 1ull;
 }
+
+// L-BFGS machine (pinn_lbfgs.cu).  slots: evaluations one call may take.  cond: the WHILE node to clear when the call
+// ends (trainer graphs), or NULL.
+size_t lbfgs_state_bytes(int history_size);
+int lbfgs_slots(const pinn_lbfgs_config& c);
+cudaError_t launch_lbfgs_begin(unsigned char* state, const pinn_lbfgs_config& c, const double* theta, float* theta32,
+                               cudaStream_t st);
+cudaError_t launch_lbfgs_advance(unsigned char* state, const double* sums, const double* grad, double* theta, float* theta32,
+                                 double* trace, long long trace_rows, const cudaGraphConditionalHandle* cond, cudaStream_t st);
+// sets cond to "the call in `state` has not finished" (the node in front of the trainer's WHILE node)
+cudaError_t launch_lbfgs_cond(const unsigned char* state, cudaGraphConditionalHandle cond, cudaStream_t st);
 
 cudaError_t measure_fp32_peak(int sm_count, cudaStream_t st, double* fma_per_s, double* ms_best, double* sm_mhz);
 cudaError_t launch_enet_curve(const float* theta, const double* R, int n, double* E, double* dE, double* d2E, double* gate,

@@ -44,6 +44,13 @@ struct pinn_trainer {
   unsigned long long* pcounts = nullptr;  // {|set1|, |set2|, ticket} of the pool's draw, [3] scratch batch word of the selection
   cudaGraphExec_t graph_ad[2] = {nullptr, nullptr};  // [cur]: adaptive draw + step
   bool ad_warmed = false;  // one plain adaptive step has run (the inference kernel's attributes are set)
+  // L-BFGS (pinn_trainer_run_lbfgs): state of lb_hist pairs, trace [lb_trace_rows][4], the WHILE graph of one evaluation
+  unsigned char* lb_state = nullptr;
+  int lb_hist = 0;
+  double* lb_trace = nullptr;
+  int64_t lb_trace_rows = 0;
+  cudaGraphExec_t graph_lb[2] = {nullptr, nullptr};  // [cur]
+  bool lb_warmed = false;  // one plain L-BFGS evaluation has run
 };
 
 // Launches of one adaptive draw on top of the pool's sampler: the pool's residual and the four selection kernels
@@ -127,6 +134,73 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool adaptive_now, 
   int rc = loss_fwd_bwd_impl(h, lc, st);
   if (rc) return rc;
   return 0;
+}
+
+// One L-BFGS evaluation on buffer t->cur: the step kernel at theta32, the reduction (no Adam, no batch drawn), the L-BFGS
+// kernel.  cond: the WHILE node of a graph body, or NULL.
+static int lbfgs_eval_enqueue(pinn_trainer* t, const cudaGraphConditionalHandle* cond, cudaStream_t st) {
+  pinn_handle* h = t->h;
+  const pinn_train_config& c = t->cfg;
+  const int b = t->cur;
+  LossCall lc;
+  lc.variant = c.variant; lc.n = c.n; lc.x = t->x[b]; lc.y = t->y[b]; lc.z = t->z[b]; lc.R = t->R[b]; lc.in_dtype = PINN_F32;
+  lc.mask = t->mask[b]; lc.theta = t->theta32; lc.weights = t->weights[b]; lc.grad_mask = c.grad_mask; lc.bcutoff = c.bcutoff;
+  lc.sums = t->sums; lc.dtheta = t->grad; lc.E_out = t->E;
+  if (int rc = loss_fwd_bwd_impl(h, lc, st)) return rc;
+  CU(h, launch_lbfgs_advance(t->lb_state, t->sums, t->grad, t->theta, t->theta32, t->lb_trace, t->lb_trace_rows, cond, st));
+  h->launches += 1;
+  return 0;
+}
+
+// The graph of one .step() call: a kernel that sets the condition to "not finished", then a conditional WHILE node whose
+// body is one evaluation; the L-BFGS kernel clears the condition when the call finishes, so no evaluation runs past it.
+static int lbfgs_capture(pinn_trainer* t, cudaGraphExec_t* out) {
+  pinn_handle* h = t->h;
+  cudaGraph_t g = nullptr;
+  CU(h, cudaGraphCreate(&g, 0));
+  cudaGraphConditionalHandle cond;
+  cudaGraphNodeParams np = {};
+  cudaGraphNode_t first = nullptr, node = nullptr;
+  size_t nfirst = 1;
+  cudaGraph_t body = nullptr;
+  int rc = 0;
+  cudaError_t e = cudaGraphConditionalHandleCreate(&cond, g, 0, 0);
+  if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(t->st, g, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal);
+  if (e == cudaSuccess) {
+    e = launch_lbfgs_cond(t->lb_state, cond, t->st);
+    cudaGraph_t same = nullptr;
+    const cudaError_t e2 = cudaStreamEndCapture(t->st, &same);
+    if (e == cudaSuccess) e = e2;
+  }
+  if (e == cudaSuccess) e = cudaGraphGetNodes(g, &first, &nfirst);
+  if (e == cudaSuccess) {
+    np.type = cudaGraphNodeTypeConditional;
+    np.conditional.handle = cond;
+    np.conditional.type = cudaGraphCondTypeWhile;
+    np.conditional.size = 1;
+    e = cudaGraphAddNode(&node, g, &first, 1, &np);
+  }
+  if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(t->st, np.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                                         cudaStreamCaptureModeThreadLocal);
+  if (e != cudaSuccess) { cudaGraphDestroy(g); return fail(h, (int)e, "pinn_trainer_run_lbfgs: conditional graph"); }
+  const int64_t launches_before = h->launches;
+  rc = lbfgs_eval_enqueue(t, &cond, t->st);
+  h->launches = launches_before;
+  e = cudaStreamEndCapture(t->st, &body);
+  if (rc) { cudaGraphDestroy(g); return rc; }
+  if (e != cudaSuccess) { cudaGraphDestroy(g); return fail(h, (int)e, "pinn_trainer_run_lbfgs: cudaStreamEndCapture"); }
+  e = cudaGraphInstantiate(out, g, 0);
+  cudaGraphDestroy(g);
+  if (e != cudaSuccess) return fail(h, (int)e, "pinn_trainer_run_lbfgs: cudaGraphInstantiate");
+  return 0;
+}
+
+static void trainer_free_lbfgs(pinn_trainer* t) {
+  for (cudaGraphExec_t& g : t->graph_lb)
+    if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+  cudaFree(t->lb_state); cudaFree(t->lb_trace);
+  t->lb_state = nullptr; t->lb_trace = nullptr;
+  t->lb_hist = 0; t->lb_trace_rows = 0;
 }
 
 static int trainer_capture(pinn_trainer* t, bool adaptive_now, bool presample_next, cudaGraphExec_t* out) {
@@ -409,6 +483,7 @@ int pinn_trainer_destroy(pinn_trainer* t) {
     for (int b = 0; b < 2; b++)
       if (t->graph[a][b]) cudaGraphExecDestroy(t->graph[a][b]);
   trainer_free_adaptive(t);
+  trainer_free_lbfgs(t);
   for (int b = 0; b < 2; b++) {
     cudaFree(t->x[b]); cudaFree(t->y[b]); cudaFree(t->z[b]); cudaFree(t->R[b]); cudaFree(t->mask[b]);
     cudaFree(t->weights[b]); cudaFree(t->counts[b]);
@@ -458,6 +533,9 @@ int pinn_trainer_load_state(pinn_trainer* t, const double* theta, const double* 
       if (t->graph[a][b]) { cudaGraphExecDestroy(t->graph[a][b]); t->graph[a][b] = nullptr; }
   for (cudaGraphExec_t& g : t->graph_ad)
     if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+  // the L-BFGS state restarts fresh (torch's empty state), like a new optimizer on the loaded parameters
+  // on the trainer's stream (created non-blocking), so the next call's kernels are ordered after it
+  if (t->lb_state) CU(h, cudaMemsetAsync(t->lb_state, 0, lbfgs_state_bytes(t->lb_hist), t->st));
   return 0;
 }
 
@@ -562,6 +640,87 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
     if (presample_next) t->next_ready = true;
     if (rs) t->have_batch = true;
     t->steps_issued++;
+  }
+  return 0;
+}
+
+int pinn_trainer_run_lbfgs(pinn_trainer* t, const pinn_lbfgs_config* cfg, int resample, int use_graph) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  pinn_lbfgs_config c;
+  {
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (int rc = lbfgs_resolve_config(h, cfg, &c)) return rc;
+  }
+  if (!resample && !t->have_batch)
+    return fail(h, PINN_EINVAL, "pinn_trainer_run_lbfgs: no batch yet (resample = 0 needs pinn_trainer_set_batch or an earlier sampled step)");
+  if (dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_run_lbfgs: L-BFGS is not available with the data-parallel exchange");
+  if (resample && t->pool_factor > 0)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_run_lbfgs: L-BFGS does not draw adaptive batches");
+  DevGuard dev_guard(h->device);
+  const int64_t slots = lbfgs_slots(c);
+  if (!t->lb_state || t->lb_hist != c.history_size || t->lb_trace_rows < slots) {
+    // (re)allocation happens here, outside any capture; a new history size is a fresh optimizer
+    CU(h, cudaStreamSynchronize(t->st));
+    for (cudaGraphExec_t& g : t->graph_lb)
+      if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+    if (!t->lb_state || t->lb_hist != c.history_size) {
+      cudaFree(t->lb_state);
+      t->lb_state = nullptr; t->lb_hist = 0;
+      const size_t bytes = lbfgs_state_bytes(c.history_size);
+      CU(h, cudaMalloc(&t->lb_state, bytes));
+      CU(h, cudaMemsetAsync(t->lb_state, 0, bytes, t->st));  // ordered before the begin kernel on the same stream
+      t->lb_hist = c.history_size;
+    }
+    if (t->lb_trace_rows < slots) {
+      cudaFree(t->lb_trace);
+      t->lb_trace = nullptr; t->lb_trace_rows = 0;
+      CU(h, cudaMalloc(&t->lb_trace, (size_t)slots * 4 * 8));
+      t->lb_trace_rows = slots;
+    }
+  }
+  if (resample) {
+    const SampleParams s = sampler_params(t, t->cur);
+    CU(h, launch_sample(s, false, t->st));
+    h->launches += 1;
+    t->have_batch = true;
+  }
+  CU(h, cudaMemsetAsync(t->lb_trace, 0, (size_t)t->lb_trace_rows * 4 * 8, t->st));
+  CU(h, launch_lbfgs_begin(t->lb_state, c, t->theta, t->theta32, t->st));
+  h->launches += 1;
+  int64_t k = 0;
+  if (!t->lb_warmed) {  // one-time kernel attributes are set outside any capture
+    if (int rc = lbfgs_eval_enqueue(t, nullptr, t->st)) return rc;
+    t->lb_warmed = true;
+    k = 1;
+  }
+  if (use_graph) {
+    cudaGraphExec_t& g = t->graph_lb[t->cur];
+    if (!g) {
+      if (int rc = lbfgs_capture(t, &g)) return rc;
+    }
+    CU(h, cudaGraphLaunch(g, t->st));
+    h->launches += 4;  // the condition kernel and one evaluation: how many evaluations run is decided on the device
+  } else {
+    for (; k < slots; k++)
+      if (int rc = lbfgs_eval_enqueue(t, nullptr, t->st)) return rc;
+  }
+  return 0;
+}
+
+int pinn_trainer_read_lbfgs(pinn_trainer* t, double* status, double* trace, int64_t rows) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  DevGuard dev_guard(h->device);
+  CU(h, cudaStreamSynchronize(t->st));
+  if (status) {
+    if (t->lb_state) CU(h, cudaMemcpy(status, t->lb_state, 8 * 8, cudaMemcpyDeviceToHost));
+    else std::memset(status, 0, 8 * 8);
+  }
+  if (trace && rows > 0 && t->lb_trace) {
+    const int64_t r = rows < t->lb_trace_rows ? rows : t->lb_trace_rows;
+    CU(h, cudaMemcpy(trace, t->lb_trace, (size_t)r * 4 * 8, cudaMemcpyDeviceToHost));
   }
   return 0;
 }

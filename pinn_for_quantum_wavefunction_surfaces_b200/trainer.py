@@ -7,6 +7,7 @@ which parity runs need); this module is the fast path for runs that do not need 
     sample(...)              <->  train.py:26-39; sampling()+radial()+torch.where  poc/main.py:124-156, 390-393
     sample_adaptive(...)        residual-adaptive batches (RAD) drawn from a pool of sample() points
     adam_step(...)           <->  optimizer.step() + best/history bookkeeping      train.py:58-72; poc/main.py:403-417
+    lbfgs_begin/lbfgs_advance   torch.optim.LBFGS.step(closure), one closure evaluation per device launch
     Trainer                  <->  train()                                          train.py:21-72; poc/main.py:359-430
     train_trainpy / train_poc   convenience drivers with the reference's defaults and return values
 """
@@ -16,7 +17,7 @@ import numpy as np
 import torch
 
 from . import params as P
-from ._lib import Handle, PinnError, TrainConfig
+from ._lib import Handle, LBFGSConfig, PinnError, TrainConfig
 
 INT64_MAX = (1 << 63) - 1
 BOX_POC = (-18.0, 18.0, -18.0, 18.0, -18.0, 18.0, 0.2, 4.0)      # set_params() poc/main.py:17-27
@@ -117,6 +118,69 @@ def adam_step(state, grad, sums, n, lr=8e-3, betas=(0.9, 0.999), eps=1e-8, grad_
     h.check(rc, "pinn_adam_step")
 
 
+LBFGS_REASONS = {0: "running", 1: "optimal at start", 2: "directional derivative", 3: "max_iter", 4: "max_eval",
+                 5: "tolerance_grad", 6: "step change", 7: "loss change", 8: "slots exhausted"}
+
+
+def lbfgs_config(max_iter=20, max_eval=None, lr=1, tolerance_grad=1e-7, tolerance_change=1e-9, history_size=100,
+                 line_search_fn=None):
+    """pinn_lbfgs_config from torch.optim.LBFGS's arguments and defaults."""
+    if line_search_fn not in (None, "strong_wolfe"):
+        raise ValueError("only 'strong_wolfe' is supported")
+    c = LBFGSConfig()
+    c.lr, c.max_iter, c.history_size = float(lr), int(max_iter), int(history_size)
+    c.max_eval = 0 if max_eval is None else int(max_eval)
+    c.line_search = 1 if line_search_fn == "strong_wolfe" else 0
+    c.tolerance_grad, c.tolerance_change = float(tolerance_grad), float(tolerance_change)
+    return c
+
+
+def lbfgs_status(status):
+    """The 8-double status header of an L-BFGS state -> dict."""
+    s = [float(x) for x in status]
+    return {"n_iter": int(s[0]), "func_evals": int(s[1]), "evals": int(s[2]), "done": bool(s[3]), "reason": int(s[4]),
+            "reason_name": LBFGS_REASONS.get(int(s[4]), "?"), "loss": s[5], "iters": int(s[6]), "t": s[7]}
+
+
+class LBFGSState:
+    """Device state of the L-BFGS machine (pinn_lbfgs_*): zero bytes = a fresh torch.optim.LBFGS.  theta (float64) and
+    theta32 hold the point the machine asks to be evaluated next, and its final iterate once it is done."""
+
+    def __init__(self, theta0, history_size=100, device=None):
+        h = _handle(device)
+        self.h = h
+        dev = torch.device("cuda", h.device)
+        self.history_size = int(history_size)
+        nbytes = int(h.L.pinn_lbfgs_state_bytes(self.history_size))
+        if nbytes == 0:
+            raise ValueError("history_size must be >= 1")
+        self.state = torch.zeros(nbytes // 8, dtype=torch.float64, device=dev)
+        self.theta = torch.as_tensor(np.asarray(theta0, np.float64)).to(dev).clone()
+        self.theta32 = self.theta.float()
+
+    def status(self):
+        """Synchronises; -> dict of the status header."""
+        return lbfgs_status(self.state[:8].cpu().numpy())
+
+
+def lbfgs_begin(state, max_iter=20, max_eval=None, lr=1, tolerance_grad=1e-7, tolerance_change=1e-9, line_search_fn=None):
+    """Start one .step() call on `state` (LBFGSState): requests an evaluation at state.theta."""
+    c = lbfgs_config(max_iter, max_eval, lr, tolerance_grad, tolerance_change, state.history_size, line_search_fn)
+    h = state.h
+    stream = torch.cuda.current_stream(state.theta.device).cuda_stream
+    h.check(h.L.pinn_lbfgs_begin(h.h, _ptr(state.state), ctypes.byref(c), _ptr(state.theta), _ptr(state.theta32),
+                                 ctypes.c_void_p(stream)), "pinn_lbfgs_begin")
+
+
+def lbfgs_advance(state, sums, grad):
+    """Consume the evaluation at the requested point (sums[0] = loss, grad: 1521 float64 CUDA tensors) and request the
+    next one, or finish."""
+    h = state.h
+    stream = torch.cuda.current_stream(state.theta.device).cuda_stream
+    h.check(h.L.pinn_lbfgs_advance(h.h, _ptr(state.state), _ptr(sums), _ptr(grad), _ptr(state.theta), _ptr(state.theta32),
+                                   ctypes.c_void_p(stream)), "pinn_lbfgs_advance")
+
+
 class Trainer:
     """pinn_trainer: everything of a training run lives on the device until read()."""
 
@@ -179,6 +243,28 @@ class Trainer:
         instead, which costs the host less (1.5 vs 7 microseconds per step) but breaks the dependent-launch chain between
         replays (measured 147.6 vs 145.5 microseconds per step at 2^18 points)."""
         self.h.check(self.h.L.pinn_trainer_run(self.t, steps, int(resample), int(use_graph)), "pinn_trainer_run")
+
+    def run_lbfgs(self, max_iter=20, max_eval=None, lr=1, tolerance_grad=1e-7, tolerance_change=1e-9, history_size=100,
+                  line_search_fn=None, resample=False, use_graph=False):
+        """One torch.optim.LBFGS.step(closure) on the device (pinn_trainer_run_lbfgs), with torch's argument names and
+        defaults; the closure is Ltot and its gradient (restricted to grad_mask) on the trainer's current batch, which
+        stays fixed (resample=True draws a new one first).  The optimizer state persists across calls.  Adam's moments,
+        step counter, history and best-model record are left alone.  Synchronises; -> (status dict, trace (evals, 4):
+        Ltot, Lpde, Lbc and step length per evaluation)."""
+        c = lbfgs_config(max_iter, max_eval, lr, tolerance_grad, tolerance_change, history_size, line_search_fn)
+        self.h.check(self.h.L.pinn_trainer_run_lbfgs(self.t, ctypes.byref(c), int(resample), int(use_graph)),
+                     "pinn_trainer_run_lbfgs")
+        return self.read_lbfgs()
+
+    def read_lbfgs(self):
+        """-> (status dict, trace of the last L-BFGS call)."""
+        st = np.zeros(8, np.float64)
+        p = lambda a: a.ctypes.data_as(ctypes.c_void_p)
+        self.h.check(self.h.L.pinn_trainer_read_lbfgs(self.t, p(st), None, 0), "pinn_trainer_read_lbfgs")
+        s = lbfgs_status(st)
+        tr = np.zeros((max(s["evals"], 1), 4), np.float64)
+        self.h.check(self.h.L.pinn_trainer_read_lbfgs(self.t, None, p(tr), s["evals"]), "pinn_trainer_read_lbfgs")
+        return s, tr[:s["evals"]]
 
     def read(self, history_rows=None):
         f = lambda: np.empty(P.N_THETA, np.float64)
