@@ -152,6 +152,26 @@ int pinn_fields(pinn_handle* h, int variant, int64_t n,
                 float* psi, float* lap, float* hpsi, float* res, float* E, void* stream);
 
 /*
+ * The loss without its gradient: the 8 sums of pinn_loss_fwd_bwd at theta over n points, from a forward-only instance of
+ * the step kernel that stores nothing per point.
+ *  - res, psi and E of every point are the float32 bits pinn_fields writes for it; the set bits come from the mask byte
+ *    (bit 0: set 1, bit 1: set 2) or, with mask NULL, from the training rule r >= bcutoff (ir * bcutoff <= 1).
+ *  - Every sum is accumulated in DOUBLE: per lane over the CTA's super-tiles, then a fixed shuffle tree, a fixed group
+ *    order and the CTA rows in index order.  Repeat calls give the same bits, and the sums do not drift with n the way
+ *    the float32 accumulators of the training kernel do.
+ *  - weights: device, 3 double {w_pde, w_bc1, w_bc2}, or NULL for {1/n, 1/|set1|, 1/|set2|} of the counted sets (no
+ *    separate counting launch).  An empty set gives a NaN Lbc, as in the training path.
+ *  - sums (device, 8 double) = {Ltot, Lpde, Lbc, sum E, sum res^2, sum psi^2 over set 1, sum psi^2 over set 2, E of the
+ *    last point}; sums[3] is the float64 sum of the float32 E.
+ * Two launches (the step kernel, one finishing block); the per-CTA rows live in the stream's workspace, so the call can
+ * be captured in a CUDA graph once it has run on the stream outside a capture.  PINN_EINVAL, with nothing launched, for
+ * n <= 0, a NULL pointer other than mask and weights, a bad in_dtype or an unknown variant.
+ */
+int pinn_loss_eval(pinn_handle* h, int variant, int64_t n, const void* x, const void* y, const void* z, const void* R,
+                   int in_dtype, const uint8_t* mask, const float* theta, const double* weights, float bcutoff,
+                   double* sums, void* stream);
+
+/*
  * pinn_loss_fwd_bwd for a caller that holds the model as its 16 PARAMETER TENSORS (an nn.Module / train.py's tuple) -
  * the call behind the torch.autograd.Function that replaces NN_ion.LossFunctions (poc/main.py:341-355) and the inline
  * block train.py:41-57.  Nothing is packed or converted in front of the launch:
@@ -335,11 +355,33 @@ int pinn_trainer_batch(pinn_trainer* t, float** x, float** y, float** z, float**
  * batch index (one index per draw).  The draw is enqueued in front of that step's step kernel: 6 launches more per
  * resampling step (8 in all), and no batch is drawn inside the reduction kernel while adaptive sampling is on.
  * use_graph = 1 replays the whole adaptive step as one graph of its own (same bits as plain launches).  The history and
- * the best-model record are evaluated on the adaptive batches, so Ltot is not comparable with a uniform run's.
+ * the best-model record are evaluated on the adaptive batches, so Ltot is not comparable with a uniform run's (the
+ * held-out loss of pinn_trainer_set_validation is).
  * pool_factor = 0 (the default) turns it off and frees the pool; the buffers of pool_factor * n points are allocated
  * here, never in pinn_trainer_run.  PINN_EINVAL for pool_factor < 0, or k or c negative or not finite; PINN_ENOTSUP while
  * the data-parallel exchange is on (pinn_trainer_run also refuses an adaptive trainer then). */
 int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c);
+/* Held-out validation loss during training.  This call draws the held-out set once, by the trainer's sampler with its box,
+ * cutoff and bcutoff: it is pinn_sample(n_val, seed, 0, ...) bit for bit.  (Take a seed other than the training seed:
+ * batch 0 of the training seed is the first training batch.)  From then on, every optimizer step of pinn_trainer_run that
+ * brings the steps done since the run (re)started to a multiple of `every` is followed by one pinn_loss_eval of the set
+ * at the float32 parameters that step left (weights: the counted sets, mask: the set's), two launches.  It writes row k
+ * = {optimizer steps done, Ltot, Lpde, Lbc} of a device history of `capacity` rows (evaluations past it are counted, not
+ * stored) and updates a best-on-validation record {best_val_loss, best_val_theta (float64), best_val_step}, which starts
+ * at +inf / the trainer's current theta / -1 and takes an evaluation only when its Ltot is strictly lower (a NaN is never
+ * taken).  Adam's history and best-model record, the batch sequence and every trainer state are unchanged by it; the
+ * evaluation reads no batch buffer.  With use_graph = 1 the evaluations are plain launches between the step graphs (the
+ * same bits).  The set, its rows and the record are allocated here, never in pinn_trainer_run; every = 0 turns
+ * validation off and frees them.  pinn_trainer_load_state restarts the rows and the record.  PINN_EINVAL for every < 0,
+ * or n_val <= 0 or capacity < 0 with every > 0; PINN_ENOTSUP while the data-parallel exchange is on (pinn_trainer_run
+ * also refuses a trainer with validation on then). */
+int pinn_trainer_set_validation(pinn_trainer* t, int64_t n_val, uint64_t seed, int64_t every, int64_t capacity);
+/* One validation evaluation now, at the current theta32 (a step-0 point, or after pinn_trainer_run_lbfgs): a row and the
+ * record as above.  PINN_EINVAL when validation is off. */
+int pinn_trainer_validate(pinn_trainer* t);
+/* Synchronise and read: up to max_rows rows of 4 doubles, best_val_theta (1521 doubles), scalars = {evaluations
+ * recorded, best_val_loss, best_val_step}.  Any pointer may be NULL.  PINN_EINVAL when validation is off. */
+int pinn_trainer_read_validation(pinn_trainer* t, double* rows, int64_t max_rows, double* best_val_theta, double* scalars);
 void* pinn_trainer_stream(pinn_trainer* t);
 
 /*

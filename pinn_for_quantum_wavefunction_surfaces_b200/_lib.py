@@ -14,7 +14,8 @@ EXPORTS = [
     "pinn_sample", "pinn_sample_adaptive", "pinn_adam_step", "pinn_enet_curve", "pinn_grid_reduce", "pinn_spheroidal_reduce", "pinn_trainer_create", "pinn_trainer_destroy",
     "pinn_trainer_load_state", "pinn_trainer_set_batch", "pinn_trainer_run", "pinn_trainer_read", "pinn_trainer_batch",
     "pinn_trainer_stream", "pinn_trainer_set_adaptive", "pinn_lbfgs_state_bytes", "pinn_lbfgs_begin", "pinn_lbfgs_advance",
-    "pinn_trainer_run_lbfgs", "pinn_trainer_read_lbfgs",
+    "pinn_trainer_run_lbfgs", "pinn_trainer_read_lbfgs", "pinn_loss_eval", "pinn_trainer_set_validation",
+    "pinn_trainer_validate", "pinn_trainer_read_validation",
     "pinn_host_timing", "pinn_dp_init", "pinn_dp_connect", "pinn_dp_connect_local", "pinn_dp_enable", "pinn_dp_status", "pinn_dp_set_timeout", "pinn_dp_shutdown",
 ]
 
@@ -141,6 +142,14 @@ def lib():
         L.pinn_trainer_run_lbfgs.restype = i32
         L.pinn_trainer_read_lbfgs.argtypes = [vp, vp, vp, i64]
         L.pinn_trainer_read_lbfgs.restype = i32
+        L.pinn_loss_eval.argtypes = [vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, f32, vp, vp]
+        L.pinn_loss_eval.restype = i32
+        L.pinn_trainer_set_validation.argtypes = [vp, i64, u64, i64, i64]
+        L.pinn_trainer_set_validation.restype = i32
+        L.pinn_trainer_validate.argtypes = [vp]
+        L.pinn_trainer_validate.restype = i32
+        L.pinn_trainer_read_validation.argtypes = [vp, vp, i64, vp, vp]
+        L.pinn_trainer_read_validation.restype = i32
         L.pinn_host_timing.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
         L.pinn_host_timing.restype = i32
         L.pinn_dp_init.argtypes = [vp, i32, i32, vp]

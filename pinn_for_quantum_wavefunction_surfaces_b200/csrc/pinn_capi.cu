@@ -397,6 +397,31 @@ int pinn_fields(pinn_handle* h, int variant, int64_t n, const void* x, const voi
   return 0;
 }
 
+int pinn_loss_eval(pinn_handle* h, int variant, int64_t n, const void* x, const void* y, const void* z, const void* R,
+                   int in_dtype, const uint8_t* mask, const float* theta, const double* weights, float bcutoff, double* sums,
+                   void* stream) {
+  if (!h) return PINN_EINVAL;
+  std::lock_guard<std::mutex> lk(h->mu);
+  StepParams p{};
+  int nev = 0;
+  if (variant_coef(variant, &p.vc, &nev)) return fail(h, PINN_EINVAL, "pinn_loss_eval: unknown variant");
+  if (n <= 0) return fail(h, PINN_EINVAL, "pinn_loss_eval: n must be positive");
+  if (!x || !y || !z || !R || !theta || !sums) return fail(h, PINN_EINVAL, "pinn_loss_eval: NULL pointer argument");
+  if (in_dtype != PINN_F32 && in_dtype != PINN_F64) return fail(h, PINN_EINVAL, "pinn_loss_eval: bad in_dtype");
+  DevGuard dev_guard(h->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  pinn_workspace* ws = ws_for(h, st, h->sm_count);
+  if (!ws) return PINN_EINVAL;
+  p.x = x; p.y = y; p.z = z; p.R = R; p.mask = mask; p.n = n; p.in_f64 = in_dtype == PINN_F64; p.bcut = bcutoff;
+  p.theta = theta;
+  p.grid.partials = ws->grid_partials;  // the LOSS instance's per-CTA rows (p.grid.on stays 0)
+  const int grid = grid_for(h, n);
+  CU(h, launch_loss_tc(nev, p, grid, st));
+  CU(h, launch_loss_finish(ws->grid_partials, grid, n, weights, sums, nullptr, st));
+  h->launches += 2;
+  return 0;
+}
+
 int pinn_loss_fwd_bwd_host(pinn_handle* h, int variant, int64_t n, const void* x, const void* y, const void* z,
                            const void* R, int in_dtype, const uint8_t* mask, const double* theta_host,
                            const double* weights_host, uint32_t grad_mask, float bcutoff, double* sums_host,

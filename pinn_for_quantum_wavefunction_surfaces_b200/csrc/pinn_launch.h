@@ -83,6 +83,23 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 // the fused step kernel (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st);
 cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, cudaStream_t st);
+// The forward-only loss reduction (pinn_loss_eval): the LOSS instance of the step kernel over n points, one row of 8
+// doubles per CTA into p.grid.partials (p.grid.on = 0), then one finishing block -> the 8 sums of pinn_loss_fwd_bwd.
+// weights: device {w_pde, w_bc1, w_bc2} or NULL (the counted sets).  val: NULL, or the trainer's validation record.
+struct LossValidation {
+  int on;
+  const unsigned long long* step;  // device: optimizer steps done (column 0 of the row)
+  unsigned long long* count;       // device: evaluations recorded; row `count` is written when count < cap
+  double* rows;                    // [cap][4] {steps done, Ltot, Lpde, Lbc}
+  long long cap;
+  double* best_loss;               // +inf when the record starts
+  long long* best_step;
+  double* best_theta;              // float64 [NTHETA] <- theta of the evaluation taken
+  const double* theta;
+};
+cudaError_t launch_loss_tc(int nev, const StepParams& p, int grid, cudaStream_t st);
+cudaError_t launch_loss_finish(const double* partials, int nrows, long long n, const double* weights, double* sums,
+                               const LossValidation* val, cudaStream_t st);
 // sums the rows_per_R rows of every R in a fixed order -> out [nR][8]; a row with R <= 0 (or NaN) is all NaN
 cudaError_t launch_sph_finish(const double* partials, int nR, int rows_per_R, const double* Rs, double* out, cudaStream_t st);
 cudaError_t launch_count(const StepParams& p, unsigned long long* counts, double* weights, cudaStream_t st);

@@ -734,6 +734,10 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
 // ---------------------------------------------------------------------------------------------
 // the fused kernel.  NEV = MLP evaluations per point (2: poc, 1: train.py); TRAIN = with reverse sweep
 //   warp = role * 4 + group;  role < NEV: MLP evaluation, role == NEV: E-net + gate
+// LOSS (inference only, its own instance): the forward-only loss reduction of pinn_loss_eval.  The points are read as in
+// the fields mode; instead of per-point stores, role 0 adds res^2, psi^2 of either boundary set, E and the set sizes in
+// double over its super-tiles, and every CTA writes one row {sum res^2, sum psi^2 [set1], sum psi^2 [set2], sum E, |set1|,
+// |set2|, E(point n-1) (owner CTA only), -} to p.grid.partials (p.grid.on = 0: the member only carries the row pointer).
 // ---------------------------------------------------------------------------------------------
 // final fold of a packed vector sum: add the two row halves (lanes l and l + 16), lanes 0..15 store their two columns
 template <typename EntryOf>
@@ -763,7 +767,7 @@ struct TcParamsInline {
   alignas(16) float theta[NTHETA + 3];
 };
 
-template <int NEV, bool TRAIN, bool INLINE>
+template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false>
 __global__ void __launch_bounds__((NEV + 1) * 128, 1)
 pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, TcParamsInline, TcParamsPlain>::type q) {
   const StepParams& p = q.p;
@@ -918,6 +922,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
     acc.s0 = acc.s1 = acc.s2 = acc.s3 = acc.s4 = make_float2(0.0f, 0.0f);
 
     double gs0 = 0.0, gs1 = 0.0, gs2 = 0.0, gs3 = 0.0, gs4 = 0.0;  // dense-grid quadrature sums (role 0, inference only)
+    double ls[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};                 // loss sums (role 0, LOSS instance only)
 
     // every warp of the CTA walks the same super-tiles (the role barriers need all 4 groups); groups whose
     // 32 points lie beyond n compute on a clamped index with zero weight
@@ -971,6 +976,11 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
         const RawPt raw = p.grid.on ? (p.grid.sph ? tc_sph_point(p.grid, pi) : tc_grid_point(p, pi)) : coord_stage_read(p, cbuf, slot);
         g = geom_from_raw(raw);
         cur_dx1 = raw.dx1; cur_dx2 = raw.dx2;
+        if constexpr (LOSS) {
+          // the staged aligned word around mask[pi] (per-lane stage), read now: the stager refills this buffer one tile on
+          if (p.mask && role == 0)
+            mk_f = (float)((*(const uint32_t*)(cbuf + 4 * COORD_COL_BYTES + slot * 4) >> (8u * (unsigned)((uintptr_t)(p.mask + pi) & 3u))) & 3u);
+        }
       } else {
         float4* gp = geo + ((it & 1) * 128 + slot) * 3;
         if (!IS_MLP) {
@@ -1057,6 +1067,25 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       const float res = fmaf(gate, inner, fmaf(cE * E, psi, lcao));
 
       if (!TRAIN) {
+        if constexpr (LOSS) {
+          if (valid && role == 0) {
+            // the set bits by the training instances' rule: mask bytes when given, else ir * bcut <= 1
+            bool in1, in2;
+            if (p.mask) {
+              const unsigned mk = (unsigned)mk_f;
+              in1 = (mk & 1u) != 0; in2 = (mk & 2u) != 0;
+            } else {
+              in1 = g.ir1 * p.bcut <= 1.0f; in2 = g.ir2 * p.bcut <= 1.0f;
+            }
+            const double pd = (double)psi * (double)psi;
+            ls[0] += (double)res * (double)res;
+            if (in1) { ls[1] += pd; ls[4] += 1.0; }
+            if (in2) { ls[2] += pd; ls[5] += 1.0; }
+            ls[3] += (double)E;
+            if (pidx == p.n - 1) p.grid.partials[8 * (size_t)blockIdx.x + 6] = (double)E;
+          }
+          continue;
+        }
         if (p.grid.sph) {
           // one row per warp of role 0 and super-tile (its 32 points share one R): no state carried across tiles, so the
           // rows of one R are the same bits whatever else the launch sweeps.  Every slot is valid (padded to 128 per R).
@@ -1171,6 +1200,22 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(c.tbase) : "memory");
     }
     if (!TRAIN) {
+      if constexpr (LOSS) {  // one row of loss sums per CTA: lane order by a fixed shuffle tree, then groups in a fixed order
+        double* red = reinterpret_cast<double*>(stash);
+        if (role == 0) {
+  #pragma unroll
+          for (int k = 0; k < 6; k++)
+  #pragma unroll
+            for (int o = 16; o > 0; o >>= 1) ls[k] += __shfl_xor_sync(0xffffffffu, ls[k], o);
+          if (lane == 0) {
+  #pragma unroll
+            for (int k = 0; k < 6; k++) red[grp * 8 + k] = ls[k];
+          }
+        }
+        __syncthreads();
+        if (tid < 6) p.grid.partials[8 * (size_t)blockIdx.x + tid] = (red[tid] + red[8 + tid]) + (red[16 + tid] + red[24 + tid]);
+        return;
+      }
       if (p.grid.on && !p.grid.sph) {  // one row of quadrature sums per CTA, fixed order
         double* red = reinterpret_cast<double*>(stash);
         if (role == 0) {
@@ -1267,9 +1312,9 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
 // =================================================================================================
 // host-side launcher
 // =================================================================================================
-template <int NEV, bool TRAIN, bool INLINE>
+template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false>
 static cudaError_t launch_step_tc_t(const StepParams& p, int grid, cudaStream_t st) {
-  auto kern = pinn_step_tc_kernel<NEV, TRAIN, INLINE>;
+  auto kern = pinn_step_tc_kernel<NEV, TRAIN, INLINE, LOSS>;
   constexpr size_t smem = tc_smem_bytes<NEV>();
   static bool configured[16] = {false};
   int dev = 0;
@@ -1336,6 +1381,66 @@ cudaError_t launch_sph_finish(const double* partials, int nR, int rows_per_R, co
   const long long n = 8ll * nR;
   sph_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partials, nR, rows_per_R, Rs, out);
   return cudaGetLastError();
+}
+
+// Adds the per-CTA rows of the LOSS instance in row order, in double, and composes the 8 sums of pinn_loss_fwd_bwd with the
+// reduction kernel's expressions.  weights: device {w_pde, w_bc1, w_bc2}, or NULL for {1/n, 1/|set1|, 1/|set2|} from the
+// counted sets (an empty set: inf weight, NaN Lbc, as in the training path).  owner: the row that holds E(point n-1).
+// val (optional, the trainer's held-out validation): the row {steps done, Ltot, Lpde, Lbc} of this evaluation and the
+// best-on-validation record (strict <, so a NaN loss is never taken).
+__global__ void __launch_bounds__(256) loss_finish_kernel(const double* __restrict__ partials, int nrows, int owner, long long n,
+                                                          const double* __restrict__ weights, double* __restrict__ sums,
+                                                          const LossValidation val) {
+  __shared__ double tot[6];
+  __shared__ int take_s;
+  const int t = threadIdx.x;
+  if (t < 6) {
+    double s = 0.0;
+    for (int r = 0; r < nrows; r++) s += partials[8 * (size_t)r + t];
+    tot[t] = s;
+  }
+  __syncthreads();
+  if (t == 0) {
+    const double r2 = tot[0], p1 = tot[1], p2 = tot[2], sE = tot[3];
+    const double w0 = weights ? weights[0] : 1.0 / (double)n;
+    const double w1 = weights ? weights[1] : 1.0 / tot[4];
+    const double w2 = weights ? weights[2] : 1.0 / tot[5];
+    const double Lpde = w0 * r2, Lbc = w1 * p1 + w2 * p2;
+    const double Ltot = Lpde + Lbc;
+    sums[0] = Ltot; sums[1] = Lpde; sums[2] = Lbc; sums[3] = sE;
+    sums[4] = r2; sums[5] = p1; sums[6] = p2;
+    sums[7] = partials[8 * (size_t)owner + 6];
+    take_s = 0;
+    if (val.on) {
+      const unsigned long long k = *val.count;
+      const double steps = (double)*val.step;
+      if ((long long)k < val.cap) {
+        double* row = val.rows + 4 * k;
+        row[0] = steps; row[1] = Ltot; row[2] = Lpde; row[3] = Lbc;
+      }
+      *val.count = k + 1ull;
+      if (Ltot < *val.best_loss) {
+        *val.best_loss = Ltot;
+        *val.best_step = (long long)*val.step;
+        take_s = 1;
+      }
+    }
+  }
+  __syncthreads();
+  if (take_s)
+    for (int i = t; i < NTHETA; i += blockDim.x) val.best_theta[i] = val.theta[i];
+}
+cudaError_t launch_loss_finish(const double* partials, int nrows, long long n, const double* weights, double* sums,
+                               const LossValidation* val, cudaStream_t st) {
+  const int owner = (int)(((n - 1) >> 7) % nrows);  // super-tile st runs on CTA st % gridDim.x
+  LossValidation v{};
+  if (val) v = *val;
+  loss_finish_kernel<<<1, 256, 0, st>>>(partials, nrows, owner, n, weights, sums, v);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_loss_tc(int nev, const StepParams& p, int grid, cudaStream_t st) {
+  return nev == 2 ? launch_step_tc_t<2, false, false, true>(p, grid, st) : launch_step_tc_t<1, false, false, true>(p, grid, st);
 }
 
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st) {

@@ -51,6 +51,14 @@ struct pinn_trainer {
   int64_t lb_trace_rows = 0;
   cudaGraphExec_t graph_lb[2] = {nullptr, nullptr};  // [cur]
   bool lb_warmed = false;  // one plain L-BFGS evaluation has run
+  // held-out validation (pinn_trainer_set_validation): val_n fixed points, evaluated every val_every steps; off at 0
+  int64_t val_every = 0, val_n = 0, val_cap = 0;
+  float *vx = nullptr, *vy = nullptr, *vz = nullptr, *vR = nullptr;
+  uint8_t* vmask = nullptr;
+  unsigned long long* vwords = nullptr;  // {|set1|, |set2|, batch index, ticket} of the set's draw; [4] evaluations recorded
+  double *vweights = nullptr, *vpart = nullptr, *vsums = nullptr, *vrows = nullptr;
+  double *vbest_loss = nullptr, *vbest_theta = nullptr;
+  long long* vbest_step = nullptr;
 };
 
 // Launches of one adaptive draw on top of the pool's sampler: the pool's residual and the four selection kernels
@@ -201,6 +209,54 @@ static void trainer_free_lbfgs(pinn_trainer* t) {
   cudaFree(t->lb_state); cudaFree(t->lb_trace);
   t->lb_state = nullptr; t->lb_trace = nullptr;
   t->lb_hist = 0; t->lb_trace_rows = 0;
+}
+
+// One validation evaluation at theta32 on the held-out set: the LOSS instance of the step kernel and the finishing block,
+// which also writes the row and updates the best-on-validation record.  Reads no batch buffer.
+static int validation_enqueue(pinn_trainer* t) {
+  pinn_handle* h = t->h;
+  StepParams p{};
+  int nev = 0;
+  variant_coef(t->cfg.variant, &p.vc, &nev);
+  p.x = t->vx; p.y = t->vy; p.z = t->vz; p.R = t->vR; p.mask = t->vmask; p.n = t->val_n; p.bcut = t->cfg.bcutoff;
+  p.theta = t->theta32;
+  p.grid.partials = t->vpart;
+  const int grid = grid_for(h, t->val_n);
+  LossValidation v{};
+  v.on = 1; v.step = t->step; v.count = t->vwords + 4; v.rows = t->vrows; v.cap = t->val_cap;
+  v.best_loss = t->vbest_loss; v.best_step = t->vbest_step; v.best_theta = t->vbest_theta; v.theta = t->theta;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CU(h, launch_loss_tc(nev, p, grid, t->st));
+  CU(h, launch_loss_finish(t->vpart, grid, t->val_n, nullptr, t->vsums, &v, t->st));
+  h->launches += 2;
+  return 0;
+}
+
+// The validation rows and record start again (the stream is idle): no rows, best loss +inf, best step -1, best theta =
+// the trainer's current theta.
+static int validation_reset(pinn_trainer* t) {
+  pinn_handle* h = t->h;
+  const double inf = INFINITY;
+  const long long neg1 = -1;
+  CU(h, cudaMemset(t->vwords + 4, 0, 8));
+  CU(h, cudaMemset(t->vrows, 0, (size_t)t->val_cap * 4 * 8));
+  CU(h, cudaMemcpy(t->vbest_loss, &inf, 8, cudaMemcpyHostToDevice));
+  CU(h, cudaMemcpy(t->vbest_step, &neg1, 8, cudaMemcpyHostToDevice));
+  CU(h, cudaMemcpy(t->vbest_theta, t->theta, NTHETA * 8, cudaMemcpyDeviceToDevice));
+  return 0;
+}
+
+// Held-out set, rows and record (the stream is idle)
+static void trainer_free_validation(pinn_trainer* t) {
+  cudaFree(t->vx); cudaFree(t->vy); cudaFree(t->vz); cudaFree(t->vR); cudaFree(t->vmask); cudaFree(t->vwords);
+  cudaFree(t->vweights); cudaFree(t->vpart); cudaFree(t->vsums); cudaFree(t->vrows);
+  cudaFree(t->vbest_loss); cudaFree(t->vbest_theta); cudaFree(t->vbest_step);
+  t->vx = t->vy = t->vz = t->vR = nullptr;
+  t->vmask = nullptr;
+  t->vwords = nullptr;
+  t->vweights = t->vpart = t->vsums = t->vrows = t->vbest_loss = t->vbest_theta = nullptr;
+  t->vbest_step = nullptr;
+  t->val_every = t->val_n = t->val_cap = 0;
 }
 
 static int trainer_capture(pinn_trainer* t, bool adaptive_now, bool presample_next, cudaGraphExec_t* out) {
@@ -484,6 +540,7 @@ int pinn_trainer_destroy(pinn_trainer* t) {
       if (t->graph[a][b]) cudaGraphExecDestroy(t->graph[a][b]);
   trainer_free_adaptive(t);
   trainer_free_lbfgs(t);
+  trainer_free_validation(t);
   for (int b = 0; b < 2; b++) {
     cudaFree(t->x[b]); cudaFree(t->y[b]); cudaFree(t->z[b]); cudaFree(t->R[b]); cudaFree(t->mask[b]);
     cudaFree(t->weights[b]); cudaFree(t->counts[b]);
@@ -536,6 +593,96 @@ int pinn_trainer_load_state(pinn_trainer* t, const double* theta, const double* 
   // the L-BFGS state restarts fresh (torch's empty state), like a new optimizer on the loaded parameters
   // on the trainer's stream (created non-blocking), so the next call's kernels are ordered after it
   if (t->lb_state) CU(h, cudaMemsetAsync(t->lb_state, 0, lbfgs_state_bytes(t->lb_hist), t->st));
+  // the validation rows and record restart with the history (the memset above is on the non-blocking trainer stream)
+  if (t->val_every > 0) {
+    CU(h, cudaStreamSynchronize(t->st));
+    if (int rc = validation_reset(t)) return rc;
+  }
+  return 0;
+}
+
+int pinn_trainer_set_validation(pinn_trainer* t, int64_t n_val, uint64_t seed, int64_t every, int64_t capacity) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  if (every < 0 || (every > 0 && (n_val <= 0 || capacity < 0)))
+    return fail(h, PINN_EINVAL, "pinn_trainer_set_validation: need every >= 0, and n_val > 0 and capacity >= 0 when every > 0");
+  if (every > 0 && dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_set_validation: validation is not available with the data-parallel exchange");
+  DevGuard dev_guard(h->device);
+  CU(h, cudaStreamSynchronize(t->st));
+  trainer_free_validation(t);
+  if (every == 0) return 0;
+  const size_t n = (size_t)n_val;
+#define VAL_CU(call)                                                           \
+  do {                                                                         \
+    cudaError_t e__ = (call);                                                  \
+    if (e__ != cudaSuccess) {                                                  \
+      trainer_free_validation(t);                                              \
+      return fail(h, (int)e__, "pinn_trainer_set_validation: " #call);         \
+    }                                                                          \
+  } while (0)
+  VAL_CU(cudaMalloc(&t->vx, n * 4)); VAL_CU(cudaMalloc(&t->vy, n * 4)); VAL_CU(cudaMalloc(&t->vz, n * 4));
+  VAL_CU(cudaMalloc(&t->vR, n * 4)); VAL_CU(cudaMalloc(&t->vmask, n));
+  VAL_CU(cudaMalloc(&t->vwords, 5 * 8)); VAL_CU(cudaMemset(t->vwords, 0, 5 * 8));
+  VAL_CU(cudaMalloc(&t->vweights, 4 * 8));
+  VAL_CU(cudaMalloc(&t->vpart, (size_t)(h->sm_count + 1) * 8 * 8));
+  VAL_CU(cudaMalloc(&t->vsums, 8 * 8));
+  VAL_CU(cudaMalloc(&t->vrows, (size_t)std::max<int64_t>(capacity, 1) * 4 * 8));
+  VAL_CU(cudaMalloc(&t->vbest_loss, 8)); VAL_CU(cudaMalloc(&t->vbest_theta, NPART * 8)); VAL_CU(cudaMalloc(&t->vbest_step, 8));
+#undef VAL_CU
+  t->val_every = every; t->val_n = n_val; t->val_cap = capacity;
+  // the held-out set: pinn_sample(n_val, seed, 0, box, cutoff, bcutoff), drawn once, here
+  const pinn_train_config& c = t->cfg;
+  SampleParams s{};
+  s.n = n_val; s.seed = seed; s.batch_counter = t->vwords + 2;
+  s.xL = c.xL; s.xR = c.xR; s.yL = c.yL; s.yR = c.yR; s.zL = c.zL; s.zR = c.zR; s.RL = c.RL; s.RR = c.RR;
+  s.cutoff = c.cutoff; s.bcutoff = c.bcutoff;
+  s.x = t->vx; s.y = t->vy; s.z = t->vz; s.R = t->vR; s.mask = t->vmask; s.counts = t->vwords;
+  s.index_offset = 0;
+  s.weights = t->vweights; s.ticket = t->vwords + 3; s.reset_counts = 0;
+  int rc = 0;
+  cudaError_t e = launch_sample(s, true, t->st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(t->st);
+  if (e != cudaSuccess) rc = fail(h, (int)e, "pinn_trainer_set_validation: drawing the held-out set");
+  if (!rc) rc = validation_reset(t);
+  if (rc) { trainer_free_validation(t); return rc; }
+  {
+    std::lock_guard<std::mutex> lk(h->mu);
+    h->launches += 1;
+  }
+  return 0;
+}
+
+int pinn_trainer_validate(pinn_trainer* t) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  if (t->val_every <= 0) return fail(h, PINN_EINVAL, "pinn_trainer_validate: validation is off (pinn_trainer_set_validation)");
+  if (dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_validate: validation is not available with the data-parallel exchange");
+  DevGuard dev_guard(h->device);
+  return validation_enqueue(t);
+}
+
+int pinn_trainer_read_validation(pinn_trainer* t, double* rows, int64_t max_rows, double* best_val_theta, double* scalars) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  if (t->val_every <= 0) return fail(h, PINN_EINVAL, "pinn_trainer_read_validation: validation is off");
+  DevGuard dev_guard(h->device);
+  CU(h, cudaStreamSynchronize(t->st));
+  if (rows && max_rows > 0) {
+    const int64_t r = std::min(max_rows, t->val_cap);
+    if (r > 0) CU(h, cudaMemcpy(rows, t->vrows, (size_t)r * 4 * 8, cudaMemcpyDeviceToHost));
+  }
+  if (best_val_theta) CU(h, cudaMemcpy(best_val_theta, t->vbest_theta, NTHETA * 8, cudaMemcpyDeviceToHost));
+  if (scalars) {
+    unsigned long long k = 0;
+    long long bs = 0;
+    double bl = 0.0;
+    CU(h, cudaMemcpy(&k, t->vwords + 4, 8, cudaMemcpyDeviceToHost));
+    CU(h, cudaMemcpy(&bl, t->vbest_loss, 8, cudaMemcpyDeviceToHost));
+    CU(h, cudaMemcpy(&bs, t->vbest_step, 8, cudaMemcpyDeviceToHost));
+    scalars[0] = (double)k; scalars[1] = bl; scalars[2] = (double)bs;
+  }
   return 0;
 }
 
@@ -608,6 +755,8 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
   const bool adaptive = t->pool_factor > 0;
   if (adaptive && dp_active(h).world > 1)
     return fail(h, PINN_ENOTSUP, "pinn_trainer_run: adaptive sampling is not available with the data-parallel exchange");
+  if (t->val_every > 0 && dp_active(h).world > 1)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_run: validation is not available with the data-parallel exchange");
   auto resamples = [&](int64_t tt) { return resample && (tt % t->cfg.sc_sampling == 0) && (tt < t->cfg.freeze_after); };
   for (int64_t k = 0; k < steps; k++) {
     const int64_t tt = t->steps_issued;
@@ -640,6 +789,10 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
     if (presample_next) t->next_ready = true;
     if (rs) t->have_batch = true;
     t->steps_issued++;
+    // held-out validation after every step that brings the steps done since the run (re)started to a multiple of
+    // val_every, at the parameters this step left; plain launches between the steps' launches or graph replays
+    if (t->val_every > 0 && (t->steps_issued - t->step_base) % t->val_every == 0)
+      if (int rc = validation_enqueue(t)) return rc;
   }
   return 0;
 }

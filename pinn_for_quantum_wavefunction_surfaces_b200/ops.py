@@ -83,6 +83,39 @@ def loss_and_grad_raw(variant, x, y, z, R, theta, mask=None, weights=None, grad_
     return sums, dtheta, E_out
 
 
+def loss_eval(variant, x, y, z, R, theta, mask=None, weights=None, bcutoff=BC_CUTOFF, sums=None):
+    """The loss without its gradient (pinn_loss_eval) for DEVICE tensors: a forward-only kernel that accumulates in float64
+    and stores nothing per point.
+
+    x,y,z,R: CUDA float32/float64 (n,) ; theta: CUDA float32 (1521,) ; mask: CUDA uint8 (n,) or None (sets by r >= bcutoff);
+    weights: CUDA float64 (3,) {w_pde, w_bc1, w_bc2} or None ({1/n, 1/|set1|, 1/|set2|} of the counted sets).  Returns the
+    8 sums of loss_and_grad_raw as a float64 CUDA tensor {Ltot, Lpde, Lbc, sum E, sum res^2, sum psi^2 set 1, sum psi^2
+    set 2, E of the last point}, enqueued on torch's current stream."""
+    variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
+    if not x.is_cuda:
+        raise PinnError("loss_eval needs CUDA tensors (there is no CPU path)")
+    dev = x.device
+    h = Handle.get(dev.index if dev.index is not None else torch.cuda.current_device())
+    n = x.numel()
+    code = _F64 if x.dtype == torch.float64 else _F32
+    for t in (x, y, z, R):
+        if t.dtype != x.dtype or t.numel() != n or not t.is_contiguous() or t.device != dev:
+            raise ValueError("x,y,z,R must share dtype/length/device and be contiguous")
+    if theta.dtype != torch.float32 or theta.numel() != P.N_THETA or not theta.is_contiguous() or theta.device != dev:
+        raise ValueError("theta must be a contiguous float32 CUDA vector of 1521 elements on the points' device")
+    if mask is not None and (mask.dtype != torch.uint8 or mask.numel() != n or not mask.is_contiguous() or mask.device != dev):
+        raise ValueError("mask must be a contiguous uint8 CUDA tensor of n elements")
+    if weights is not None and (weights.dtype != torch.float64 or weights.numel() < 3 or weights.device != dev):
+        raise ValueError("weights must be a float64 CUDA tensor of 3 elements")
+    if sums is None:
+        sums = torch.empty(8, dtype=torch.float64, device=dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    rc = h.L.pinn_loss_eval(h.h, int(variant), n, _ptr(x), _ptr(y), _ptr(z), _ptr(R), code, _ptr(mask), _ptr(theta),
+                            _ptr(weights), float(bcutoff), _ptr(sums), ctypes.c_void_p(stream))
+    h.check(rc, "pinn_loss_eval")
+    return sums
+
+
 def _host_step(variant, x, y, z, R, theta64, mask, weights, grad_mask, want_E, bcutoff):
     """CPU tensors in, CPU float64 results out, through pinn_loss_fwd_bwd_host on cuda:current."""
     if not torch.cuda.is_available():

@@ -6,6 +6,7 @@ which parity runs need); this module is the fast path for runs that do not need 
 
     sample(...)              <->  train.py:26-39; sampling()+radial()+torch.where  poc/main.py:124-156, 390-393
     sample_adaptive(...)        residual-adaptive batches (RAD) drawn from a pool of sample() points
+    Trainer.set_validation      held-out validation loss during training (forward-only loss_eval, best-on-validation record)
     adam_step(...)           <->  optimizer.step() + best/history bookkeeping      train.py:58-72; poc/main.py:403-417
     lbfgs_begin/lbfgs_advance   torch.optim.LBFGS.step(closure), one closure evaluation per device launch
     Trainer                  <->  train()                                          train.py:21-72; poc/main.py:359-430
@@ -186,7 +187,7 @@ class Trainer:
 
     def __init__(self, variant, n, theta0, seed=12345, lr=8e-3, betas=(0.9, 0.999), eps=1e-8, box=None, cutoff=0.005,
                  bcutoff=17.5, grad_mask=0xFFFF, best_mode=None, best_after=0, sc_sampling=1, freeze_after=INT64_MAX,
-                 history_capacity=0, history_mean_E=None, device=None, handle=None, adaptive=None):
+                 history_capacity=0, history_mean_E=None, device=None, handle=None, adaptive=None, validation=None):
         variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
         self.h = handle if handle is not None else _handle(device)   # default: the cached per-device Handle
         if box is None:
@@ -210,14 +211,47 @@ class Trainer:
         self._step_base = 0
         if adaptive:
             self.set_adaptive(**adaptive)
+        self._val_cap = 0
+        if validation:
+            self.set_validation(**validation)
 
     def set_adaptive(self, pool_factor=4, k=1.0, c=1.0):
         """Residual-adaptive batches (pinn_trainer_set_adaptive): every resampling step draws its n points from
         pool_factor * n candidates in proportion to |res|^k / mean |res|^k + c at the current parameters; pool_factor=0
         turns it off.  The history and best-model record are then evaluated on the adaptive batches, so Ltot is not
-        comparable with a uniform run's."""
+        comparable with a uniform run's; set_validation records a held-out loss that is."""
         self.h.check(self.h.L.pinn_trainer_set_adaptive(self.t, int(pool_factor), float(k), float(c)),
                      "pinn_trainer_set_adaptive")
+
+    def set_validation(self, n, seed, every, capacity=None):
+        """Held-out validation loss (pinn_trainer_set_validation): n points drawn once now, sample(n, seed, 0) with the
+        trainer's box and cutoffs, evaluated (pinn_loss_eval, forward only) after every step that brings the steps done
+        since the run (re)started to a multiple of `every`, into `capacity` rows (None: 1024) and a best-on-validation
+        record.  The seed has no default: batch 0 of the training seed is the first training batch.  every=0 turns it
+        off.  Nothing else the trainer computes changes."""
+        if every and capacity is None:
+            capacity = 1024
+        capacity = int(capacity or 0)
+        self.h.check(self.h.L.pinn_trainer_set_validation(self.t, int(n), int(seed), int(every), capacity),
+                     "pinn_trainer_set_validation")
+        self._val_cap = capacity if every else 0
+
+    def validate(self):
+        """Enqueue one validation evaluation now, at the current parameters (a step-0 point, or after run_lbfgs)."""
+        self.h.check(self.h.L.pinn_trainer_validate(self.t), "pinn_trainer_validate")
+
+    def read_validation(self):
+        """-> dict(rows (k, 4): steps done, Ltot, Lpde, Lbc of each evaluation recorded; evaluations; best_val_theta;
+        best_val_loss; best_val_step (-1 while no evaluation was taken))."""
+        rows = np.zeros((max(self._val_cap, 1), 4), np.float64)
+        best = np.empty(P.N_THETA, np.float64)
+        sc = np.zeros(3, np.float64)
+        p = lambda a: a.ctypes.data_as(ctypes.c_void_p)
+        self.h.check(self.h.L.pinn_trainer_read_validation(self.t, p(rows), self._val_cap, p(best), p(sc)),
+                     "pinn_trainer_read_validation")
+        k = int(sc[0])
+        return {"rows": rows[:min(k, self._val_cap)], "evaluations": k, "best_val_theta": best,
+                "best_val_loss": float(sc[1]), "best_val_step": int(sc[2])}
 
     def load_state(self, theta, m=None, v=None, step=0):
         """Resume: parameters, Adam moments (None = zeros) and the number of optimizer steps already done.  The resumed run
@@ -326,15 +360,29 @@ def init_poc(seed=0):
     return P.pack_poc(ts, dtype=torch.float64).numpy()
 
 
+def _validation_rows(validation, steps):
+    """validation dict of train_poc / train_trainpy -> Trainer.set_validation arguments with room for every row of the run
+    (the step-0 evaluation and one per `every` steps)"""
+    v = dict(validation)
+    if v.get("capacity") is None:
+        v["capacity"] = steps // max(int(v["every"]), 1) + 1
+    return v
+
+
 def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_tune=False, use_graph=False, log_every=0,
-                  adaptive=None):
+                  adaptive=None, validation=None):
     """train(params, lr, epochs) of train.py on the device.  Like the reference it evaluates epochs+1 losses, takes `epochs`
     optimizer steps and returns the parameters of the best loss seen (train.py:58-69).  Returns (theta_best, info).
-    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive)."""
+    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive).
+    validation: None, or dict(n, seed, every, capacity=None) for a held-out loss (Trainer.set_validation), evaluated at the
+    initial parameters and every `every` steps; info then has a "validation" entry (Trainer.read_validation)."""
     if theta0 is None:
         theta0 = init_trainpy(seed)
     mask = P.FINE_TUNE_GRAD_MASK if fine_tune else 0xFFFF  # train.py:111 (commented) trains the E-net tensors only
-    tr = Trainer("trainpy", n, theta0, seed=seed, lr=lr, grad_mask=mask, history_capacity=epochs + 1, adaptive=adaptive)
+    tr = Trainer("trainpy", n, theta0, seed=seed, lr=lr, grad_mask=mask, history_capacity=epochs + 1, adaptive=adaptive,
+                 validation=_validation_rows(validation, epochs + 1) if validation else None)
+    if validation:
+        tr.validate()
     done = 0
     while done < epochs:
         k = min(log_every or epochs, epochs - done)
@@ -351,14 +399,18 @@ def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_t
     best = after["best_theta"]
     info = {"history": after["history"], "best_loss": after["best_loss"], "best_step": after["best_step"],
             "theta_last": before["theta"], "batches": after["batches"]}
+    if validation:
+        info["validation"] = tr.read_validation()
     tr.close()
     return best, info
 
 
-def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False, adaptive=None):
+def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False, adaptive=None, validation=None):
     """train(params, loadWeights, freezeUnits) of poc/main.py:359-430 on the device.  `params` uses the reference's keys
     (set_params(), poc/main.py:14-45).  Returns (theta_last, theta_saved or None, lossDictionary like poc/main.py:422-427).
-    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive)."""
+    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive).
+    validation: None, or dict(n, seed, every, capacity=None) for a held-out loss (Trainer.set_validation), evaluated at
+    theta0 and every `every` steps; the loss dictionary then has a "validation" entry (Trainer.read_validation)."""
     pr = {"xL": -18, "xR": 18, "yL": -18, "yR": 18, "zL": -18, "zR": 18, "RxL": 0.2, "RxR": 4, "cutOff": 0.005,
           "BCcutoff": 17.5, "sc_sampling": 1, "n_train": 100000, "epochs": 5000, "lr": 8e-3}
     pr.update(params or {})
@@ -371,11 +423,17 @@ def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False, a
     tr = Trainer("poc", int(pr["n_train"]), theta0, seed=seed, lr=pr["lr"], box=box, cutoff=pr["cutOff"],
                  bcutoff=pr["BCcutoff"], grad_mask=P.FINE_TUNE_GRAD_MASK if freezeUnits else 0xFFFF, best_mode=1,
                  best_after=best_after, sc_sampling=int(pr["sc_sampling"]), freeze_after=freeze_after,
-                 history_capacity=epochs, history_mean_E=False, adaptive=adaptive)
+                 history_capacity=epochs, history_mean_E=False, adaptive=adaptive,
+                 validation=_validation_rows(validation, epochs) if validation else None)
+    if validation:
+        tr.validate()
     tr.run(epochs, use_graph=use_graph)
     r = tr.read()
+    val = tr.read_validation() if validation else None
     tr.close()
     hcol = lambda k: r["history"][:, k:k + 1].copy()
     loss = {"Ltot": hcol(0), "Lpde": hcol(1), "Lbc": hcol(2), "Energy": hcol(3)}
+    if validation:
+        loss["validation"] = val
     saved = r["best_theta"] if r["best_step"] >= 0 else None
     return r["theta"], saved, loss
