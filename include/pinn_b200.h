@@ -141,6 +141,21 @@ int pinn_loss_fwd_bwd(pinn_handle* h, int variant, int64_t n,
                       double* sums, double* dtheta, float* E_out, void* stream);
 
 /*
+ * pinn_loss_fwd_bwd with a per-point loss weight: point_w (device, n float32, finite and >= 0) multiplies every per-point
+ * term of the sums and of their gradient,
+ *   Lpde = w_pde sum_p om_p res_p^2,   Lbc = w_bc1 sum_p om_p m1_p psi_p^2 + w_bc2 sum_p om_p m2_p psi_p^2,
+ *   sums[3] = sum_p om_p E_p,
+ * while the set sizes counted for weights = NULL stay counts of points.  om = 1 gives pinn_loss_fwd_bwd's bits.  Its use:
+ * an importance-weighted adaptive batch (pinn_sample_adaptive_importance), whose weighted sums estimate the pool's
+ * unweighted ones without bias.  Device-resident inputs only (the *_host entry has no weighted form).  PINN_EINVAL, with
+ * nothing launched, for a NULL point_w and everything pinn_loss_fwd_bwd refuses.
+ */
+int pinn_loss_fwd_bwd_weighted(pinn_handle* h, int variant, int64_t n, const void* x, const void* y, const void* z,
+                               const void* R, int in_dtype, const uint8_t* mask, const float* theta, const double* weights,
+                               const float* point_w, uint32_t grad_mask, float bcutoff, double* sums, double* dtheta,
+                               float* E_out, void* stream);
+
+/*
  * Inference: replaces the pair parametricPsi + hamiltonian (poc/main.py:321, 118;
  * call sites 451-454) and the residual of train.py:54.  Any output may be NULL.
  *  psi, lap (laplacian of psi), hpsi (-1/2 lap psi + V psi, Hartree form), res
@@ -301,6 +316,23 @@ int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_
                          void* stream);
 
 /*
+ * pinn_sample_adaptive with importance weights.  The batch (x, y, z, R, mask, idx, counts) is the same bits; in addition
+ *  - point_w (device, n float32): om_j = float32(T / (N w_i)) = 1 / (N P_i) of the candidate i that output j took, with
+ *    w_i formed again in float64 exactly as step 2 formed it (the same Q) and T = pool_cdf[N-1].  om <= (1 + c) / c; in
+ *    the uniform fallback om = 1.
+ *  - weights = {1/n, N / (n |set1 of the pool|), N / (n |set2 of the pool|)} (an empty set of the pool: inf, a NaN Lbc).
+ * Candidate i is taken c_i times with E_u0[c_i] = n P_i, so the expectation over u0 of pinn_loss_fwd_bwd_weighted on this
+ * batch with these weights - its loss and its gradient - is the pool's uniform loss {1/N, 1/|set1|, 1/|set2|}.
+ * Importance mode needs c > 0 (Lbc weights psi^2, not res^2, so a candidate of zero residual must keep a positive
+ * probability): PINN_EINVAL for c <= 0 or a NULL point_w, and everything pinn_sample_adaptive refuses; nothing launched.
+ */
+int pinn_sample_adaptive_importance(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed,
+                                    uint64_t batch, const float box[8], float cutoff, float bcutoff, float k, float c,
+                                    float* pool_x, float* pool_y, float* pool_z, float* pool_R, uint8_t* pool_mask,
+                                    float* pool_res, double* pool_cdf, float* x, float* y, float* z, float* R, uint8_t* mask,
+                                    int64_t* idx, uint64_t* counts, double* weights, float* point_w, void* stream);
+
+/*
  * One optimizer step of torch.optim.Adam (no weight decay, no amsgrad) over the 1521 float64 parameters, fused with
  * the reference loops' bookkeeping (train.py:58-72; poc/main.py:403-417).  All pointers are device memory.
  *  theta, m, v   in/out float64 [1521];  grad: dLtot/dtheta;  sums: the 8 sums of pinn_loss_fwd_bwd
@@ -361,6 +393,13 @@ int pinn_trainer_batch(pinn_trainer* t, float** x, float** y, float** z, float**
  * here, never in pinn_trainer_run.  PINN_EINVAL for pool_factor < 0, or k or c negative or not finite; PINN_ENOTSUP while
  * the data-parallel exchange is on (pinn_trainer_run also refuses an adaptive trainer then). */
 int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c);
+/* Importance weights for the adaptive batches of this trainer (on = 1; off = 0, the default): each adaptive draw is
+ * pinn_sample_adaptive_importance, and every step on such a batch - the drawing step and the steps up to the next draw -
+ * is pinn_loss_fwd_bwd_weighted with its omega and the pool-based loss weights.  The history and best-model record are
+ * then an unbiased estimate of the pool's uniform loss.  use_graph replays the same launches.  pinn_trainer_set_adaptive
+ * turns it off again.  PINN_EINVAL when adaptive sampling is off or its c is not > 0.  pinn_trainer_run_lbfgs refuses
+ * (PINN_ENOTSUP) to evaluate an importance batch. */
+int pinn_trainer_set_importance(pinn_trainer* t, int on);
 /* Held-out validation loss during training.  This call draws the held-out set once, by the trainer's sampler with its box,
  * cutoff and bcutoff: it is pinn_sample(n_val, seed, 0, ...) bit for bit.  (Take a seed other than the training seed:
  * batch 0 of the training seed is the first training batch.)  From then on, every optimizer step of pinn_trainer_run that

@@ -15,7 +15,8 @@ EXPORTS = [
     "pinn_trainer_load_state", "pinn_trainer_set_batch", "pinn_trainer_run", "pinn_trainer_read", "pinn_trainer_batch",
     "pinn_trainer_stream", "pinn_trainer_set_adaptive", "pinn_lbfgs_state_bytes", "pinn_lbfgs_begin", "pinn_lbfgs_advance",
     "pinn_trainer_run_lbfgs", "pinn_trainer_read_lbfgs", "pinn_loss_eval", "pinn_trainer_set_validation",
-    "pinn_trainer_validate", "pinn_trainer_read_validation",
+    "pinn_trainer_validate", "pinn_trainer_read_validation", "pinn_loss_fwd_bwd_weighted", "pinn_sample_adaptive_importance",
+    "pinn_trainer_set_importance",
     "pinn_host_timing", "pinn_dp_init", "pinn_dp_connect", "pinn_dp_connect_local", "pinn_dp_enable", "pinn_dp_status", "pinn_dp_set_timeout", "pinn_dp_shutdown",
 ]
 
@@ -85,6 +86,8 @@ def lib():
         L.pinn_profile_collect.restype = i32
         L.pinn_loss_fwd_bwd.argtypes = [vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, u32, f32, vp, vp, vp, vp]
         L.pinn_loss_fwd_bwd.restype = i32
+        L.pinn_loss_fwd_bwd_weighted.argtypes = [vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, vp, vp, u32, f32, vp, vp, vp, vp]
+        L.pinn_loss_fwd_bwd_weighted.restype = i32
         L.pinn_loss_fwd_bwd_tensors.argtypes = [vp, i32, i64, vp, vp, vp, vp, i32, vp, vp, i32, i32, vp, u32, f32, vp, vp, vp, i32, vp]
         L.pinn_loss_fwd_bwd_tensors.restype = i32
         L.pinn_mask_from_index_sets.argtypes = [vp, i64, vp, i64, vp, i64, vp, vp]
@@ -104,6 +107,8 @@ def lib():
         L.pinn_sample_adaptive.argtypes = [vp, i32, vp, i64, i64, u64, u64, ctypes.POINTER(f32), f32, f32, f32, f32,
                                            vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.pinn_sample_adaptive.restype = i32
+        L.pinn_sample_adaptive_importance.argtypes = L.pinn_sample_adaptive.argtypes[:-1] + [vp, vp]
+        L.pinn_sample_adaptive_importance.restype = i32
         L.pinn_adam_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, f64, f64, f64, f64, u32,
                                      i32, i64, i32, vp]
         L.pinn_adam_step.restype = i32
@@ -132,6 +137,8 @@ def lib():
         L.pinn_trainer_stream.restype = vp
         L.pinn_trainer_set_adaptive.argtypes = [vp, i32, f32, f32]
         L.pinn_trainer_set_adaptive.restype = i32
+        L.pinn_trainer_set_importance.argtypes = [vp, i32]
+        L.pinn_trainer_set_importance.restype = i32
         L.pinn_lbfgs_state_bytes.argtypes = [i32]
         L.pinn_lbfgs_state_bytes.restype = ctypes.c_size_t
         L.pinn_lbfgs_begin.argtypes = [vp, vp, ctypes.POINTER(LBFGSConfig), vp, vp, vp]

@@ -6,6 +6,7 @@
 //                      finishing last folds the block totals into the block offsets (sequentially) and draws u0
 //   rad_offset_kernel  cdf = block offset + in-block prefix
 //   rad_select_kernel  output j takes the first i with cdf[i] > (j + u0) / n * cdf[N-1]; gather, set sizes, loss weights
+//                      (importance mode: also omega_j = T / (N w_i), from w_i formed again exactly as the scan formed it)
 // Every sum has a fixed association order and there are no floating-point atomics, so cdf and the selection are the same
 // bits on every run.  Each partial prefix is a sequential fold, cdf[i+1] = fl(.. + w_i+1) with w >= 0 across every block
 // and thread boundary too, so cdf never decreases and a binary search finds the first index the rule names.
@@ -19,7 +20,7 @@ constexpr int RAD_THREADS = 256, RAD_PER_THREAD = 16, RAD_TILE = RAD_THREADS * R
 
 long long adaptive_scratch_doubles(long long pool) {
   const long long blocks = (pool + RAD_TILE - 1) / RAD_TILE;
-  return 3 * blocks + 2;  // block sums of q, block totals of w, block offsets + total, u0
+  return 3 * blocks + 3;  // block sums of q, block totals of w, block offsets + total, u0, Q
 }
 
 __device__ __forceinline__ double rad_q(float r, double k) {
@@ -130,6 +131,7 @@ __global__ void __launch_bounds__(RAD_THREADS) rad_scan_kernel(const AdaptivePar
     philox4x32_10((uint32_t)gi, (uint32_t)(gi >> 32), (uint32_t)batch, (uint32_t)(batch >> 32), (uint32_t)a.out.seed,
                   (uint32_t)(a.out.seed >> 32), r);
     boff[nb + 1] = (double)r[0] * 2.3283064365386963e-10;  // 2^-32
+    boff[nb + 2] = Q;  // the importance weights form w_i again from it
     *a.out.ticket = 0ull;
   }
 }
@@ -162,6 +164,12 @@ __global__ void __launch_bounds__(RAD_THREADS) rad_select_kernel(const AdaptiveP
     const uint8_t m = a.pmask[i];
     s.mask[j] = m;
     if (a.idx) a.idx[j] = i;
+    if (a.point_w) {
+      const double Q = a.part[3 * (long long)scan_blocks + 2];
+      const double Nd = (double)N;
+      const double w = (Q > 0.0 && isfinite(Q)) ? rad_q(a.res[i], a.k) * Nd / Q + a.c : 1.0;  // rad_scan_kernel's w_i
+      a.point_w[j] = (float)(total / (Nd * w));
+    }
     c1 += m & 1u; c2 += (m >> 1) & 1u;
   }
   c1 = __reduce_add_sync(0xffffffffu, c1);
@@ -179,7 +187,16 @@ __global__ void __launch_bounds__(RAD_THREADS) rad_select_kernel(const AdaptiveP
     last_block = atomicAdd(s.ticket, 1ull) == (unsigned long long)gridDim.x - 1;
   }
   __syncthreads();
-  if (last_block && threadIdx.x < 32) sample_finish(s);  // the loss weights exactly as the uniform sampler forms them
+  if (last_block && threadIdx.x < 32) {
+    sample_finish(s);  // the loss weights exactly as the uniform sampler forms them
+    if (a.point_w && threadIdx.x == 0) {
+      // importance batch: each weighted batch sum estimates the pool's sum times n / N, so the means take the pool's sizes
+      const double nd = (double)s.n, Nd = (double)N;
+      s.weights[1] = Nd / (nd * (double)a.pool_counts[0]);  // an empty set of the pool: inf, a NaN loss, as uniform
+      s.weights[2] = Nd / (nd * (double)a.pool_counts[1]);
+      a.pool_counts[0] = 0ull; a.pool_counts[1] = 0ull;
+    }
+  }
 }
 
 cudaError_t launch_adaptive_select(const AdaptiveParams& a, cudaStream_t st) {

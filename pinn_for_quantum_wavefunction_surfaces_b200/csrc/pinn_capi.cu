@@ -248,6 +248,7 @@ static int enqueue_step_chunk(pinn_handle* h, pinn_workspace* ws, int nev, StepP
   p.x = (const char*)p.x + first * es; p.y = (const char*)p.y + first * es;
   p.z = (const char*)p.z + first * es; p.R = (const char*)p.R + first * es;
   if (p.mask) p.mask += first;
+  if (p.point_w) p.point_w += first;
   if (p.E_out) p.E_out += first;
   p.n = cnt;
   p.partials = ws->partials + (size_t)row0 * NPART;
@@ -284,6 +285,8 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
   if (!c.x || !c.y || !c.z || !c.R || (!c.theta && !c.theta_inline && !c.theta_tensors) || !c.sums || !c.dtheta)
     return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: NULL pointer argument");
   if (c.in_dtype != PINN_F32 && c.in_dtype != PINN_F64) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd: bad in_dtype");
+  if (c.point_w && (c.theta_inline || c.nchunk))
+    return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd_weighted: per-point weights need device-resident inputs");
   const int nchunk = c.nchunk ? c.nchunk : 1;
   int need_rows = 0;  // one partial row per CTA of every chunk launch
   for (int k = 0; k < nchunk; k++) need_rows += train_grid_for(h, c.nchunk ? c.chunk[k].count : c.n);
@@ -292,6 +295,7 @@ int loss_fwd_bwd_impl(pinn_handle* h, const LossCall& c, cudaStream_t st) {
   if (!ws) return PINN_EINVAL;
   if (int rc = dp_serialize(h, st)) return rc;
   p.x = c.x; p.y = c.y; p.z = c.z; p.R = c.R; p.mask = c.mask; p.n = c.n; p.in_f64 = c.in_dtype == PINN_F64;
+  p.point_w = c.point_w;
   p.bcut = c.bcutoff; p.E_out = static_cast<float*>(c.E_out); p.E_f64 = c.E_f64;
   p.base_grads = (c.grad_mask & 0x003Fu) != 0;
   p.gate_grads = (c.grad_mask & 0xF000u) != 0;
@@ -340,6 +344,19 @@ int pinn_loss_fwd_bwd(pinn_handle* h, int variant, int64_t n, const void* x, con
   c.variant = variant; c.n = n; c.x = x; c.y = y; c.z = z; c.R = R; c.in_dtype = in_dtype; c.mask = mask;
   c.theta = theta; c.weights = weights; c.grad_mask = grad_mask; c.bcutoff = bcutoff; c.sums = sums; c.dtheta = dtheta;
   c.E_out = E_out;
+  return loss_fwd_bwd_impl(h, c, (cudaStream_t)stream);
+}
+
+int pinn_loss_fwd_bwd_weighted(pinn_handle* h, int variant, int64_t n, const void* x, const void* y, const void* z,
+                               const void* R, int in_dtype, const uint8_t* mask, const float* theta, const double* weights,
+                               const float* point_w, uint32_t grad_mask, float bcutoff, double* sums, double* dtheta,
+                               float* E_out, void* stream) {
+  if (!h) return PINN_EINVAL;
+  if (!theta || !point_w) return fail(h, PINN_EINVAL, "pinn_loss_fwd_bwd_weighted: NULL pointer argument");
+  LossCall c;
+  c.variant = variant; c.n = n; c.x = x; c.y = y; c.z = z; c.R = R; c.in_dtype = in_dtype; c.mask = mask;
+  c.theta = theta; c.weights = weights; c.point_w = point_w; c.grad_mask = grad_mask; c.bcutoff = bcutoff; c.sums = sums;
+  c.dtheta = dtheta; c.E_out = E_out;
   return loss_fwd_bwd_impl(h, c, (cudaStream_t)stream);
 }
 

@@ -85,6 +85,7 @@ struct LossCall {
   const void *x = nullptr, *y = nullptr, *z = nullptr, *R = nullptr;  // device (or mapped page-locked host) columns
   int in_dtype = PINN_F32;
   const uint8_t* mask = nullptr;
+  const float* point_w = nullptr;  // device float32 [n] per-point loss weights (pinn_loss_fwd_bwd_weighted), or NULL
   // theta: exactly one of - packed float32 device vector; HOST float32[1521] that travels inside the kernel parameters;
   // the caller's 16 tensors (device pointers in canonical order, float32/float64, (out,in) or train.py (in,out) layout)
   const float* theta = nullptr;

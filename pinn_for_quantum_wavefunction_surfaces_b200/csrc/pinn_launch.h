@@ -29,10 +29,11 @@ struct GridDesc {
 struct StepParams {
   const void *x, *y, *z, *R;
   const uint8_t* mask;
-  // 8 unused bytes.  Without them every member behind moves up by 8 bytes, and ptxas schedules the training kernel
-  // <2,true,false> differently (5866 instead of 5874 SASS instructions): measured 0.2 % slower, 0.11085 vs 0.11062 ms
-  // per 2^18-point step (tools/ab_time.py, 5 interleaved rounds, B200 at 1000 W).
-  const void* unused_slot;
+  // Per-point loss weights (device float32 [n], pinn_loss_fwd_bwd_weighted), read only by the WEIGHTED training instances.
+  // The member sits in what were 8 unused bytes: without them every member behind moves up by 8 bytes, and ptxas
+  // schedules the training kernel <2,true,false> differently (5866 instead of 5874 SASS instructions): measured 0.2 %
+  // slower, 0.11085 vs 0.11062 ms per 2^18-point step (tools/ab_time.py, 5 interleaved rounds, B200 at 1000 W).
+  const float* point_w;
   const float* theta;     // the raw parameter vector; every CTA builds its own operand images in shared memory
   const double* weights;  // {w_pde, w_bc1, w_bc2}
   double* partials;       // [gridDim.x][NPART]
@@ -80,7 +81,8 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #endif
 
-// the fused step kernel (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM
+// the fused step kernel (pinn_step_tc.cu): super-tiles of 128 points, one persistent CTA per SM.  A training launch with
+// p.point_w set runs the WEIGHTED instance (device-resident batches only: no theta_inline, no grid)
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st);
 cudaError_t launch_grid_finish(const double* partials, int nrows, double* out, cudaStream_t st);
 // The forward-only loss reduction (pinn_loss_eval): the LOSS instance of the step kernel over n points, one row of 8

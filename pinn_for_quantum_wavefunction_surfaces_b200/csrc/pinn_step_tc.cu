@@ -58,11 +58,15 @@ __host__ __device__ constexpr int tc_group_stash_floats() { return NEV * EVAL_ST
 // geometry hand-off: the E-net warp of a group computes the per-point geometry once and publishes it to the group's MLP
 // warps: 12 floats per point {f1, f2, ir1, ir2 | al1, al2, al11, al12 | al22, dx1, dx2, set bits}, two buffers
 constexpr int GEO_BYTES = 2 * 128 * 12 * 4;
-template <int NEV>
+// WEIGHTED instances: the per-point loss weights of the next super-tile travel with its coordinates, one float per point
+// and stage, in an area behind the geometry buffers (so that every other offset, and the other instances, stay as they are)
+constexpr int PW_STAGE_BYTES = 128 * 4;
+template <int NEV, bool WEIGHTED = false>
 __host__ __device__ constexpr size_t tc_smem_bytes() {
   return sizeof(Wts) + 64 /*mbarriers + tmem base*/ + sizeof(float2) * 4 * 2 * 3 * 32 + sizeof(float) * 4 * tc_group_stash_floats<NEV>() +
-         COORD_STAGES * COORD_STAGE_BYTES + GEO_BYTES;
+         COORD_STAGES * COORD_STAGE_BYTES + GEO_BYTES + (WEIGHTED ? COORD_STAGES * PW_STAGE_BYTES : 0);
 }
+static_assert(tc_smem_bytes<2, true>() <= 227 * 1024, "the weighted poc instance must fit the shared memory of a block");
 
 // ---------------------------------------------------------------------------------------------
 // coordinate stage: the x,y,z,R (and set mask) of the NEXT super-tile travel global -> shared with cp.async while the
@@ -738,6 +742,10 @@ __device__ __forceinline__ void tc_enet_backward(const Wts& w, TcCtx& c, float R
 // the fields mode; instead of per-point stores, role 0 adds res^2, psi^2 of either boundary set, E and the set sizes in
 // double over its super-tiles, and every CTA writes one row {sum res^2, sum psi^2 [set1], sum psi^2 [set2], sum E, |set1|,
 // |set2|, E(point n-1) (owner CTA only), -} to p.grid.partials (p.grid.on = 0: the member only carries the row pointer).
+// WEIGHTED (training only, its own instance): point p carries a loss weight om_p (p.point_w, device float32 [n]).  It enters
+// every per-point term of the sums - res^2, psi^2 of either set, E and the seeds of the reverse sweep - where the valid
+// flag enters, and not the set sizes.  The E-net warp stages om with the coordinates (cp.async, one tile ahead) and hands
+// it to the MLP warps in the geometry slot of dx1, which training launches do not read.
 // ---------------------------------------------------------------------------------------------
 // final fold of a packed vector sum: add the two row halves (lanes l and l + 16), lanes 0..15 store their two columns
 template <typename EntryOf>
@@ -767,7 +775,7 @@ struct TcParamsInline {
   alignas(16) float theta[NTHETA + 3];
 };
 
-template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false>
+template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false, bool WEIGHTED = false>
 __global__ void __launch_bounds__((NEV + 1) * 128, 1)
 pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, TcParamsInline, TcParamsPlain>::type q) {
   const StepParams& p = q.p;
@@ -781,6 +789,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
   float* stash = reinterpret_cast<float*>(smem_raw + sizeof(Wts) + 64 + sizeof(float2) * G * 2 * 3 * 32);
   unsigned char* cstage = smem_raw + tc_smem_bytes<NEV>() - COORD_STAGES * COORD_STAGE_BYTES - GEO_BYTES;
   float4* geo = reinterpret_cast<float4*>(smem_raw + tc_smem_bytes<NEV>() - GEO_BYTES);  // [2][128][3]
+  unsigned char* pwstage = smem_raw + tc_smem_bytes<NEV>();  // WEIGHTED: [COORD_STAGES][128] float
 
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);  // provably warp-uniform: role/group branches and MMA operands
@@ -834,6 +843,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
   } else if (stager) {
     const long long i0 = (long long)blockIdx.x * 128 + slot;
     coord_stage_issue(p, cstage, slot, i0 < p.n ? i0 : p.n - 1);
+    if constexpr (WEIGHTED) cp_async4(smem_u32(pwstage) + slot * 4, p.point_w + (i0 < p.n ? i0 : p.n - 1));
     cp_async_commit();
   }
 
@@ -971,7 +981,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
       // Training launches only: without a reverse sweep the E-net role is not ahead of the MLP roles, and waiting for it
       // cost the 10^8-point grid quadrature 8 % (7.6e9 vs 8.2e9 points/s) - there every role forms its own geometry.
       Geom g;
-      float cur_dx1, cur_dx2, mk_f = 0.0f;
+      float cur_dx1, cur_dx2, mk_f = 0.0f, pw = 1.0f;
       if (!TRAIN) {
         const RawPt raw = p.grid.on ? (p.grid.sph ? tc_sph_point(p.grid, pi) : tc_grid_point(p, pi)) : coord_stage_read(p, cbuf, slot);
         g = geom_from_raw(raw);
@@ -992,9 +1002,10 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
                                           : *(const uint32_t*)(cbuf + 4 * COORD_COL_BYTES + slot * 4) >> (8u * (unsigned)((uintptr_t)(p.mask + pi) & 3u));
             mk_f = (float)(mk & 3u);
           }
+          if constexpr (WEIGHTED) pw = *(const float*)(pwstage + (it % COORD_STAGES) * PW_STAGE_BYTES + slot * 4);
           gp[0] = make_float4(g.f1, g.f2, g.ir1, g.ir2);
           gp[1] = make_float4(g.al1, g.al2, g.al11, g.al12);
-          gp[2] = make_float4(g.al22, cur_dx1, cur_dx2, mk_f);
+          gp[2] = make_float4(g.al22, WEIGHTED ? pw : cur_dx1, cur_dx2, mk_f);
           asm volatile("bar.arrive %0, %1;" ::"r"(8 + grp), "r"((NEV + 1) * 32) : "memory");
         } else {
           named_barrier(8 + grp, (NEV + 1) * 32);
@@ -1002,6 +1013,7 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
           g.f1 = q0.x; g.f2 = q0.y; g.ir1 = q0.z; g.ir2 = q0.w;
           g.al1 = q1.x; g.al2 = q1.y; g.al11 = q1.z; g.al12 = q1.w;
           g.al22 = q2.x; cur_dx1 = q2.y; cur_dx2 = q2.z; mk_f = q2.w;
+          if constexpr (WEIGHTED) pw = q2.y;
           g.R = 0.0f;  // only the E-net warp uses R
         }
       }
@@ -1018,6 +1030,8 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
             if (bulk_issuer) coord_stage_issue_bulk(p, nbuf, &cfull[(it + 1) % COORD_STAGES], stn);
           } else {
             coord_stage_issue(p, nbuf, slot, in < p.n ? in : p.n - 1);
+            if constexpr (WEIGHTED)
+              cp_async4(smem_u32(pwstage + ((it + 1) % COORD_STAGES) * PW_STAGE_BYTES) + slot * 4, p.point_w + (in < p.n ? in : p.n - 1));
           }
         }
         cp_async_commit();
@@ -1150,7 +1164,8 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
         m1f = (g.ir1 * p.bcut <= 1.0f) ? 1.0f : 0.0f;
         m2f = (g.ir2 * p.bcut <= 1.0f) ? 1.0f : 0.0f;
       }
-      const float vw = valid ? 1.0f : 0.0f;
+      const float vw = valid ? (WEIGHTED ? pw : 1.0f) : 0.0f;  // the point's weight in the sums
+      const float vc = valid ? 1.0f : 0.0f;                     // ... and in the set sizes
       const float rbar = 2.0f * w_pde * res * vw;
       const float pbar = 2.0f * fmaf(w_bc1, m1f, w_bc2 * m2f) * psi * vw;
       if (IS_MLP) {
@@ -1165,8 +1180,8 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
           extra[2] = psi * psi * m2f * vw;
           extra[3] = E * vw;
           extra[4] = p.base_grads ? lamN : 0.0f;  // dL/dbo
-          extra[5] = m1f * vw;
-          extra[6] = m2f * vw;
+          extra[5] = m1f * vc;
+          extra[6] = m2f * vc;
         }
         if (p.base_grads) {
           tc_mlp_backward(w, c, cb, a, b, al1, al2, al11, al12, al22, sN * lamN, sN * lamD, Hs, Gs, lane, extra, acc);
@@ -1312,10 +1327,10 @@ pinn_step_tc_kernel(const __grid_constant__ typename std::conditional<INLINE, Tc
 // =================================================================================================
 // host-side launcher
 // =================================================================================================
-template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false>
+template <int NEV, bool TRAIN, bool INLINE, bool LOSS = false, bool WEIGHTED = false>
 static cudaError_t launch_step_tc_t(const StepParams& p, int grid, cudaStream_t st) {
-  auto kern = pinn_step_tc_kernel<NEV, TRAIN, INLINE, LOSS>;
-  constexpr size_t smem = tc_smem_bytes<NEV>();
+  auto kern = pinn_step_tc_kernel<NEV, TRAIN, INLINE, LOSS, WEIGHTED>;
+  constexpr size_t smem = tc_smem_bytes<NEV, WEIGHTED>();
   static bool configured[16] = {false};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -1444,6 +1459,10 @@ cudaError_t launch_loss_tc(int nev, const StepParams& p, int grid, cudaStream_t 
 }
 
 cudaError_t launch_step_tc(int nev, bool train, const StepParams& p, int grid, cudaStream_t st) {
+  if (train && p.point_w) {
+    if (p.theta_inline || p.grid.on) return cudaErrorInvalidValue;
+    return nev == 2 ? launch_step_tc_t<2, true, false, false, true>(p, grid, st) : launch_step_tc_t<1, true, false, false, true>(p, grid, st);
+  }
   if (train && p.theta_inline)
     return nev == 2 ? launch_step_tc_t<2, true, true>(p, grid, st) : launch_step_tc_t<1, true, true>(p, grid, st);
   if (nev == 2) return train ? launch_step_tc_t<2, true, false>(p, grid, st) : launch_step_tc_t<2, false, false>(p, grid, st);

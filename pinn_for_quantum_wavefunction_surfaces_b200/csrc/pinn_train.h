@@ -61,6 +61,11 @@ struct AdaptiveParams {
   double* part;                                   // device [adaptive_scratch_doubles(N)]
   const unsigned long long* pool_batch;           // device: the batch counter as the pool's draw left it (one past the pool)
   long long* idx;                                 // device [n] pool index of every output point, or NULL
+  // importance weights (pinn_sample_adaptive_importance), or NULL: point_w[j] = float(T / (N w_i)) of the candidate i
+  // output j takes, and out.weights = {1/n, N/(n |set1 of the pool|), N/(n |set2 of the pool|)} from pool_counts (the
+  // pool's set sizes as its draw counted them: its sampler must not reset them; the selection zeroes them after use)
+  float* point_w;
+  unsigned long long* pool_counts;
   SampleParams out;                               // the batch: n, seed, x..mask, counts, weights, ticket, batch_counter
                                                   // (moved on by sample_finish: point it at a scratch word), reset_counts
 };

@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 
 #include "pinn_handle.h"
 #include "pinn_train.h"
@@ -38,11 +39,17 @@ struct pinn_trainer {
   // residual-adaptive sampling (pinn_trainer_set_adaptive): pool_factor * n candidates per resampling step; off at 0
   int pool_factor = 0;
   float ad_k = 1.0f, ad_c = 1.0f;
+  // importance weights (pinn_trainer_set_importance): the adaptive draw also writes omega into pw (n floats, allocated by
+  // the first call that turns it on), and every step whose batch came from such a draw (pw_batch) runs the weighted
+  // training evaluation on it
+  bool importance = false, pw_batch = false;
+  float* pw = nullptr;
   float *px = nullptr, *py = nullptr, *pz = nullptr, *pR = nullptr, *pres = nullptr;
   uint8_t* pmask = nullptr;
   double *pcdf = nullptr, *pweights = nullptr, *ppart = nullptr;
   unsigned long long* pcounts = nullptr;  // {|set1|, |set2|, ticket} of the pool's draw, [3] scratch batch word of the selection
   cudaGraphExec_t graph_ad[2] = {nullptr, nullptr};  // [cur]: adaptive draw + step
+  cudaGraphExec_t graph_w[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // as graph[][], on an importance batch
   bool ad_warmed = false;  // one plain adaptive step has run (the inference kernel's attributes are set)
   // L-BFGS (pinn_trainer_run_lbfgs): state of lb_hist pairs, trace [lb_trace_rows][4], the WHILE graph of one evaluation
   unsigned char* lb_state = nullptr;
@@ -117,6 +124,10 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool adaptive_now, 
     a.cdf = t->pcdf; a.part = t->ppart; a.pool_batch = t->batch; a.idx = nullptr;
     a.out = sampler_params(t, b);
     a.out.index_offset = 0; a.out.batch_counter = t->pcounts + 3;
+    if (t->importance) {  // the selection reads the pool's set sizes, then zeroes them
+      a.point_w = t->pw; a.pool_counts = t->pcounts;
+      pool.reset_counts = 0;
+    }
     VariantCoef vc;
     int nev = 0;
     variant_coef(c.variant, &vc, &nev);
@@ -139,6 +150,7 @@ static int trainer_enqueue(pinn_trainer* t, bool sample_now, bool adaptive_now, 
   lc.mask = t->mask[b]; lc.theta = t->theta32; lc.weights = t->weights[b]; lc.grad_mask = c.grad_mask; lc.bcutoff = c.bcutoff;
   lc.sums = t->sums; lc.dtheta = t->grad; lc.E_out = t->E; lc.adam = &a; lc.adam_ticket = t->adam_ticket;
   lc.presample = presample_next ? &next : nullptr;
+  if (adaptive_now ? t->importance : t->pw_batch) lc.point_w = t->pw;
   int rc = loss_fwd_bwd_impl(h, lc, st);
   if (rc) return rc;
   return 0;
@@ -276,9 +288,11 @@ static int trainer_capture(pinn_trainer* t, bool adaptive_now, bool presample_ne
 }
 
 // Pool buffers and the adaptive graphs (the stream is idle)
+// (the importance flag goes with the pool; pw and an importance batch in use stay: its remaining steps keep their weights)
 static void trainer_free_adaptive(pinn_trainer* t) {
   for (cudaGraphExec_t& g : t->graph_ad)
     if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+  t->importance = false;
   cudaFree(t->px); cudaFree(t->py); cudaFree(t->pz); cudaFree(t->pR); cudaFree(t->pres); cudaFree(t->pmask);
   cudaFree(t->pcdf); cudaFree(t->pweights); cudaFree(t->ppart); cudaFree(t->pcounts);
   t->px = t->py = t->pz = t->pR = t->pres = nullptr;
@@ -314,26 +328,31 @@ int pinn_sample(pinn_handle* h, int64_t n, uint64_t seed, uint64_t batch, const 
   return 0;
 }
 
-int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed, uint64_t batch,
-                         const float box[8], float cutoff, float bcutoff, float k, float c, float* pool_x, float* pool_y,
-                         float* pool_z, float* pool_R, uint8_t* pool_mask, float* pool_res, double* pool_cdf, float* x,
-                         float* y, float* z, float* R, uint8_t* mask, int64_t* idx, uint64_t* counts, double* weights,
-                         void* stream) {
-  if (!h) return PINN_EINVAL;
+}  // extern "C"
+
+// pinn_sample_adaptive and its importance form (point_w != NULL); `fn` names the entry in error messages
+static int sample_adaptive_impl(const char* fn, pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool,
+                                uint64_t seed, uint64_t batch, const float box[8], float cutoff, float bcutoff, float k, float c,
+                                float* pool_x, float* pool_y, float* pool_z, float* pool_R, uint8_t* pool_mask, float* pool_res,
+                                double* pool_cdf, float* x, float* y, float* z, float* R, uint8_t* mask, int64_t* idx,
+                                uint64_t* counts, double* weights, float* point_w, void* stream) {
   std::lock_guard<std::mutex> lk(h->mu);
-  if (n <= 0 || pool < n) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: need 0 < n <= pool");
+  std::string e = std::string(fn) + ": ";
+  if (n <= 0 || pool < n) return fail(h, PINN_EINVAL, (e + "need 0 < n <= pool").c_str());
   if (!(k >= 0.0f) || !std::isfinite(k) || !(c >= 0.0f) || !std::isfinite(c))
-    return fail(h, PINN_EINVAL, "pinn_sample_adaptive: k and c must be finite and >= 0");
+    return fail(h, PINN_EINVAL, (e + "k and c must be finite and >= 0").c_str());
+  // Lbc weights psi^2, not res^2: a candidate with zero residual must keep a positive probability
+  if (point_w && !(c > 0.0f)) return fail(h, PINN_EINVAL, (e + "importance weights need c > 0").c_str());
   if (!theta || !box || !pool_x || !pool_y || !pool_z || !pool_R || !pool_mask || !pool_res || !pool_cdf || !x || !y || !z ||
       !R || !mask || !counts || !weights)
-    return fail(h, PINN_EINVAL, "pinn_sample_adaptive: NULL pointer argument");
+    return fail(h, PINN_EINVAL, (e + "NULL pointer argument").c_str());
   VariantCoef vc;
   int nev = 0;
-  if (variant_coef(variant, &vc, &nev)) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: unknown variant");
+  if (variant_coef(variant, &vc, &nev)) return fail(h, PINN_EINVAL, (e + "unknown variant").c_str());
   DevGuard dev_guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   const long long scratch_rows = (adaptive_scratch_doubles(pool) + NPART - 1) / NPART;
-  if (scratch_rows > 0x7fffffffll) return fail(h, PINN_EINVAL, "pinn_sample_adaptive: pool too large");
+  if (scratch_rows > 0x7fffffffll) return fail(h, PINN_EINVAL, (e + "pool too large").c_str());
   pinn_workspace* ws = ws_for(h, st, std::max(h->sm_count, (int)scratch_rows));
   if (!ws) return PINN_EINVAL;
   unsigned long long* batch_counter = ws->counts + 2;  // [0..1] the pool's set sizes, [2] its batch index, [3] block ticket
@@ -350,12 +369,38 @@ int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_
   a.pool = pool; a.k = k; a.c = c;
   a.px = pool_x; a.py = pool_y; a.pz = pool_z; a.pR = pool_R; a.pmask = pool_mask; a.res = pool_res;
   a.cdf = pool_cdf; a.part = ws->partials; a.pool_batch = batch_counter; a.idx = reinterpret_cast<long long*>(idx);
+  a.point_w = point_w; a.pool_counts = ws->counts;
   a.out = ps;
   a.out.n = n; a.out.x = x; a.out.y = y; a.out.z = z; a.out.R = R; a.out.mask = mask;
   a.out.counts = (unsigned long long*)counts; a.out.weights = weights;
   // rad_scan_kernel has read the pool's batch index by the time the selection's finish moves this word on again
   a.out.batch_counter = batch_counter;
   return adaptive_enqueue(h, nev, vc, theta, ps, true, a, st);
+}
+
+extern "C" {
+
+int pinn_sample_adaptive(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed, uint64_t batch,
+                         const float box[8], float cutoff, float bcutoff, float k, float c, float* pool_x, float* pool_y,
+                         float* pool_z, float* pool_R, uint8_t* pool_mask, float* pool_res, double* pool_cdf, float* x,
+                         float* y, float* z, float* R, uint8_t* mask, int64_t* idx, uint64_t* counts, double* weights,
+                         void* stream) {
+  if (!h) return PINN_EINVAL;
+  return sample_adaptive_impl("pinn_sample_adaptive", h, variant, theta, n, pool, seed, batch, box, cutoff, bcutoff, k, c, pool_x,
+                              pool_y, pool_z, pool_R, pool_mask, pool_res, pool_cdf, x, y, z, R, mask, idx, counts, weights,
+                              nullptr, stream);
+}
+
+int pinn_sample_adaptive_importance(pinn_handle* h, int variant, const float* theta, int64_t n, int64_t pool, uint64_t seed,
+                                    uint64_t batch, const float box[8], float cutoff, float bcutoff, float k, float c,
+                                    float* pool_x, float* pool_y, float* pool_z, float* pool_R, uint8_t* pool_mask,
+                                    float* pool_res, double* pool_cdf, float* x, float* y, float* z, float* R, uint8_t* mask,
+                                    int64_t* idx, uint64_t* counts, double* weights, float* point_w, void* stream) {
+  if (!h) return PINN_EINVAL;
+  if (!point_w) return fail(h, PINN_EINVAL, "pinn_sample_adaptive_importance: NULL pointer argument");
+  return sample_adaptive_impl("pinn_sample_adaptive_importance", h, variant, theta, n, pool, seed, batch, box, cutoff, bcutoff,
+                              k, c, pool_x, pool_y, pool_z, pool_R, pool_mask, pool_res, pool_cdf, x, y, z, R, mask, idx, counts,
+                              weights, point_w, stream);
 }
 
 int pinn_adam_step(pinn_handle* h, double* theta, double* m, double* v, const double* grad, const double* sums, float* theta32,
@@ -536,9 +581,12 @@ int pinn_trainer_destroy(pinn_trainer* t) {
   DevGuard dev_guard(t->h->device);
   if (t->st) cudaStreamSynchronize(t->st);
   for (int a = 0; a < 2; a++)
-    for (int b = 0; b < 2; b++)
+    for (int b = 0; b < 2; b++) {
       if (t->graph[a][b]) cudaGraphExecDestroy(t->graph[a][b]);
+      if (t->graph_w[a][b]) cudaGraphExecDestroy(t->graph_w[a][b]);
+    }
   trainer_free_adaptive(t);
+  cudaFree(t->pw);
   trainer_free_lbfgs(t);
   trainer_free_validation(t);
   for (int b = 0; b < 2; b++) {
@@ -586,8 +634,10 @@ int pinn_trainer_load_state(pinn_trainer* t, const double* theta, const double* 
   t->step_base = step;
   // captured graphs carry the old step_base in their kernel parameters
   for (int a = 0; a < 2; a++)
-    for (int b = 0; b < 2; b++)
+    for (int b = 0; b < 2; b++) {
       if (t->graph[a][b]) { cudaGraphExecDestroy(t->graph[a][b]); t->graph[a][b] = nullptr; }
+      if (t->graph_w[a][b]) { cudaGraphExecDestroy(t->graph_w[a][b]); t->graph_w[a][b] = nullptr; }
+    }
   for (cudaGraphExec_t& g : t->graph_ad)
     if (g) { cudaGraphExecDestroy(g); g = nullptr; }
   // the L-BFGS state restarts fresh (torch's empty state), like a new optimizer on the loaded parameters
@@ -719,6 +769,26 @@ int pinn_trainer_set_adaptive(pinn_trainer* t, int pool_factor, float k, float c
   return 0;
 }
 
+int pinn_trainer_set_importance(pinn_trainer* t, int on) {
+  if (!t) return PINN_EINVAL;
+  pinn_handle* h = t->h;
+  if (on && t->pool_factor <= 0)
+    return fail(h, PINN_EINVAL, "pinn_trainer_set_importance: adaptive sampling is off (pinn_trainer_set_adaptive)");
+  if (on && !(t->ad_c > 0.0f))
+    return fail(h, PINN_EINVAL, "pinn_trainer_set_importance: importance weights need c > 0");
+  DevGuard dev_guard(h->device);
+  CU(h, cudaStreamSynchronize(t->st));
+  if (on && !t->pw) CU(h, cudaMalloc(&t->pw, (size_t)t->cfg.n * 4));
+  if ((on != 0) != t->importance) {
+    // the adaptive graphs were captured with the other selection and step; the first draw in the new mode runs plain
+    for (cudaGraphExec_t& g : t->graph_ad)
+      if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+    t->ad_warmed = false;
+  }
+  t->importance = on != 0;
+  return 0;
+}
+
 // Caller-provided batch instead of the sampler (parity runs feed the reference's own points): device float32 columns,
 // mask bytes and the weights {1/n, 1/|set1|, 1/|set2|}; stays in use until the next resampling step.
 int pinn_trainer_set_batch(pinn_trainer* t, const float* x, const float* y, const float* z, const float* R, const uint8_t* mask,
@@ -737,6 +807,7 @@ int pinn_trainer_set_batch(pinn_trainer* t, const float* x, const float* y, cons
   CU(h, cudaMemcpyAsync(t->weights[b], weights_host, 3 * 8, cudaMemcpyDefault, t->st));
   CU(h, cudaStreamSynchronize(t->st));
   t->have_batch = true;
+  t->pw_batch = false;
   return 0;
 }
 
@@ -769,9 +840,11 @@ int pinn_trainer_run(pinn_trainer* t, int64_t steps, int resample, int use_graph
       if (t->next_ready) { t->cur ^= 1; t->next_ready = false; }  // drawn while the previous step was reduced
       else sample_now = true;
     }
+    if (rs) t->pw_batch = adaptive_now && t->importance;  // the batch of this step, and of the steps up to the next draw
     const bool presample_next = !adaptive && (k + 1 < steps) && resamples(tt + 1);
     if (use_graph && t->warmed && !sample_now && (!adaptive_now || t->ad_warmed)) {
-      cudaGraphExec_t& g = adaptive_now ? t->graph_ad[t->cur] : t->graph[t->cur][presample_next ? 1 : 0];
+      cudaGraphExec_t& g = adaptive_now ? t->graph_ad[t->cur]
+                           : t->pw_batch ? t->graph_w[t->cur][presample_next ? 1 : 0] : t->graph[t->cur][presample_next ? 1 : 0];
       if (!g) {
         int rc = trainer_capture(t, adaptive_now, presample_next, &g);
         if (rc) return rc;
@@ -811,6 +884,8 @@ int pinn_trainer_run_lbfgs(pinn_trainer* t, const pinn_lbfgs_config* cfg, int re
     return fail(h, PINN_ENOTSUP, "pinn_trainer_run_lbfgs: L-BFGS is not available with the data-parallel exchange");
   if (resample && t->pool_factor > 0)
     return fail(h, PINN_ENOTSUP, "pinn_trainer_run_lbfgs: L-BFGS does not draw adaptive batches");
+  if (!resample && t->pw_batch)
+    return fail(h, PINN_ENOTSUP, "pinn_trainer_run_lbfgs: L-BFGS does not evaluate importance-weighted batches");
   DevGuard dev_guard(h->device);
   const int64_t slots = lbfgs_slots(c);
   if (!t->lb_state || t->lb_hist != c.history_size || t->lb_trace_rows < slots) {
@@ -838,6 +913,7 @@ int pinn_trainer_run_lbfgs(pinn_trainer* t, const pinn_lbfgs_config* cfg, int re
     CU(h, launch_sample(s, false, t->st));
     h->launches += 1;
     t->have_batch = true;
+    t->pw_batch = false;
   }
   CU(h, cudaMemsetAsync(t->lb_trace, 0, (size_t)t->lb_trace_rows * 4 * 8, t->st));
   CU(h, launch_lbfgs_begin(t->lb_state, c, t->theta, t->theta32, t->st));

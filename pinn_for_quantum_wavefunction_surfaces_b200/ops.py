@@ -51,13 +51,28 @@ def indices_to_mask(n, idx1, idx2, device):
     return mask, int(r1.numel()), int(r2.numel())
 
 
+def check_point_weights(point_weights, n, device):
+    """Refuse malformed per-point loss weights: a contiguous float32 tensor of n finite values >= 0 on `device`.  The
+    value check reads the tensor back (one synchronisation of torch's current stream)."""
+    w = point_weights
+    if not torch.is_tensor(w) or w.dtype != torch.float32 or w.dim() != 1 or w.numel() != n or not w.is_contiguous():
+        raise ValueError("point_weights must be a contiguous float32 vector of n = %d elements" % n)
+    if w.device != device:
+        raise ValueError("point_weights must be on %s, got %s" % (device, w.device))
+    if not bool(torch.isfinite(w).all()) or bool((w < 0).any()):
+        raise ValueError("point_weights must be finite and >= 0")
+
+
 def loss_and_grad_raw(variant, x, y, z, R, theta, mask=None, weights=None, grad_mask=0xFFFF, want_E=False,
-                      bcutoff=BC_CUTOFF, sums=None, dtheta=None, E_out=None):
+                      bcutoff=BC_CUTOFF, sums=None, dtheta=None, E_out=None, point_weights=None):
     """Thin wrapper over pinn_loss_fwd_bwd for DEVICE tensors (no allocation when the outputs are given).
 
     x,y,z,R: CUDA float32/float64 (n,) ; theta: CUDA float32 (1521,) ; mask: CUDA uint8 (n,) or None ;
     weights: CUDA float64 (3,) or None.  Returns (sums[8] f64, dtheta[1521] f64, E_out or None), all on
-    the device, enqueued on torch's current stream."""
+    the device, enqueued on torch's current stream.
+    point_weights: None, or CUDA float32 (n,) per-point loss weights om >= 0 (pinn_loss_fwd_bwd_weighted): every
+    per-point term of the sums and of the gradient takes its om, the counted set sizes do not - e.g. the "point_weights"
+    of sample_adaptive(importance=True) with its "weights"."""
     if not x.is_cuda:
         raise PinnError("loss_and_grad_raw needs CUDA tensors (there is no CPU path)")
     dev = x.device
@@ -76,6 +91,13 @@ def loss_and_grad_raw(variant, x, y, z, R, theta, mask=None, weights=None, grad_
     if want_E and E_out is None:
         E_out = torch.empty(n, dtype=torch.float32, device=dev)
     stream = torch.cuda.current_stream(dev).cuda_stream
+    if point_weights is not None:
+        check_point_weights(point_weights, n, dev)
+        rc = h.L.pinn_loss_fwd_bwd_weighted(h.h, int(variant), n, _ptr(x), _ptr(y), _ptr(z), _ptr(R), code, _ptr(mask),
+                                            _ptr(theta), _ptr(weights), _ptr(point_weights), int(grad_mask),
+                                            float(bcutoff), _ptr(sums), _ptr(dtheta), _ptr(E_out), ctypes.c_void_p(stream))
+        h.check(rc, "pinn_loss_fwd_bwd_weighted")
+        return sums, dtheta, E_out
     rc = h.L.pinn_loss_fwd_bwd(h.h, int(variant), n, _ptr(x), _ptr(y), _ptr(z), _ptr(R), code, _ptr(mask),
                                _ptr(theta), _ptr(weights), int(grad_mask), float(bcutoff), _ptr(sums),
                                _ptr(dtheta), _ptr(E_out), ctypes.c_void_p(stream))

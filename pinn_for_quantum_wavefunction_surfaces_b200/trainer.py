@@ -53,12 +53,16 @@ def sample(n, seed, batch, box=BOX_POC, cutoff=0.005, bcutoff=17.5, device=None)
 
 
 def sample_adaptive(variant, theta, n, pool_factor=4, k=1.0, c=1.0, seed=0, batch=0, box=None, cutoff=0.005, bcutoff=17.5,
-                    device=None):
+                    device=None, importance=False):
     """Residual-adaptive batch (pinn_sample_adaptive): n points out of pool_factor * n uniform candidates
     (= sample(pool_factor * n, seed, batch)), candidate i taken with probability proportional to
     |res_i|^k * N / sum |res|^k + c, res = the residual of `theta` (packed parameters) there, by systematic resampling.
     -> dict(x, y, z, R, mask, counts, weights as sample(); idx int64 (n,) pool index of each point; pool = dict(x, y, z,
-    R, mask) of the candidates; res float32 and cdf float64 (N,), the candidates' residuals and weight prefix sums)."""
+    R, mask) of the candidates; res float32 and cdf float64 (N,), the candidates' residuals and weight prefix sums).
+    importance=True (pinn_sample_adaptive_importance; needs c > 0): the same batch, plus "point_weights" float32 (n,),
+    om_j = 1 / (N P_i) of the candidate each point came from, and "weights" = {1/n, N/(n |set1 of the pool|),
+    N/(n |set2 of the pool|)}: loss_and_grad_raw(..., weights, point_weights=...) on it is an unbiased estimate of the
+    pool's uniform loss and gradient."""
     variant = {"poc": 0, "trainpy": 1}.get(variant, variant)
     if box is None:
         box = BOX_POC if variant == 0 else BOX_TRAINPY
@@ -78,10 +82,15 @@ def sample_adaptive(variant, theta, n, pool_factor=4, k=1.0, c=1.0, seed=0, batc
     out["pool"], out["res"], out["cdf"] = pool, col(N), col(N, torch.float64)
     b = (ctypes.c_float * 8)(*box)
     stream = torch.cuda.current_stream(dev).cuda_stream
-    rc = h.L.pinn_sample_adaptive(h.h, variant, _ptr(th), n, N, seed, batch, b, cutoff, bcutoff, k, c,
-                                  *[_ptr(pool[k_]) for k_ in ("x", "y", "z", "R", "mask")], _ptr(out["res"]),
-                                  _ptr(out["cdf"]), *[_ptr(out[k_]) for k_ in ("x", "y", "z", "R", "mask", "idx", "counts",
-                                                                              "weights")], ctypes.c_void_p(stream))
+    args = [h.h, variant, _ptr(th), n, N, seed, batch, b, cutoff, bcutoff, k, c,
+            *[_ptr(pool[k_]) for k_ in ("x", "y", "z", "R", "mask")], _ptr(out["res"]), _ptr(out["cdf"]),
+            *[_ptr(out[k_]) for k_ in ("x", "y", "z", "R", "mask", "idx", "counts", "weights")]]
+    if importance:
+        out["point_weights"] = col(n)
+        rc = h.L.pinn_sample_adaptive_importance(*args, _ptr(out["point_weights"]), ctypes.c_void_p(stream))
+        h.check(rc, "pinn_sample_adaptive_importance")
+        return out
+    rc = h.L.pinn_sample_adaptive(*args, ctypes.c_void_p(stream))
     h.check(rc, "pinn_sample_adaptive")
     return out
 
@@ -215,13 +224,18 @@ class Trainer:
         if validation:
             self.set_validation(**validation)
 
-    def set_adaptive(self, pool_factor=4, k=1.0, c=1.0):
+    def set_adaptive(self, pool_factor=4, k=1.0, c=1.0, importance=False):
         """Residual-adaptive batches (pinn_trainer_set_adaptive): every resampling step draws its n points from
         pool_factor * n candidates in proportion to |res|^k / mean |res|^k + c at the current parameters; pool_factor=0
-        turns it off.  The history and best-model record are then evaluated on the adaptive batches, so Ltot is not
-        comparable with a uniform run's; set_validation records a held-out loss that is."""
+        turns it off.  Without importance weights the history and best-model record are evaluated on the adaptive
+        batches, a residual-weighted mean that is not comparable with a uniform run's; set_validation records a
+        held-out loss that is.  importance=True (pinn_trainer_set_importance; needs c > 0) weights every point of an
+        adaptive batch by 1 / (N P_i) and takes the pool's set sizes in the loss weights, so that each step's loss and
+        gradient are unbiased estimates of the pool's uniform ones."""
         self.h.check(self.h.L.pinn_trainer_set_adaptive(self.t, int(pool_factor), float(k), float(c)),
                      "pinn_trainer_set_adaptive")
+        if importance:
+            self.h.check(self.h.L.pinn_trainer_set_importance(self.t, 1), "pinn_trainer_set_importance")
 
     def set_validation(self, n, seed, every, capacity=None):
         """Held-out validation loss (pinn_trainer_set_validation): n points drawn once now, sample(n, seed, 0) with the
@@ -373,7 +387,8 @@ def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_t
                   adaptive=None, validation=None):
     """train(params, lr, epochs) of train.py on the device.  Like the reference it evaluates epochs+1 losses, takes `epochs`
     optimizer steps and returns the parameters of the best loss seen (train.py:58-69).  Returns (theta_best, info).
-    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive).
+    adaptive: None (uniform batches) or dict(pool_factor, k, c[, importance]) for residual-adaptive batches
+    (Trainer.set_adaptive).
     validation: None, or dict(n, seed, every, capacity=None) for a held-out loss (Trainer.set_validation), evaluated at the
     initial parameters and every `every` steps; info then has a "validation" entry (Trainer.read_validation)."""
     if theta0 is None:
@@ -408,7 +423,8 @@ def train_trainpy(theta0=None, n=10000, epochs=1000, lr=8e-3, seed=12345, fine_t
 def train_poc(theta0, params=None, freezeUnits=False, seed=0, use_graph=False, adaptive=None, validation=None):
     """train(params, loadWeights, freezeUnits) of poc/main.py:359-430 on the device.  `params` uses the reference's keys
     (set_params(), poc/main.py:14-45).  Returns (theta_last, theta_saved or None, lossDictionary like poc/main.py:422-427).
-    adaptive: None (uniform batches) or dict(pool_factor, k, c) for residual-adaptive batches (Trainer.set_adaptive).
+    adaptive: None (uniform batches) or dict(pool_factor, k, c[, importance]) for residual-adaptive batches
+    (Trainer.set_adaptive).
     validation: None, or dict(n, seed, every, capacity=None) for a held-out loss (Trainer.set_validation), evaluated at
     theta0 and every `every` steps; the loss dictionary then has a "validation" entry (Trainer.read_validation)."""
     pr = {"xL": -18, "xR": 18, "yL": -18, "yR": 18, "zL": -18, "zR": 18, "RxL": 0.2, "RxR": 4, "cutOff": 0.005,
